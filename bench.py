@@ -7,7 +7,7 @@ random-init weights.  One "step" = one image per GPU (images are independent uni
 scaling, no data-path collective -- SURVEY §8e).  configs[1] (training step) needs the backward
 kernels, which are not built yet; configs[0] is the CPU-runnable parity case.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|bf16]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|bf16] [--dump-outputs DIR]
 
 * value : whole-job HR MPix/s with the inputs resident in HBM (CUDA events, barrier + sync on both
           sides, max over ranks).  The 553 MB of inputs per step exceed the 126 MB L2.
@@ -19,6 +19,11 @@ kernels, which are not built yet; configs[0] is the CPU-runnable parity case.
 * cpu_baseline : the oracle (CPU port of the reference forward) on the host cores, rank 0, N=1.
 * --impl reference : the reference's CPU implementation of the path = the oracle port (the
           reference is pure Python and does not travel to the GPU box), all host threads.
+* --dump-outputs DIR : after the timed steps of the C3 job, DIR/sr_sample.npy (float32, one row per image of this rank's
+          last timed step; sr_sample_rank<r>.npy per rank with several GPUs) holds a fixed, seeded sample of the SR images
+          that step returned (dump_sample_index).  Inputs and weights are seeded, so two builds run with the same
+          arguments can be compared output for output.  The gathers that take the sample run inside the last timed step:
+          the line then carries a `dump_outputs` note, and timings are taken from runs without the option.
 """
 import argparse
 import json
@@ -243,7 +248,7 @@ def run_reference_train(args):
     threads = os.cpu_count() or 1
     hw = 64 if args.workload == "c2" else 96
     batch = 2                                                   # bounded sample of the global batch
-    v, t = cpu_oracle_train_throughput(hw, batch, max(1, min(args.steps, 3)), 1, threads, STAGE_WEIGHTS[args.workload])
+    v, t = cpu_oracle_train_throughput(hw, batch, args.steps, args.warmup, threads, STAGE_WEIGHTS[args.workload])
     line = {
         "impl": "reference", "metric": "fusion_train_patches_per_s", "value": v, "unit": "patches/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": t * 1e3,
@@ -701,6 +706,21 @@ def train_config(workload, patches, B, hw, precision):
 
 N_JOB_IMAGES = 100                            # BASELINE configs[2]: "100 images tiled across 1/2/4/8 B200"
 N_INPUT_SETS = 4                              # distinct synthetic images cycled through (4 x 553 MB > the 126 MB L2)
+DUMP_BUDGET_BYTES = 48 << 20                  # --dump-outputs: the float32 samples of all ranks together
+
+
+def dump_sample_index(rows, numel, world=1):
+    """Indices into the flattened SR images (rows x k, each row sorted) that --dump-outputs keeps: every element while
+    rows x numel x world floats fit DUMP_BUDGET_BYTES, else k seeded random elements per image.  Each row draws its own
+    elements, so the images of one input set (the job cycles N_INPUT_SETS inputs) together cover more of that output."""
+    import torch
+    if rows == 0:                                 # a rank the job schedule gives no image
+        return torch.empty(0, 0, dtype=torch.long)
+    k = DUMP_BUDGET_BYTES // (4 * rows * world)
+    if k >= numel:
+        return torch.arange(numel).repeat(rows, 1)
+    g = torch.Generator().manual_seed(0)
+    return torch.randint(0, numel, (rows, k), generator=g).sort(dim=1).values
 
 
 def c3_config(H, W):
@@ -900,7 +920,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-eager", action="store_true", help="skip the PyTorch-eager-on-the-same-GPU baseline of the C3 line")
     ap.add_argument("--no-train", action="store_true", help="skip the C2 training-step figure added to the C3 line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="C3 job: write a seeded sample of the SR images of the last timed "
+                                                          "step to DIR/sr_sample.npy (float32, at most 48 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c3"):
+        ap.error("--dump-outputs is implemented for the c3 workload of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "c3t":
@@ -959,20 +985,35 @@ def main():
     from isr_b200.serving import ConcurrentFusion
     conc = ConcurrentFusion(m, ways=args.in_flight, device=dev) if args.in_flight > 1 else None
 
-    def job_resident():
+    def job_resident(sink=None):
+        """sink(i, sr): called with the SR image of this rank's i-th image of the step, on the stream that computed it."""
         if conc is not None:                                    # whole images of this rank: `in_flight` forwards on as many streams
-            conc.run(sets[i % N_INPUT_SETS] for i in mine)
+            conc.run((sets[i % N_INPUT_SETS] for i in mine), sink)
         else:
-            for i in mine:
+            for j, i in enumerate(mine):
                 lr_, im_, ft_ = sets[i % N_INPUT_SETS]
-                m.forward_with_precomputed(lr_, im_, ft_)
-        for img, ranks, grid in my_tail:
+                sr = m.forward_with_precomputed(lr_, im_, ft_)
+                if sink is not None:
+                    sink(j, sr)
+        for j, (img, ranks, grid) in enumerate(my_tail):
             lr_, im_, ft_ = sets[img % N_INPUT_SETS]
-            fuse_tiled(m, lr_, im_, ft_, grid=grid, rank=ranks.index(rank), world=len(ranks), group=groups.get(img))
+            sr = fuse_tiled(m, lr_, im_, ft_, grid=grid, rank=ranks.index(rank), world=len(ranks), group=groups.get(img))
+            if sink is not None:
+                sink(len(mine) + j, sr)
+
+    keep = dump = None
+    if args.dump_outputs:
+        dump_idx = dump_sample_index(len(mine) + len(my_tail), 3 * 16 * H * W, world).to(dev)
+        dump = torch.empty(dump_idx.shape, device=dev)
+
+        def keep(i, sr):                                        # one gather kernel per image, last timed step only
+            torch.index_select(sr.reshape(-1), 0, dump_idx[i], out=dump[i])
 
     for _ in range(warmup):                                     # >= 3 warm-up forwards per distinct path (not whole jobs)
         lr_, im_, ft_ = sets[0]
         m.forward_with_precomputed(lr_, im_, ft_)
+    if keep is not None and dump.shape[0]:                      # first launch (module load) of the gather before the timed region
+        keep(0, m.forward_with_precomputed(*sets[0]))
     if conc is not None:
         for _ in range(warmup):
             conc.run(sets[i % N_INPUT_SETS] for i in range(args.in_flight))
@@ -989,11 +1030,17 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for step in range(args.steps):
-        job_resident()
+        job_resident(keep if step == args.steps - 1 else None)
     e1.record()
     barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop()
+    if dump is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = "sr_sample" if world == 1 else f"sr_sample_rank{rank}"
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), dump.cpu().numpy())
+        keep = dump = dump_idx = None
     # the dominant kernel's launch time: CUDA-event pairs around the hot layers of 100 further forwards on ONE stream (with
     # several images in flight a launch's wall time would include kernels of the other stream)
     eng.timed_layers = timed = {n: [] for n in hot}
@@ -1155,6 +1202,10 @@ def main():
                          "whole_forward_tflops": whole_tflops, "whole_forward_frac": whole_tflops / tensor_peak,
                          "whole_forward_target_frac": 0.40},
         }
+        if args.dump_outputs:
+            line["dump_outputs"] = {"dir": args.dump_outputs,
+                                    "note": "the timed region of this run includes one gather kernel per image of its last step "
+                                            "(the sample written to the dump); take timings from runs without --dump-outputs"}
         if trace_rows:
             line["forward_breakdown"] = forward_breakdown(trace_rows, H, W, hbm_peak, tensor_peak)
         if train is not None:

@@ -7,7 +7,7 @@ how the geometric augmentation draws from ``random`` and transforms every tensor
 
 Parity pin: ``tests/golden/cache_golden.json`` holds SHA-256 digests of the samples the *reference class itself*
 returns on a seeded mock cache (``oracle/make_cache_golden.py``); ``tests/test_cache_format.py`` checks this
-restatement against them, and against the reference class directly when ``/root/reference`` is present.
+restatement against them.
 """
 from __future__ import annotations
 

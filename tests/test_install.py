@@ -5,8 +5,9 @@ import sys
 
 import pytest
 
+from oracle.reference_layout import write_reference_layout
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 def test_install_exports_reference_names():
@@ -23,8 +24,9 @@ def test_install_exports_reference_names():
     del sys.modules["src.models.enhanced_fusion_v2"]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
-def test_reference_package_import_resolves_to_our_module():
+def test_reference_package_import_resolves_to_our_module(tmp_path):
+    """Through a package with the reference's layout whose own enhanced_fusion_v2 refuses to import."""
+    ref = write_reference_layout(tmp_path)
     code = (
         "import sys; sys.path.insert(0, %r); import isr_b200, isr_b200.install as I; I.install();"
         "sys.path.insert(0, %r);"
@@ -32,21 +34,22 @@ def test_reference_package_import_resolves_to_our_module():
         "from src.models.enhanced_fusion_v2 import CompleteEnhancedFusionSR as B2;"
         "assert A is isr_b200.CompleteEnhancedFusionSR and B2 is A;"
         "m = create_enhanced_fusion(None); assert m.cached_mode and len(m.state_dict()) == 226; print('ok')"
-    ) % (ROOT, REF)
+    ) % (ROOT, ref)
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600,
                        env=dict(os.environ, PYTHONDONTWRITEBYTECODE="1"))
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-2000:]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
-def test_reference_data_package_resolves_to_shard_loader():
+def test_reference_data_package_resolves_to_shard_loader(tmp_path):
+    """Through a package with the reference's layout whose own cached_dataset is the pickle loader."""
+    ref = write_reference_layout(tmp_path)
     code = (
         "import sys; sys.path.insert(0, %r); import isr_b200, isr_b200.install as I; I.install(loader=True);"
         "sys.path.insert(0, %r);"
         "from src.data import CachedSRDataset, create_cached_dataloader;"
         "from isr_b200 import cache as CA;"
         "assert CachedSRDataset is CA.ShardDataset and create_cached_dataloader.__module__ == 'isr_b200.install'; print('ok')"
-    ) % (ROOT, REF)
+    ) % (ROOT, ref)
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600,
                        env=dict(os.environ, PYTHONDONTWRITEBYTECODE="1"))
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-2000:]

@@ -103,24 +103,3 @@ def test_loss_oracle_matches_reference_losses(golden_dir):
     total, comps = L.combined_loss(a, b, L.STAGE_WEIGHTS[3])
     want = sum(L.STAGE_WEIGHTS[3][k] * float(d[k]) for k in L.STAGE_WEIGHTS[3])
     assert abs(float(total) - want) <= 1e-6 and set(comps) == {"l1", "swt", "fft", "ssim"}
-
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference checkout only exists in the build container")
-def test_metric_oracle_matches_reference_metrics():
-    """oracle metric_psnr / metric_ssim against the reference's own src/utils/metrics.py (imported in a subprocess
-    so that its `src` package does not shadow anything here)."""
-    import subprocess
-    import sys
-    code = (
-        "import sys, torch; sys.path.insert(0, '/root/reference'); sys.path.insert(0, %r);"
-        "from src.utils import metrics as M; from oracle import loss_oracle as L;"
-        "g = torch.Generator().manual_seed(3); a = torch.rand(2, 3, 40, 56, generator=g);"
-        "b = (a + 0.05 * torch.randn(2, 3, 40, 56, generator=g)).clamp(0, 1);"
-        "ok = True\n"
-        "for crop, y in ((0, False), (4, True), (4, False)):\n"
-        "    ok &= abs(M.calculate_psnr(a, b, crop, y) - L.metric_psnr(a, b, crop, y)) < 1e-4\n"
-        "    ok &= abs(M.calculate_ssim(a[0], b[0], crop, y) - L.metric_ssim(a[0], b[0], crop, y)) < 1e-5\n"
-        "print('ok' if ok else 'MISMATCH')"
-    ) % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and r.stdout.strip().endswith("ok"), (r.stdout[-500:], r.stderr[-1500:])

@@ -3,8 +3,8 @@ eval.py -- ~1.5 MB) from /root/reference into baseline/_ref/, which is git-ignor
 history) but NOT gpurun-ignored, so it travels to the GPU box.  Used there, and only there, as a measured baseline and as
 the caller side of the drop-in boundary:
   * bench.py --impl reference        : the reference module's own CPU forward (kind "reference");
-  * bench.py gpu_eager_baseline      : the reference module in PyTorch eager on the same GPU;
-  * tests/test_gpu_reference_scripts.py : the reference's own scripts running against the installed sm_100a module.
+  * bench.py gpu_eager_baseline      : the reference module in PyTorch eager on the same GPU.
+Nothing in tests/ reads it: the drop-in boundary tests use oracle/reference_layout.py.
 Nothing under image-super-resolution_b200/ imports it.      python tools/install_reference.py [src_root] [dst]
 """
 import os
