@@ -122,21 +122,28 @@ PROTOTYPES = {
     "ffsr_cast_f32_to_bf16": (_I, [_P, _P, _L, _P]),
     "ffsr_final_combine": (_I, [_P, _LL, _P, _P, _P, _P, _I, _I, _I, _I, _P, _P]),
     # ---- train-mode / backward ----
-    "ffsr_conv2d_wgrad": (_I, [C.POINTER(WgradParams), _P]),
+    "ffsr_conv2d_wgrad_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I, _I]),
+    "ffsr_conv2d_wgrad": (_I, [C.POINTER(WgradParams), _P, _SZ, _P]),
     "ffsr_wgrad_params_size": (_SZ, []),
-    "ffsr_colsum": (_I, [_P, _I, _I, _I, _I, _I, _LL, _LL, _LL, _P, _P]),
+    "ffsr_colsum_workspace_bytes": (_SZ, [_I, _I, _I, _I]),
+    "ffsr_colsum": (_I, [_P, _I, _I, _I, _I, _I, _LL, _LL, _LL, _P, _P, _SZ, _P]),
     "ffsr_act_forward": (_I, [_P, _P, _L, _I, _I, _P]),
     "ffsr_act_backward": (_I, [_P, _P, _P, _L, _I, _I, _P]),
-    "ffsr_layernorm_backward": (_I, [_P, _P, _L, _I, _P, _P, _P, _P, _P]),
-    "ffsr_bn_stats": (_I, [_P, _I, _L, _I, _P, _P, _P]),
+    "ffsr_layernorm_backward_workspace_bytes": (_SZ, [_L, _I]),
+    "ffsr_layernorm_backward": (_I, [_P, _P, _L, _I, _P, _P, _P, _P, _P, _SZ, _P]),
+    "ffsr_bn_stats_workspace_bytes": (_SZ, [_I, _L, _I]),
+    "ffsr_bn_stats": (_I, [_P, _I, _L, _I, _P, _P, _P, _SZ, _P]),
     "ffsr_bn_apply": (_I, [_P, _I, _L, _I, _P, _P, _P, _P, _P, _P]),
-    "ffsr_bn_backward": (_I, [_P, _P, _I, _L, _I, _P, _P, _P, _P, _P, _P, _P]),
+    "ffsr_bn_backward_workspace_bytes": (_SZ, [_I, _L, _I]),
+    "ffsr_bn_backward": (_I, [_P, _P, _I, _L, _I, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "ffsr_token_attention_train": (_I, [_P, _I, _I, _L, _I, _P, _P, _F, _U64, _P, _P]),
     "ffsr_token_attention_backward": (_I, [_P, _P, _P, _I, _I, _L, _I, _P, _P, _F, _U64, _P, _P]),
     "ffsr_dwconv_stage": (_I, [_P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
-    "ffsr_dwconv_wgrad": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P]),
+    "ffsr_dwconv_wgrad_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I]),
+    "ffsr_dwconv_wgrad": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P, _SZ, _P]),
     # ---- fused losses ----
-    "ffsr_loss_l1": (_I, [_P, _P, _L, _F, _P, _P, _P]),
+    "ffsr_loss_l1_workspace_bytes": (_SZ, [_L]),
+    "ffsr_loss_l1": (_I, [_P, _P, _L, _F, _P, _P, _SZ, _P, _P]),
     "ffsr_loss_swt_workspace_bytes": (_SZ, [_I, _I, _I]),
     "ffsr_loss_swt": (_I, [_P, _P, _I, _I, _I, _F, _P, _P, _SZ, _P, _P]),
     "ffsr_loss_ssim_workspace_bytes": (_SZ, [_I, _I, _I]),
@@ -152,7 +159,8 @@ PROTOTYPES = {
     "ffsr_gate_mul_forward": (_I, [_P, _P, _L, _I, _P, _I, _P]),
     "ffsr_gate_mul_backward": (_I, [_P, _P, _P, _L, _I, _P, _P, _I, _P]),
     "ffsr_axpby_forward": (_I, [_P, _P, _P, _L, _P, _P, _L, _I, _P, _I, _P]),
-    "ffsr_axpby_backward": (_I, [_P, _P, _P, _L, _P, _P, _L, _I, _P, _P, _P, _I, _P]),
+    "ffsr_axpby_backward_workspace_bytes": (_SZ, [_L, _I]),
+    "ffsr_axpby_backward": (_I, [_P, _P, _P, _L, _P, _P, _L, _I, _P, _P, _P, _P, _SZ, _I, _P]),
     "ffsr_fft_lowpass_workspace_bytes": (_SZ, [_I, _I, _I]),
     "ffsr_fft_lowpass": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, _SZ, _P, _P]),
     "ffsr_fft_lowpass_backward": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _SZ, _P, _P]),
@@ -170,7 +178,8 @@ PROTOTYPES = {
     "ffsr_cache_unpack": (_I, [_P, _SZ, _I, _P, _I, _P, _I, _P]),
     "ffsr_cache_segment_size": (_I, []),
     # ---- fused optimizer ----
-    "ffsr_sumsq": (_I, [_P, _L, _P, _P]),
+    "ffsr_sumsq_workspace_bytes": (_SZ, [_L]),
+    "ffsr_sumsq": (_I, [_P, _L, _P, _P, _SZ, _P]),
     "ffsr_adamw_ema_step": (_I, [_P, _P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _I, _P, _P, _P, _F, _F, _F, _P]),
 }
 

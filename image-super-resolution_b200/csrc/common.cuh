@@ -24,6 +24,73 @@ int ffsr_check_launch(const char* what);
 
 static inline int ceil_div(long a, long b) { return (int)((a + b - 1) / b); }
 
+// Fixed-order cross-block reduction of the training kernels.  A partial kernel partitions its work by shape
+// alone and writes one slot per block, slots[k][0..L), each entry of each slot exactly once (no atomics);
+// k_sum_slots then adds sum_k slots[k][i] to out[i] (entries i >= L1 go to out2[i - L1]).  One 1024-thread block
+// per 32 entries: thread (x = tid % 32, y = tid / 32) sums slots y, y+32, ... of entry x in order and row y == 0
+// adds the 32 group sums in order, so the result depends on (nslots, L) only, never on block scheduling: training
+// steps are bitwise reproducible.  Outputs keep their accumulate-into semantics.  One launch can finish two
+// independent reductions (a weight gradient and its bias sums).
+template <typename T>
+struct SlotSum {
+  const T* slots;
+  int nslots;
+  long L, L1;
+  T* out;
+  T* out2;
+};
+template <typename T>
+inline SlotSum<T> slot_sum(const T* slots, int nslots, long L, T* out, T* out2 = nullptr, long L1 = -1) {
+  return SlotSum<T>{slots, nslots, L, L1 < 0 ? L : L1, out, out2};
+}
+template <typename T>
+__host__ __device__ inline long slot_sum_blocks(const SlotSum<T>& j) { return j.slots ? (j.L + 31) / 32 : 0; }
+
+// the 32 entries [32*chunk, 32*chunk + 32) of j; every thread of a 1024-thread block calls it
+template <typename T>
+__device__ __forceinline__ void sum_slots_chunk(const SlotSum<T>& j, long chunk) {
+  __shared__ T sh[32][33];
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  const long i = chunk * 32 + tx;
+  T s = 0;
+  if (i < j.L) {
+#pragma unroll 4
+    for (int k = ty; k < j.nslots; k += 32) s += j.slots[(long)k * j.L + i];
+  }
+  sh[ty][tx] = s;
+  __syncthreads();
+  if (ty == 0 && i < j.L) {
+    T t = 0;
+    for (int g = 0; g < 32; ++g) t += sh[g][tx];
+    if (i < j.L1) j.out[i] += t;
+    else j.out2[i - j.L1] += t;
+  }
+}
+
+template <typename T>
+__global__ void __launch_bounds__(1024) k_sum_slots(const SlotSum<T> a, const SlotSum<T> b) {
+  const long na = slot_sum_blocks(a);
+  if ((long)blockIdx.x < na) sum_slots_chunk(a, blockIdx.x);
+  else sum_slots_chunk(b, blockIdx.x - na);
+}
+
+template <typename T>
+static inline void launch_sum_slots(const SlotSum<T>& a, const SlotSum<T>& b, cudaStream_t stream) {
+  k_sum_slots<T><<<(unsigned)(slot_sum_blocks(a) + slot_sum_blocks(b)), 1024, 0, stream>>>(a, b);
+}
+template <typename T>
+static inline void launch_sum_slots(const T* slots, int nslots, long L, T* out, cudaStream_t stream, T* out2 = nullptr,
+                                    long L1 = -1) {
+  launch_sum_slots<T>(slot_sum(slots, nslots, L, out, out2, L1), SlotSum<T>{}, stream);
+}
+
+// bias sums of the weight-gradient entry points: column-sum partials [nslots][C] of ffsr_colsum into part
+// (ffsr_colsum_workspace_bytes), finished by the caller's k_sum_slots launch
+int colsum_partials(const void* v, int dtype, int N, int H, int W, int C, long long sN, long long sY, long long sX,
+                    float* part, int* nslots, cudaStream_t stream);
+// partial slots placed after `bytes` of other scratch in one workspace
+inline size_t ws_align(size_t bytes) { return (bytes + 255) / 256 * 256; }
+
 // activation codes shared with the host side
 enum { ACT_NONE = 0, ACT_GELU = 1, ACT_RELU = 2, ACT_SIGMOID = 3 };
 

@@ -326,19 +326,36 @@ extern "C" int ffsr_dwconv_stage(const float* in, int N, int H, int W, int C, in
 namespace {
 constexpr int WG_R = 8;    // outputs per thread along the conv axis in the 21-tap weight-gradient kernel
 
-// AXIS 0: taps along W, AXIS 1: taps along H.  blockDim = (channels, items); each thread owns one
-// channel and WG_R consecutive outputs; per-block partial sums in shared memory, then global atomics.
+// Both weight-gradient kernels: blockDim = (channels, item rows); grid = (channel blocks, Y, images), and
+// thread row ty of block y takes items y*blockDim.y + ty, stepping by Y*blockDim.y, summing in registers.
+// The rows of a block are summed in order in shared memory and the block's [channels][taps] partial goes to
+// slot (n*Y + y) of part [N*Y][C][taps], reduced in slot order by k_sum_slots: no atomics, bitwise reproducible.
+template <int TAPS>
+__device__ __forceinline__ void dw_wgrad_store(const float (&acc)[TAPS], int C, float* sdw, float* __restrict__ part) {
+  const int tl = threadIdx.y * blockDim.x + threadIdx.x;
+  const int CB = blockDim.x * TAPS;
+#pragma unroll
+  for (int t = 0; t < TAPS; ++t) sdw[(threadIdx.y * blockDim.x + threadIdx.x) * TAPS + t] = acc[t];
+  __syncthreads();
+  float* slot = part + ((long)blockIdx.z * gridDim.y + blockIdx.y) * C * TAPS + (long)blockIdx.x * CB;
+  for (int i = tl; i < CB; i += blockDim.x * blockDim.y) {
+    float s = 0.f;
+    for (int r = 0; r < (int)blockDim.y; ++r) s += sdw[r * CB + i];
+    slot[i] = s;
+  }
+}
+
+// AXIS 0: taps along W, AXIS 1: taps along H.  Each thread owns one channel and WG_R consecutive outputs per item.
 template <int AXIS>
 __global__ void __launch_bounds__(256) k_dw21_wgrad(const float* __restrict__ in, const float* __restrict__ g, int H,
-                                                    int W, int C, long items, float* __restrict__ dw) {
-  extern __shared__ float sdw[];            // [blockDim.x][21]
-  const int tl = threadIdx.y * blockDim.x + threadIdx.x;
-  for (int i = tl; i < blockDim.x * 21; i += blockDim.x * blockDim.y) sdw[i] = 0.f;
-  __syncthreads();
+                                                    int W, int C, long items, float* __restrict__ part) {
+  extern __shared__ float sdw[];            // [blockDim.y][blockDim.x][21]
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   const int n = blockIdx.z;
-  const long idx = (long)blockIdx.y * blockDim.y + threadIdx.y;
-  if (c < C && idx < items) {
+  float acc[21];
+#pragma unroll
+  for (int t = 0; t < 21; ++t) acc[t] = 0.f;
+  for (long idx = (long)blockIdx.y * blockDim.y + threadIdx.y; c < C && idx < items; idx += (long)gridDim.y * blockDim.y) {
     int y, x;
     if (AXIS == 0) {
       const int runs = (W + WG_R - 1) / WG_R;
@@ -371,26 +388,21 @@ __global__ void __launch_bounds__(256) k_dw21_wgrad(const float* __restrict__ in
       float a = 0.f;
 #pragma unroll
       for (int r = 0; r < WG_R; ++r) a = fmaf(v[r + t], gr[r], a);
-      atomicAdd(&sdw[threadIdx.x * 21 + t], a);
+      acc[t] += a;
     }
   }
-  __syncthreads();
-  for (int i = tl; i < blockDim.x * 21; i += blockDim.x * blockDim.y) {
-    const int cc = blockIdx.x * blockDim.x + i / 21;
-    if (cc < C) atomicAdd(dw + (long)cc * 21 + i % 21, sdw[i]);
-  }
+  dw_wgrad_store<21>(acc, C, sdw, part);
 }
 
 __global__ void __launch_bounds__(256) k_dw5_wgrad(const float* __restrict__ in, const float* __restrict__ g, int H,
-                                                   int W, int C, long items, float* __restrict__ dw) {
-  extern __shared__ float sdw[];            // [blockDim.x][25]
-  const int tl = threadIdx.y * blockDim.x + threadIdx.x;
-  for (int i = tl; i < blockDim.x * 25; i += blockDim.x * blockDim.y) sdw[i] = 0.f;
-  __syncthreads();
+                                                   int W, int C, long items, float* __restrict__ part) {
+  extern __shared__ float sdw[];            // [blockDim.y][blockDim.x][25]
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   const int n = blockIdx.z;
-  const long idx = (long)blockIdx.y * blockDim.y + threadIdx.y;
-  if (c < C && idx < items) {
+  float acc[25];
+#pragma unroll
+  for (int i = 0; i < 25; ++i) acc[i] = 0.f;
+  for (long idx = (long)blockIdx.y * blockDim.y + threadIdx.y; c < C && idx < items; idx += (long)gridDim.y * blockDim.y) {
     const int runs_x = (W + R5 - 1) / R5;
     const int y0 = (int)(idx / runs_x) * R5, x0 = (int)(idx % runs_x) * R5;
     const float* img = in + (long)n * H * W * C;
@@ -401,9 +413,6 @@ __global__ void __launch_bounds__(256) k_dw5_wgrad(const float* __restrict__ in,
 #pragma unroll
       for (int b = 0; b < R5; ++b)
         gr[a][b] = (y0 + a < H && x0 + b < W) ? gim[((long)(y0 + a) * W + x0 + b) * C + c] : 0.f;
-    float acc[25];
-#pragma unroll
-    for (int i = 0; i < 25; ++i) acc[i] = 0.f;
 #pragma unroll
     for (int iy = 0; iy < R5 + 4; ++iy) {
       const int yy = y0 + iy - 2;
@@ -423,37 +432,49 @@ __global__ void __launch_bounds__(256) k_dw5_wgrad(const float* __restrict__ in,
           for (int dx = 0; dx < 5; ++dx) acc[dy * 5 + dx] = fmaf(v[b + dx], gr[a][b], acc[dy * 5 + dx]);
       }
     }
-#pragma unroll
-    for (int i = 0; i < 25; ++i) atomicAdd(&sdw[threadIdx.x * 25 + i], acc[i]);
   }
-  __syncthreads();
-  for (int i = tl; i < blockDim.x * 25; i += blockDim.x * blockDim.y) {
-    const int cc = blockIdx.x * blockDim.x + i / 25;
-    if (cc < C) atomicAdd(dw + (long)cc * 25 + i % 25, sdw[i]);
-  }
+  dw_wgrad_store<25>(acc, C, sdw, part);
+}
+
+constexpr int DWG_CX = 32, DWG_TY = 8;
+
+// items of one image and the item-row blocks Y per image (about 8 blocks per SM over the whole grid)
+inline long dw_wgrad_items(int H, int W, int kind) {
+  if (kind == 0) return (long)ceil_div(H, R5) * ceil_div(W, R5);
+  if (kind == 1) return (long)H * ceil_div(W, WG_R);
+  return (long)ceil_div(H, WG_R) * W;
+}
+inline int dw_wgrad_Y(int N, int H, int W, int C, int kind) {
+  const long rows = ceil_div(dw_wgrad_items(H, W, kind), DWG_TY);
+  long Y = (148L * 8) / ((long)(C / DWG_CX) * N);
+  if (Y > rows) Y = rows;
+  return Y < 1 ? 1 : (int)Y;
 }
 }  // namespace
 
+extern "C" size_t ffsr_dwconv_wgrad_workspace_bytes(int N, int H, int W, int C, int kind) {
+  if (N <= 0 || H <= 0 || W <= 0 || C <= 0 || C % DWG_CX != 0 || kind < 0 || kind > 2) return 0;
+  return (size_t)N * dw_wgrad_Y(N, H, W, C, kind) * C * (kind == 0 ? 25 : 21) * sizeof(float);
+}
+
 // dw: [C][taps] fp32, ACCUMULATED into (caller zeroes)
 extern "C" int ffsr_dwconv_wgrad(const float* in, const float* g, int N, int H, int W, int C, int kind, float* dw,
-                                 cudaStream_t stream) {
-  FFSR_REQUIRE(in && g && dw, FFSR_ERR_ARG, "dwconv_wgrad: null pointer");
+                                 void* ws, size_t ws_bytes, cudaStream_t stream) {
+  FFSR_REQUIRE(in && g && dw && ws, FFSR_ERR_ARG, "dwconv_wgrad: null pointer");
   FFSR_REQUIRE(N > 0 && N <= 65535 && H > 0 && W > 0 && C > 0 && C % 32 == 0, FFSR_ERR_ARG, "dwconv_wgrad: bad shape");
   FFSR_REQUIRE(kind >= 0 && kind <= 2, FFSR_ERR_ARG, "dwconv_wgrad: kind must be 0, 1 or 2");
-  const int cx = 32, ty = 8;
-  dim3 block(cx, ty);
-  if (kind == 0) {
-    const long items = (long)ceil_div(H, R5) * ceil_div(W, R5);
-    dim3 grid(C / cx, ceil_div(items, ty), N);
-    k_dw5_wgrad<<<grid, block, cx * 25 * sizeof(float), stream>>>(in, g, H, W, C, items, dw);
-  } else if (kind == 1) {
-    const long items = (long)H * ceil_div(W, WG_R);
-    dim3 grid(C / cx, ceil_div(items, ty), N);
-    k_dw21_wgrad<0><<<grid, block, cx * 21 * sizeof(float), stream>>>(in, g, H, W, C, items, dw);
-  } else {
-    const long items = (long)ceil_div(H, WG_R) * W;
-    dim3 grid(C / cx, ceil_div(items, ty), N);
-    k_dw21_wgrad<1><<<grid, block, cx * 21 * sizeof(float), stream>>>(in, g, H, W, C, items, dw);
-  }
-  return ffsr_check_launch("dwconv_wgrad");
+  FFSR_REQUIRE(ws_bytes >= ffsr_dwconv_wgrad_workspace_bytes(N, H, W, C, kind), FFSR_ERR_ARG, "dwconv_wgrad: workspace too small");
+  const int Y = dw_wgrad_Y(N, H, W, C, kind);
+  const long items = dw_wgrad_items(H, W, kind);
+  const int taps = kind == 0 ? 25 : 21;
+  dim3 block(DWG_CX, DWG_TY), grid(C / DWG_CX, Y, N);
+  const size_t smem = (size_t)DWG_CX * DWG_TY * taps * sizeof(float);
+  float* part = (float*)ws;
+  if (kind == 0) k_dw5_wgrad<<<grid, block, smem, stream>>>(in, g, H, W, C, items, part);
+  else if (kind == 1) k_dw21_wgrad<0><<<grid, block, smem, stream>>>(in, g, H, W, C, items, part);
+  else k_dw21_wgrad<1><<<grid, block, smem, stream>>>(in, g, H, W, C, items, part);
+  const int rc = ffsr_check_launch("dwconv_wgrad");
+  if (rc) return rc;
+  launch_sum_slots<float>(part, N * Y, (long)C * taps, dw, stream);
+  return ffsr_check_launch("dwconv_wgrad_reduce");
 }

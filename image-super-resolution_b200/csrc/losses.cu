@@ -1,6 +1,8 @@
 // Fused stage-2/3 training losses with their backward passes (SURVEY 8a rows L-L1, L-SWT, L-FFT, L-SSIM):
 // each entry point accumulates the loss partial sums (fp64) AND adds  weight * dLoss/dPred  into `dpred`
-// in the same pass over the data, so loss.backward() costs nothing extra.
+// in the same pass over the data, so loss.backward() costs nothing extra.  Each block writes its fp64 partial
+// sums to a slot of the workspace and k_sum_slots adds them in slot order: the loss values are bitwise
+// reproducible (no atomics).
 //   L1    src/losses/perceptual_loss.py:86-104
 //   SSIM  src/losses/perceptual_loss.py:225-291   (11x11 Gaussian sigma 1.5, zero pad 5, C1=1e-4, C2=9e-4)
 //   FFT   src/losses/perceptual_loss.py:533-598   (fft2 ortho, |mag| + 0.1 |phase| L1, radial weights)
@@ -15,8 +17,9 @@ namespace {
 
 __device__ __forceinline__ float sgn(float v) { return (float)((v > 0.f) - (v < 0.f)); }
 
+// block sum of v -> part[linear block index][0..NV)
 template <int NV>
-__device__ __forceinline__ void block_sum_atomic(double (&v)[NV], double* out) {
+__device__ __forceinline__ void block_sum_slot(double (&v)[NV], double* part) {
   __shared__ double sh[NV][32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
 #pragma unroll
@@ -32,7 +35,7 @@ __device__ __forceinline__ void block_sum_atomic(double (&v)[NV], double* out) {
       double s = lane < nw ? sh[i][lane] : 0.0;
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
-      if (lane == 0) atomicAdd(out + i, s);
+      if (lane == 0) part[((long)(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * NV + i] = s;
     }
   }
 }
@@ -50,7 +53,7 @@ __global__ void __launch_bounds__(256) k_loss_l1(const float* __restrict__ p, co
     if (++cnt == 32) { acc[0] += f; f = 0.f; cnt = 0; }
   }
   acc[0] += f;
-  block_sum_atomic<1>(acc, sum);
+  block_sum_slot<1>(acc, sum);
 }
 
 // ------------------------------------------------------------------------------------ SWT
@@ -102,7 +105,7 @@ __global__ void __launch_bounds__(256) k_swt_level(const float* __restrict__ a, 
   if (sums) {
 #pragma unroll
     for (int k = 0; k < 4; ++k) acc[k] += fa[k];
-    block_sum_atomic<4>(acc, sums);
+    block_sum_slot<4>(acc, sums);
   }
 }
 
@@ -187,7 +190,7 @@ __global__ void __launch_bounds__(256) k_ssim_fwd(const float* __restrict__ X, c
     D[2 * total + o] = gs * (2.f * A1 * inv);
   }
   acc[0] = f;
-  block_sum_atomic<1>(acc, sum);
+  block_sum_slot<1>(acc, sum);
 }
 
 __global__ void __launch_bounds__(256) k_ssim_bwd(const float* __restrict__ X, const float* __restrict__ Y, int H, int W,
@@ -406,7 +409,7 @@ __global__ void __launch_bounds__(256) k_fft_spectrum(const float2* __restrict__
     G[idx] = make_float2(ga, gb);
   }
   acc[0] += fm; acc[1] += fp;
-  block_sum_atomic<2>(acc, sums);
+  block_sum_slot<2>(acc, sums);
 }
 
 bool factorize(int n, Radices& rad) {
@@ -419,16 +422,32 @@ bool factorize(int n, Radices& rad) {
 }
 
 inline int ew_grid(long n) { return (int)((n + 255) / 256 < 148L * 16 ? (n + 255) / 256 : 148L * 16); }
+
+// the partial-sum slots follow the entry point's own scratch in the workspace
+constexpr size_t LOSS_PART_ALIGN = 256;
+inline size_t part_offset(size_t scratch) { return (scratch + LOSS_PART_ALIGN - 1) / LOSS_PART_ALIGN * LOSS_PART_ALIGN; }
+inline double* part_ptr(void* ws, size_t scratch) { return (double*)((char*)ws + part_offset(scratch)); }
+inline long ssim_blocks(int P, int H, int W) { return (long)ceil_div(W, ST) * ceil_div(H, ST) * P; }
 }  // namespace
 
-extern "C" int ffsr_loss_l1(const float* pred, const float* target, long n, float gscale, double* sum, float* dpred,
-                            cudaStream_t stream) {
-  FFSR_REQUIRE(pred && target && sum && dpred && n > 0, FFSR_ERR_ARG, "loss_l1: bad argument");
-  k_loss_l1<<<ew_grid(n), 256, 0, stream>>>(pred, target, n, gscale, sum, dpred);
-  return ffsr_check_launch("loss_l1");
+extern "C" size_t ffsr_loss_l1_workspace_bytes(long n) { return n > 0 ? (size_t)ew_grid(n) * sizeof(double) : 0; }
+
+extern "C" int ffsr_loss_l1(const float* pred, const float* target, long n, float gscale, double* sum, void* ws,
+                            size_t ws_bytes, float* dpred, cudaStream_t stream) {
+  FFSR_REQUIRE(pred && target && sum && ws && dpred && n > 0, FFSR_ERR_ARG, "loss_l1: bad argument");
+  FFSR_REQUIRE(ws_bytes >= ffsr_loss_l1_workspace_bytes(n), FFSR_ERR_ARG, "loss_l1: workspace too small");
+  const int grid = ew_grid(n);
+  k_loss_l1<<<grid, 256, 0, stream>>>(pred, target, n, gscale, (double*)ws, dpred);
+  const int rc = ffsr_check_launch("loss_l1");
+  if (rc) return rc;
+  launch_sum_slots<double>((const double*)ws, grid, 1, sum, stream);
+  return ffsr_check_launch("loss_l1_reduce");
 }
 
-extern "C" size_t ffsr_loss_swt_workspace_bytes(int P, int H, int W) { return (size_t)6 * P * H * W * sizeof(float); }
+extern "C" size_t ffsr_loss_swt_workspace_bytes(int P, int H, int W) {
+  const long total = (long)P * H * W;
+  return part_offset((size_t)6 * total * sizeof(float)) + (size_t)ew_grid(total) * 4 * sizeof(double);
+}
 
 extern "C" int ffsr_loss_swt(const float* pred, const float* target, int P, int H, int W, float gscale, double* sums8,
                              void* ws, size_t ws_bytes, float* dpred, cudaStream_t stream) {
@@ -440,16 +459,21 @@ extern "C" int ffsr_loss_swt(const float* pred, const float* target, int P, int 
   float* gA0 = A0 + total;
   float* G = gA0 + total;
   const int grid = ew_grid(total);
+  double* part = part_ptr(ws, (size_t)6 * total * sizeof(float));
   // level 0: approximation + sums;  level 1: sums + tap gradients;  adjoint to dA0;  level 0 again with dA0;  adjoint
-  k_swt_level<<<grid, 256, 0, stream>>>(pred, target, total, H, W, 1, A0, nullptr, gscale, sums8, nullptr);
-  k_swt_level<<<grid, 256, 0, stream>>>(A0, nullptr, total, H, W, 2, nullptr, nullptr, gscale, sums8 + 4, G);
+  k_swt_level<<<grid, 256, 0, stream>>>(pred, target, total, H, W, 1, A0, nullptr, gscale, part, nullptr);
+  launch_sum_slots<double>(part, grid, 4, sums8, stream);
+  k_swt_level<<<grid, 256, 0, stream>>>(A0, nullptr, total, H, W, 2, nullptr, nullptr, gscale, part, G);
+  launch_sum_slots<double>(part, grid, 4, sums8 + 4, stream);
   k_swt_gather<<<grid, 256, 0, stream>>>(G, total, H, W, 2, gA0, 0);
   k_swt_level<<<grid, 256, 0, stream>>>(pred, target, total, H, W, 1, nullptr, gA0, gscale, nullptr, G);
   k_swt_gather<<<grid, 256, 0, stream>>>(G, total, H, W, 1, dpred, 1);
   return ffsr_check_launch("loss_swt");
 }
 
-extern "C" size_t ffsr_loss_ssim_workspace_bytes(int P, int H, int W) { return (size_t)3 * P * H * W * sizeof(float); }
+extern "C" size_t ffsr_loss_ssim_workspace_bytes(int P, int H, int W) {
+  return part_offset((size_t)3 * P * H * W * sizeof(float)) + (size_t)ssim_blocks(P, H, W) * sizeof(double);
+}
 
 extern "C" int ffsr_loss_ssim(const float* pred, const float* target, int P, int H, int W, float gscale, double* sum,
                               void* ws, size_t ws_bytes, float* dpred, cudaStream_t stream) {
@@ -462,12 +486,17 @@ extern "C" int ffsr_loss_ssim(const float* pred, const float* target, int P, int
   const long total = (long)P * H * W;
   dim3 grid(ceil_div(W, ST), ceil_div(H, ST), P);
   // loss = 1 - mean(S): dLoss/dS = -1/n, the caller's gscale carries weight/n
-  k_ssim_fwd<<<grid, 256, 0, stream>>>(pred, target, H, W, gw, -gscale, sum, (float*)ws, total);
+  double* part = part_ptr(ws, (size_t)3 * total * sizeof(float));
+  k_ssim_fwd<<<grid, 256, 0, stream>>>(pred, target, H, W, gw, -gscale, part, (float*)ws, total);
+  launch_sum_slots<double>(part, (int)ssim_blocks(P, H, W), 1, sum, stream);
   k_ssim_bwd<<<grid, 256, 0, stream>>>(pred, target, H, W, gw, (const float*)ws, total, dpred);
   return ffsr_check_launch("loss_ssim");
 }
 
-extern "C" size_t ffsr_loss_fft_workspace_bytes(int P, int H, int W) { return (size_t)2 * P * H * W * sizeof(float2); }
+extern "C" size_t ffsr_loss_fft_workspace_bytes(int P, int H, int W) {
+  const long total = (long)P * H * W;
+  return part_offset((size_t)2 * total * sizeof(float2)) + (size_t)ew_grid(total) * 2 * sizeof(double);
+}
 
 extern "C" int ffsr_loss_fft(const float* pred, const float* target, int P, int H, int W, float gscale, double* sums2,
                              void* ws, size_t ws_bytes, float* dpred, cudaStream_t stream) {
@@ -496,7 +525,9 @@ extern "C" int ffsr_loss_fft(const float* pred, const float* target, int P, int 
   k_fft_rows<0><<<(unsigned)ceil_div(nrows, FFT_ROWS), 256, sm_rows, stream>>>(pred, target, Z, nrows, W, rw, sc_w, nullptr);
   dim3 cgrid(ceil_div(W, FFT_ROWS), P);
   k_fft_cols<<<cgrid, 256, sm_cols, stream>>>(Z, H, W, rh, -1.f, sc_h);
-  k_fft_spectrum<<<ew_grid(total), 256, 0, stream>>>(Z, total, H, W, gscale, sums2, G);
+  double* part = part_ptr(ws, (size_t)2 * total * sizeof(float2));
+  k_fft_spectrum<<<ew_grid(total), 256, 0, stream>>>(Z, total, H, W, gscale, part, G);
+  launch_sum_slots<double>(part, ew_grid(total), 2, sums2, stream);
   k_fft_cols<<<cgrid, 256, sm_cols, stream>>>(G, H, W, rh, 1.f, sc_h);
   k_fft_rows<1><<<(unsigned)ceil_div(nrows, FFT_ROWS), 256, sm_rows, stream>>>(nullptr, nullptr, G, nrows, W, rw, sc_w, dpred);
   return ffsr_check_launch("loss_fft");

@@ -9,7 +9,8 @@
 #include "../../include/ffsr_b200.h"
 
 namespace {
-__global__ void __launch_bounds__(256) k_sumsq(const float* __restrict__ g, long n, double* __restrict__ out) {
+// block sums of g^2 -> part[blockIdx.x], added in block order by k_sum_slots (bitwise reproducible clip coefficient)
+__global__ void __launch_bounds__(256) k_sumsq(const float* __restrict__ g, long n, double* __restrict__ part) {
   __shared__ double sh[8];
   double acc = 0.0;
   float f = 0.f;
@@ -26,7 +27,7 @@ __global__ void __launch_bounds__(256) k_sumsq(const float* __restrict__ g, long
   if (threadIdx.x == 0) {
     double s = 0.0;
     for (int i = 0; i < 8; ++i) s += sh[i];
-    atomicAdd(out, s);
+    part[blockIdx.x] = s;
   }
 }
 
@@ -60,11 +61,19 @@ __global__ void __launch_bounds__(256) k_adamw_ema(float* __restrict__ p, const 
 }
 }  // namespace
 
-extern "C" int ffsr_sumsq(const float* g, long n, double* out, cudaStream_t stream) {
-  FFSR_REQUIRE(g && out && n > 0, FFSR_ERR_ARG, "sumsq: bad argument");
-  const int grid = (int)((n + 255) / 256 < 148L * 4 ? (n + 255) / 256 : 148L * 4);
-  k_sumsq<<<grid, 256, 0, stream>>>(g, n, out);
-  return ffsr_check_launch("sumsq");
+static inline int sumsq_grid(long n) { return (int)((n + 255) / 256 < 148L * 4 ? (n + 255) / 256 : 148L * 4); }
+
+extern "C" size_t ffsr_sumsq_workspace_bytes(long n) { return n > 0 ? (size_t)sumsq_grid(n) * sizeof(double) : 0; }
+
+extern "C" int ffsr_sumsq(const float* g, long n, double* out, void* ws, size_t ws_bytes, cudaStream_t stream) {
+  FFSR_REQUIRE(g && out && ws && n > 0, FFSR_ERR_ARG, "sumsq: bad argument");
+  FFSR_REQUIRE(ws_bytes >= ffsr_sumsq_workspace_bytes(n), FFSR_ERR_ARG, "sumsq: workspace too small");
+  const int grid = sumsq_grid(n);
+  k_sumsq<<<grid, 256, 0, stream>>>(g, n, (double*)ws);
+  const int rc = ffsr_check_launch("sumsq");
+  if (rc) return rc;
+  launch_sum_slots<double>((const double*)ws, grid, 1, out, stream);
+  return ffsr_check_launch("sumsq_reduce");
 }
 
 extern "C" int ffsr_adamw_ema_step(float* p, const float* g, float* m, float* v, float* ema, long n, float lr,

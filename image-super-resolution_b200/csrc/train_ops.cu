@@ -86,7 +86,7 @@ __device__ __forceinline__ int frag_index(int t, int j) {
 }
 
 template <int TM, int TN>
-__global__ void __launch_bounds__(256) k_conv_wgrad(const ffsr_wgrad_params p, long chunk) {
+__global__ void __launch_bounds__(256) k_conv_wgrad(const ffsr_wgrad_params p, long chunk, float* __restrict__ part) {
   constexpr int MI = TM / 16, NI = TN / 16;
   __shared__ __align__(16) float sX[WG_KP][TM];
   __shared__ __align__(16) float sD[WG_KP][TN];
@@ -159,34 +159,49 @@ __global__ void __launch_bounds__(256) k_conv_wgrad(const ffsr_wgrad_params p, l
 #pragma unroll
     for (int j = 0; j < NI; ++j) {
       const int co = co0 + frag_index<NI>(tx, j);
-      if (co < p.Cout) atomicAdd(p.dw + ((long)tap * p.Cin + ci) * p.Cout + co, acc[i][j]);
+      if (co < p.Cout) part[(((long)blockIdx.x * gridDim.y + tap) * p.Cin + ci) * p.Cout + co] = acc[i][j];
     }
   }
 }
 
-template <int TM, int TN>
-int launch_wgrad(const ffsr_wgrad_params& p, cudaStream_t stream) {
-  const int taps = p.ksize * p.ksize;
-  const int tiles = ceil_div(p.Cin, TM) * ceil_div(p.Cout, TN);
-  const long NP = (long)p.N * p.H * p.W;
+// register tile of the weight-gradient kernel and its pixel split P (chunk pixels per block): a function of the shape
+struct WgradPlan {
+  int TM, TN;
+  long P, chunk;
+};
+inline WgradPlan wgrad_plan(int N, int H, int W, int Cin, int Cout, int ksize) {
+  WgradPlan pl;
+  pl.TM = Cin > 64 ? 128 : Cin > 32 ? 64 : Cin > 16 ? 32 : 16;
+  pl.TN = Cout > 64 ? 128 : Cout > 32 ? 64 : Cout > 16 ? 32 : 16;
+  const int taps = ksize * ksize;
+  const int tiles = ceil_div(Cin, pl.TM) * ceil_div(Cout, pl.TN);
+  const long NP = (long)N * H * W;
   long P = ceil_div(148 * 6, taps * tiles);
   const long maxP = (NP + 511) / 512;
   if (P > maxP) P = maxP;
   if (P < 1) P = 1;
   long chunk = (NP + P - 1) / P;
   chunk = (chunk + WG_KP - 1) / WG_KP * WG_KP;
-  P = (NP + chunk - 1) / chunk;
-  dim3 grid((unsigned)P, taps, tiles);
-  k_conv_wgrad<TM, TN><<<grid, 256, 0, stream>>>(p, chunk);
+  pl.P = (NP + chunk - 1) / chunk;
+  pl.chunk = chunk;
+  return pl;
+}
+
+// partials [P][taps][Cin][Cout] into part (reduced in pixel-chunk order by the caller)
+template <int TM, int TN>
+int launch_wgrad(const ffsr_wgrad_params& p, const WgradPlan& pl, float* part, cudaStream_t stream) {
+  const int taps = p.ksize * p.ksize;
+  dim3 grid((unsigned)pl.P, taps, ceil_div(p.Cin, TM) * ceil_div(p.Cout, TN));
+  k_conv_wgrad<TM, TN><<<grid, 256, 0, stream>>>(p, pl.chunk, part);
   return ffsr_check_launch("conv2d_wgrad");
 }
 
 template <int TM>
-int dispatch_wgrad_n(const ffsr_wgrad_params& p, cudaStream_t s) {
-  if (p.Cout > 64) return launch_wgrad<TM, 128>(p, s);
-  if (p.Cout > 32) return launch_wgrad<TM, 64>(p, s);
-  if (p.Cout > 16) return launch_wgrad<TM, 32>(p, s);
-  return launch_wgrad<TM, 16>(p, s);
+int dispatch_wgrad_n(const ffsr_wgrad_params& p, const WgradPlan& pl, float* part, cudaStream_t s) {
+  if (pl.TN == 128) return launch_wgrad<TM, 128>(p, pl, part, s);
+  if (pl.TN == 64) return launch_wgrad<TM, 64>(p, pl, part, s);
+  if (pl.TN == 32) return launch_wgrad<TM, 32>(p, pl, part, s);
+  return launch_wgrad<TM, 16>(p, pl, part, s);
 }
 
 // ------------------------------------------------------------------------------------
@@ -194,7 +209,7 @@ int dispatch_wgrad_n(const ffsr_wgrad_params& p, cudaStream_t s) {
 // ------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_colsum(const void* __restrict__ v, int dtype, long long sN, long long sY,
                                                 long long sX, int H, int W, long NP, int C, long rows_per_block,
-                                                float* __restrict__ out) {
+                                                float* __restrict__ part) {
   extern __shared__ float sred[];          // [rows_in_block][CT]
   const int CT = blockDim.x;               // channel threads (power of two <= 64)
   const int RT = blockDim.y;
@@ -216,14 +231,14 @@ __global__ void __launch_bounds__(256) k_colsum(const void* __restrict__ v, int 
   if (threadIdx.y == 0 && c < C) {
     float s = 0.f;
     for (int i = 0; i < RT; ++i) s += sred[i * CT + threadIdx.x];
-    atomicAdd(out + c, s);
+    part[(long)blockIdx.x * C + c] = s;
   }
 }
 
 // dense channels-last fast path: rows of `pitch` elements, no index arithmetic per element, VEC channels per thread
 template <typename T, int VEC>
 __global__ void __launch_bounds__(256) k_colsum_rows(const T* __restrict__ v, long NP, int C, long pitch, int TPR,
-                                                     long rows_per_block, float* __restrict__ out) {
+                                                     long rows_per_block, float* __restrict__ part) {
   __shared__ float sred[256 * VEC];
   const int lane_c = threadIdx.x % TPR, rt = threadIdx.x / TPR, RT = 256 / TPR;
   const int c0 = lane_c * VEC;
@@ -257,7 +272,7 @@ __global__ void __launch_bounds__(256) k_colsum_rows(const T* __restrict__ v, lo
       if (c0 + i >= C) continue;
       float s = 0.f;
       for (int k = 0; k < RT; ++k) s += sred[(k * TPR + lane_c) * VEC + i];
-      atomicAdd(out + c0 + i, s);
+      part[(long)blockIdx.x * C + c0 + i] = s;
     }
   }
 }
@@ -314,15 +329,12 @@ __global__ void __launch_bounds__(256) k_act_bwd(const T* __restrict__ x, const 
 }
 
 // ------------------------------------------------------------------------------------
-// LayerNorm backward: one warp per row; dw/db reduced per block then atomically.
+// LayerNorm backward: one warp per row; per-block dw/db (warps summed in order) to slot blockIdx.x of part [grid][2E].
 // ------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_layernorm_bwd(const float* __restrict__ x, const float* __restrict__ dy,
                                                        long rows, int E, const float* __restrict__ w,
-                                                       float* __restrict__ dx, float* __restrict__ dw,
-                                                       float* __restrict__ db) {
-  extern __shared__ float sacc[];            // [2][E]
-  for (int i = threadIdx.x; i < 2 * E; i += blockDim.x) sacc[i] = 0.f;
-  __syncthreads();
+                                                       float* __restrict__ dx, float* __restrict__ part) {
+  extern __shared__ float sacc[];            // [warps][2][E]
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, wpb = blockDim.x >> 5;
   const int per = E / 32;
   float lw[8], ldw[8], ldb[8];
@@ -371,13 +383,14 @@ __global__ void __launch_bounds__(256) k_layernorm_bwd(const float* __restrict__
 #pragma unroll
   for (int i = 0; i < 8; ++i)
     if (i < per) {
-      atomicAdd(&sacc[lane + 32 * i], ldw[i]);
-      atomicAdd(&sacc[E + lane + 32 * i], ldb[i]);
+      sacc[wib * 2 * E + lane + 32 * i] = ldw[i];
+      sacc[wib * 2 * E + E + lane + 32 * i] = ldb[i];
     }
   __syncthreads();
-  for (int i = threadIdx.x; i < E; i += blockDim.x) {
-    atomicAdd(dw + i, sacc[i]);
-    atomicAdd(db + i, sacc[E + i]);
+  for (int i = threadIdx.x; i < 2 * E; i += blockDim.x) {
+    float s = 0.f;
+    for (int k = 0; k < wpb; ++k) s += sacc[k * 2 * E + i];
+    part[(long)blockIdx.x * 2 * E + i] = s;
   }
 }
 
@@ -386,9 +399,10 @@ __global__ void __launch_bounds__(256) k_layernorm_bwd(const float* __restrict__
 // (one LKABlock call each), R = rows (images*H*W) per group.
 //   stats : sum[g][c], sumsq[g][c]  (fp64 accumulation -> mean / biased var on the host side)
 //   bwd   : sdy[g][c] = sum dy, sdyx[g][c] = sum dy * xhat   (xhat from mean / rstd)
+// Both write slot blockIdx.x of part [grid.x][2][G][C] (the two sums of every (g, c)), reduced by k_sum_slots.
 // ------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_bn_stats(const float* __restrict__ x, long R, int C, long rows_per_block,
-                                                  double* __restrict__ sum, double* __restrict__ sumsq) {
+                                                  double* __restrict__ part) {
   extern __shared__ double sbn[];            // [2][RT][CT]
   const int CT = blockDim.x, RT = blockDim.y;
   const int c = blockIdx.y * CT + threadIdx.x;
@@ -412,15 +426,15 @@ __global__ void __launch_bounds__(256) k_bn_stats(const float* __restrict__ x, l
   if (threadIdx.y == 0 && c < C) {
     double s = 0.0, q = 0.0;
     for (int i = 0; i < RT; ++i) { s += sbn[i * CT + threadIdx.x]; q += sbn[(RT + i) * CT + threadIdx.x]; }
-    atomicAdd(sum + (long)g * C + c, s);
-    atomicAdd(sumsq + (long)g * C + c, q);
+    double* slot = part + (long)blockIdx.x * 2 * gridDim.z * C;
+    slot[(long)g * C + c] = s;
+    slot[(long)(gridDim.z + g) * C + c] = q;
   }
 }
 
 __global__ void __launch_bounds__(256) k_bn_bwd_reduce(const float* __restrict__ x, const float* __restrict__ dy, long R,
                                                        int C, long rows_per_block, const float* __restrict__ mean,
-                                                       const float* __restrict__ rstd, float* __restrict__ sdy,
-                                                       float* __restrict__ sdyx) {
+                                                       const float* __restrict__ rstd, float* __restrict__ part) {
   extern __shared__ float sbr[];             // [2][RT][CT]
   const int CT = blockDim.x, RT = blockDim.y;
   const int c = blockIdx.y * CT + threadIdx.x;
@@ -443,8 +457,9 @@ __global__ void __launch_bounds__(256) k_bn_bwd_reduce(const float* __restrict__
   if (threadIdx.y == 0 && c < C) {
     float s = 0.f, q = 0.f;
     for (int i = 0; i < RT; ++i) { s += sbr[i * CT + threadIdx.x]; q += sbr[(RT + i) * CT + threadIdx.x]; }
-    atomicAdd(sdy + (long)g * C + c, s);
-    atomicAdd(sdyx + (long)g * C + c, q);
+    float* slot = part + (long)blockIdx.x * 2 * gridDim.z * C;
+    slot[(long)g * C + c] = s;
+    slot[(long)(gridDim.z + g) * C + c] = q;
   }
 }
 
@@ -732,22 +747,23 @@ __global__ void __launch_bounds__(256) k_bilinear_fwd8(const T* __restrict__ src
   }
 }
 
-constexpr int BL_MAXC = 16;   // candidate outputs per axis that can read one input sample (scale factors up to ~6x)
+// Candidate output indices per axis are visited in chunks of BL_MAXC (one chunk up to ~6x upscaling; any factor works).
+constexpr int BL_MAXC = 16;
 
-// candidates [lo, hi] of output indices whose taps may touch input index `i`, and their weights
-__device__ __forceinline__ int bilin_adjoint_taps(int i, int in_size, int out_size, int& lo, float (&wt)[BL_MAXC]) {
+// candidates [lo, hi] of output indices whose taps may touch input index `i`
+__device__ __forceinline__ void bilin_adjoint_range(int i, int in_size, int out_size, int& lo, int& hi) {
   const float inv_r = (float)out_size / (float)in_size;
-  int l = (int)floorf(((float)i - 0.5f) * inv_r - 0.5f) - 1;
-  int hgh = (int)ceilf(((float)i + 1.5f) * inv_r - 0.5f) + 1;
-  l = max(l, 0);
-  hgh = min(hgh, out_size - 1);
-  int n = hgh - l + 1;
-  if (n > BL_MAXC) n = BL_MAXC;
-  lo = l;
+  lo = max((int)floorf(((float)i - 0.5f) * inv_r - 0.5f) - 1, 0);
+  hi = min((int)ceilf(((float)i + 1.5f) * inv_r - 0.5f) + 1, out_size - 1);
+}
+
+// weights of input index `i` in the taps of outputs lo .. lo + n - 1 (n = min(hi - lo + 1, BL_MAXC))
+__device__ __forceinline__ int bilin_adjoint_taps(int i, int in_size, int out_size, int lo, int hi, float (&wt)[BL_MAXC]) {
+  const int n = min(hi - lo + 1, BL_MAXC);
   for (int k = 0; k < BL_MAXC; ++k) {
     float wgt = 0.f;
     if (k < n) {
-      const BilinTap t = bilin_tap(l + k, in_size, out_size);
+      const BilinTap t = bilin_tap(lo + k, in_size, out_size);
       if (t.i0 == i) wgt += t.w0;
       if (t.i1 == i) wgt += t.w1;
     }
@@ -766,21 +782,27 @@ __global__ void __launch_bounds__(256) k_bilinear_bwd(const T* __restrict__ gout
     const int x = (int)(pix % w), y = (int)((pix / w) % h);
     const long n = pix / ((long)w * h);
     float wy[BL_MAXC], wx[BL_MAXC];
-    int ylo, xlo;
-    const int ny = bilin_adjoint_taps(y, h, H, ylo, wy);
-    const int nx = bilin_adjoint_taps(x, w, W, xlo, wx);
+    int ylo, yhi, xlo, xhi;
+    bilin_adjoint_range(y, h, H, ylo, yhi);
+    bilin_adjoint_range(x, w, W, xlo, xhi);
     float acc[VEC];
 #pragma unroll
     for (int k = 0; k < VEC; ++k) acc[k] = 0.f;
     const T* base = gout + n * H * W * C + cg * VEC;
-    for (int a = 0; a < ny; ++a) {
-      if (wy[a] == 0.f) continue;
-      for (int b = 0; b < nx; ++b) {
-        const float wgt = wy[a] * wx[b];
-        if (wgt == 0.f) continue;
-        const T* p = base + ((long)(ylo + a) * W + xlo + b) * C;
+    for (int y0 = ylo; y0 <= yhi; y0 += BL_MAXC) {
+      const int ny = bilin_adjoint_taps(y, h, H, y0, yhi, wy);
+      for (int x0 = xlo; x0 <= xhi; x0 += BL_MAXC) {
+        const int nx = bilin_adjoint_taps(x, w, W, x0, xhi, wx);
+        for (int a = 0; a < ny; ++a) {
+          if (wy[a] == 0.f) continue;
+          for (int b = 0; b < nx; ++b) {
+            const float wgt = wy[a] * wx[b];
+            if (wgt == 0.f) continue;
+            const T* p = base + ((long)(y0 + a) * W + x0 + b) * C;
 #pragma unroll
-        for (int k = 0; k < VEC; ++k) acc[k] = fmaf(wgt, to_f32<T>(p[k]), acc[k]);
+            for (int k = 0; k < VEC; ++k) acc[k] = fmaf(wgt, to_f32<T>(p[k]), acc[k]);
+          }
+        }
       }
     }
     T* o = gin + pix * C + cg * VEC;
@@ -904,7 +926,7 @@ template <typename T>
 __global__ void __launch_bounds__(256) k_axpby_bwd8(const T* __restrict__ g, const T* __restrict__ b, const T* __restrict__ c,
                                                     long c_pitch, const float* __restrict__ s1, const float* __restrict__ s2,
                                                     long NP, int C, T* __restrict__ db, T* __restrict__ dc,
-                                                    float* __restrict__ ds) {
+                                                    float* __restrict__ part) {
   __shared__ float sh[2][8];
   const float k1 = s1[0], k2 = c ? s2[0] : 0.f;
   const int G = C >> 3;
@@ -936,8 +958,8 @@ __global__ void __launch_bounds__(256) k_axpby_bwd8(const T* __restrict__ g, con
   if (threadIdx.x == 0) {
     float t1 = 0.f, t2 = 0.f;
     for (int i = 0; i < 8; ++i) { t1 += sh[0][i]; t2 += sh[1][i]; }
-    atomicAdd(ds, t1);
-    if (c) atomicAdd(ds + 1, t2);
+    part[(long)blockIdx.x * (c ? 2 : 1)] = t1;
+    if (c) part[(long)blockIdx.x * 2 + 1] = t2;
   }
 }
 
@@ -957,12 +979,12 @@ __global__ void __launch_bounds__(256) k_axpby_fwd(const T* __restrict__ a, cons
     out[i] = from_f32<T>(v);
   }
 }
-// db = s1*g, dc = s2*g, ds1 += sum g*b, ds2 += sum g*c
+// db = s1*g, dc = s2*g; slot blockIdx.x of part [grid][1 or 2] = partial sum g*b (, sum g*c)
 template <typename T>
 __global__ void __launch_bounds__(256) k_axpby_bwd(const T* __restrict__ g, const T* __restrict__ b, const T* __restrict__ c,
                                                    long c_pitch, const float* __restrict__ s1, const float* __restrict__ s2,
                                                    long NP, int C, T* __restrict__ db, T* __restrict__ dc,
-                                                   float* __restrict__ ds) {
+                                                   float* __restrict__ part) {
   __shared__ float sh[2][8];
   const float k1 = s1[0], k2 = c ? s2[0] : 0.f;
   const long total = NP * C;
@@ -987,8 +1009,8 @@ __global__ void __launch_bounds__(256) k_axpby_bwd(const T* __restrict__ g, cons
   if (threadIdx.x == 0) {
     float t1 = 0.f, t2 = 0.f;
     for (int i = 0; i < 8; ++i) { t1 += sh[0][i]; t2 += sh[1][i]; }
-    atomicAdd(ds, t1);
-    if (c) atomicAdd(ds + 1, t2);
+    part[(long)blockIdx.x * (c ? 2 : 1)] = t1;
+    if (c) part[(long)blockIdx.x * 2 + 1] = t2;
   }
 }
 
@@ -1002,22 +1024,28 @@ __global__ void __launch_bounds__(256) k_bilinear_bwd8(const T* __restrict__ gou
     const int x = (int)(pix % w), y = (int)((pix / w) % h);
     const long n = pix / ((long)w * h);
     float wy[BL_MAXC], wx[BL_MAXC];
-    int ylo, xlo;
-    const int ny = bilin_adjoint_taps(y, h, H, ylo, wy);
-    const int nx = bilin_adjoint_taps(x, w, W, xlo, wx);
+    int ylo, yhi, xlo, xhi;
+    bilin_adjoint_range(y, h, H, ylo, yhi);
+    bilin_adjoint_range(x, w, W, xlo, xhi);
     float acc[8];
 #pragma unroll
     for (int k = 0; k < 8; ++k) acc[k] = 0.f;
     const T* base = gout + n * H * W * C + cg * 8;
-    for (int a = 0; a < ny; ++a) {
-      if (wy[a] == 0.f) continue;
-      for (int b = 0; b < nx; ++b) {
-        const float wgt = wy[a] * wx[b];
-        if (wgt == 0.f) continue;
-        float v[8];
-        load8<T>(base + ((long)(ylo + a) * W + xlo + b) * C, v);
+    for (int y0 = ylo; y0 <= yhi; y0 += BL_MAXC) {
+      const int ny = bilin_adjoint_taps(y, h, H, y0, yhi, wy);
+      for (int x0 = xlo; x0 <= xhi; x0 += BL_MAXC) {
+        const int nx = bilin_adjoint_taps(x, w, W, x0, xhi, wx);
+        for (int a = 0; a < ny; ++a) {
+          if (wy[a] == 0.f) continue;
+          for (int b = 0; b < nx; ++b) {
+            const float wgt = wy[a] * wx[b];
+            if (wgt == 0.f) continue;
+            float v[8];
+            load8<T>(base + ((long)(y0 + a) * W + x0 + b) * C, v);
 #pragma unroll
-        for (int k = 0; k < 8; ++k) acc[k] = fmaf(wgt, v[k], acc[k]);
+            for (int k = 0; k < 8; ++k) acc[k] = fmaf(wgt, v[k], acc[k]);
+          }
+        }
       }
     }
     store8<T>(gin + pix * C + cg * 8, acc);
@@ -1029,45 +1057,83 @@ inline void colsum_geom(int C, dim3& block, int& CT) {
   while (CT < C && CT < 64) CT <<= 1;
   block = dim3(CT, 256 / CT);
 }
+
+// grid of the BN reductions: (row chunks, channel tiles, groups)
+inline void bn_geom(int G, long R, int C, dim3& block, dim3& grid, long& rpb) {
+  int CT;
+  colsum_geom(C, block, CT);
+  long blocks = 148 * 4 / ((long)ceil_div(C, CT) * G);
+  if (blocks < 1) blocks = 1;
+  rpb = (R + blocks - 1) / blocks;
+  if (rpb < 64) rpb = 64;
+  grid = dim3(ceil_div(R, rpb), ceil_div(C, CT), G);
+}
+
+constexpr long COLSUM_MAX_BLOCKS = 148 * 8;     // row chunks of either colsum path
+constexpr long LN_MAX_BLOCKS = 148 * 8;
+constexpr long AXPBY_MAX_BLOCKS = 148 * 8;
 }  // namespace
 
-extern "C" int ffsr_conv2d_wgrad(const ffsr_wgrad_params* pp, cudaStream_t stream) {
+extern "C" size_t ffsr_conv2d_wgrad_workspace_bytes(int N, int H, int W, int Cin, int Cout, int ksize) {
+  if (N <= 0 || H <= 0 || W <= 0 || Cin <= 0 || Cout <= 0 || (ksize != 1 && ksize != 3)) return 0;
+  const WgradPlan pl = wgrad_plan(N, H, W, Cin, Cout, ksize);
+  return ws_align((size_t)pl.P * ksize * ksize * Cin * Cout * sizeof(float)) + ffsr_colsum_workspace_bytes(N, H, W, Cout);
+}
+
+extern "C" int ffsr_conv2d_wgrad(const ffsr_wgrad_params* pp, void* ws, size_t ws_bytes, cudaStream_t stream) {
   FFSR_REQUIRE(pp, FFSR_ERR_ARG, "conv2d_wgrad: null params");
   const ffsr_wgrad_params& p = *pp;
-  FFSR_REQUIRE(p.x && p.dy && p.dw, FFSR_ERR_ARG, "conv2d_wgrad: null pointer");
+  FFSR_REQUIRE(p.x && p.dy && p.dw && ws, FFSR_ERR_ARG, "conv2d_wgrad: null pointer");
   FFSR_REQUIRE(p.N > 0 && p.H > 0 && p.W > 0 && p.Cin > 0 && p.Cout > 0, FFSR_ERR_ARG, "conv2d_wgrad: bad shape");
   FFSR_REQUIRE(p.ksize == 1 || p.ksize == 3, FFSR_ERR_ARG, "conv2d_wgrad: ksize must be 1 or 3");
+  FFSR_REQUIRE(ws_bytes >= ffsr_conv2d_wgrad_workspace_bytes(p.N, p.H, p.W, p.Cin, p.Cout, p.ksize), FFSR_ERR_ARG,
+               "conv2d_wgrad: workspace too small");
+  const WgradPlan pl = wgrad_plan(p.N, p.H, p.W, p.Cin, p.Cout, p.ksize);
+  const int taps = p.ksize * p.ksize;
+  float* part = (float*)ws;
+  float* bpart = (float*)((char*)ws + ws_align((size_t)pl.P * taps * p.Cin * p.Cout * sizeof(float)));
   int rc;
-  if (p.Cin > 64) rc = dispatch_wgrad_n<128>(p, stream);
-  else if (p.Cin > 32) rc = dispatch_wgrad_n<64>(p, stream);
-  else if (p.Cin > 16) rc = dispatch_wgrad_n<32>(p, stream);
-  else rc = dispatch_wgrad_n<16>(p, stream);
+  if (pl.TM == 128) rc = dispatch_wgrad_n<128>(p, pl, part, stream);
+  else if (pl.TM == 64) rc = dispatch_wgrad_n<64>(p, pl, part, stream);
+  else if (pl.TM == 32) rc = dispatch_wgrad_n<32>(p, pl, part, stream);
+  else rc = dispatch_wgrad_n<16>(p, pl, part, stream);
   if (rc) return rc;
-  if (p.dbias) return ffsr_colsum(p.dy, p.dy_dtype, p.N, p.H, p.W, p.Cout, p.dy_sN, p.dy_sY, p.dy_sX, p.dbias, stream);
-  return FFSR_OK;
+  SlotSum<float> bias{};
+  if (p.dbias) {
+    int nb;
+    rc = colsum_partials(p.dy, p.dy_dtype, p.N, p.H, p.W, p.Cout, p.dy_sN, p.dy_sY, p.dy_sX, bpart, &nb, stream);
+    if (rc) return rc;
+    bias = slot_sum<float>(bpart, nb, p.Cout, p.dbias);
+  }
+  launch_sum_slots<float>(slot_sum<float>(part, (int)pl.P, (long)taps * p.Cin * p.Cout, p.dw), bias, stream);
+  return ffsr_check_launch("conv2d_wgrad_reduce");
 }
 
 extern "C" size_t ffsr_wgrad_params_size(void) { return sizeof(ffsr_wgrad_params); }
 
-extern "C" int ffsr_colsum(const void* v, int dtype, int N, int H, int W, int C, long long sN, long long sY,
-                           long long sX, float* out, cudaStream_t stream) {
-  FFSR_REQUIRE(v && out && N > 0 && H > 0 && W > 0 && C > 0, FFSR_ERR_ARG, "colsum: bad argument");
+extern "C" size_t ffsr_colsum_workspace_bytes(int N, int H, int W, int C) {
+  (void)N; (void)H; (void)W;
+  return C > 0 ? (size_t)COLSUM_MAX_BLOCKS * C * sizeof(float) : 0;
+}
+
+int colsum_partials(const void* v, int dtype, int N, int H, int W, int C, long long sN, long long sY, long long sX,
+                    float* part, int* nslots, cudaStream_t stream) {
   if (sY == (long long)W * sX && sN == (long long)H * W * sX && C <= 512) {      // dense channels-last rows
     const long NP = (long)N * H * W;
     const int VEC = C >= 64 ? 4 : 1;
     int TPR = 1;
     while (TPR * VEC < C) TPR <<= 1;                   // power of two, <= 128
-    long blocks = 148 * 8;
-    long rpb = (NP + blocks - 1) / blocks;
+    long rpb = (NP + COLSUM_MAX_BLOCKS - 1) / COLSUM_MAX_BLOCKS;
     if (rpb < 256) rpb = 256;
     const unsigned grid = (unsigned)((NP + rpb - 1) / rpb);
     if (dtype == FFSR_DT_BF16) {
-      if (VEC == 4) k_colsum_rows<__nv_bfloat16, 4><<<grid, 256, 0, stream>>>((const __nv_bfloat16*)v, NP, C, sX, TPR, rpb, out);
-      else k_colsum_rows<__nv_bfloat16, 1><<<grid, 256, 0, stream>>>((const __nv_bfloat16*)v, NP, C, sX, TPR, rpb, out);
+      if (VEC == 4) k_colsum_rows<__nv_bfloat16, 4><<<grid, 256, 0, stream>>>((const __nv_bfloat16*)v, NP, C, sX, TPR, rpb, part);
+      else k_colsum_rows<__nv_bfloat16, 1><<<grid, 256, 0, stream>>>((const __nv_bfloat16*)v, NP, C, sX, TPR, rpb, part);
     } else {
-      if (VEC == 4) k_colsum_rows<float, 4><<<grid, 256, 0, stream>>>((const float*)v, NP, C, sX, TPR, rpb, out);
-      else k_colsum_rows<float, 1><<<grid, 256, 0, stream>>>((const float*)v, NP, C, sX, TPR, rpb, out);
+      if (VEC == 4) k_colsum_rows<float, 4><<<grid, 256, 0, stream>>>((const float*)v, NP, C, sX, TPR, rpb, part);
+      else k_colsum_rows<float, 1><<<grid, 256, 0, stream>>>((const float*)v, NP, C, sX, TPR, rpb, part);
     }
+    *nslots = (int)grid;
     return ffsr_check_launch("colsum_rows");
   }
   dim3 block;
@@ -1079,8 +1145,20 @@ extern "C" int ffsr_colsum(const void* v, int dtype, int N, int H, int W, int C,
   long rpb = (NP + blocks - 1) / blocks;
   if (rpb < 64) rpb = 64;
   dim3 grid(ceil_div(NP, rpb), ceil_div(C, CT));
-  k_colsum<<<grid, block, 256 * sizeof(float), stream>>>(v, dtype, sN, sY, sX, H, W, NP, C, rpb, out);
+  k_colsum<<<grid, block, 256 * sizeof(float), stream>>>(v, dtype, sN, sY, sX, H, W, NP, C, rpb, part);
+  *nslots = (int)grid.x;
   return ffsr_check_launch("colsum");
+}
+
+extern "C" int ffsr_colsum(const void* v, int dtype, int N, int H, int W, int C, long long sN, long long sY,
+                           long long sX, float* out, void* ws, size_t ws_bytes, cudaStream_t stream) {
+  FFSR_REQUIRE(v && out && ws && N > 0 && H > 0 && W > 0 && C > 0, FFSR_ERR_ARG, "colsum: bad argument");
+  FFSR_REQUIRE(ws_bytes >= ffsr_colsum_workspace_bytes(N, H, W, C), FFSR_ERR_ARG, "colsum: workspace too small");
+  int nslots;
+  const int rc = colsum_partials(v, dtype, N, H, W, C, sN, sY, sX, (float*)ws, &nslots, stream);
+  if (rc) return rc;
+  launch_sum_slots<float>((const float*)ws, nslots, C, out, stream);
+  return ffsr_check_launch("colsum_reduce");
 }
 
 extern "C" int ffsr_act_forward(const void* x, void* y, long n, int act, int dtype, cudaStream_t stream) {
@@ -1101,27 +1179,46 @@ extern "C" int ffsr_act_backward(const void* x, const void* dy, void* dx, long n
   return ffsr_check_launch("act_backward");
 }
 
-extern "C" int ffsr_layernorm_backward(const float* x, const float* dy, long rows, int E, const float* w, float* dx,
-                                       float* dw, float* db, cudaStream_t stream) {
-  FFSR_REQUIRE(x && dy && w && dx && dw && db, FFSR_ERR_ARG, "layernorm_backward: null pointer");
-  FFSR_REQUIRE(E % 32 == 0 && E >= 32 && E <= 256, FFSR_ERR_ARG, "layernorm_backward: E must be a multiple of 32 in [32,256]");
-  const int grid = (int)min((long)148 * 8, (rows + 7) / 8);
-  k_layernorm_bwd<<<grid, 256, 2 * E * sizeof(float), stream>>>(x, dy, rows, E, w, dx, dw, db);
-  return ffsr_check_launch("layernorm_backward");
+extern "C" size_t ffsr_layernorm_backward_workspace_bytes(long rows, int E) {
+  if (rows <= 0 || E <= 0) return 0;
+  return (size_t)min(LN_MAX_BLOCKS, (rows + 7) / 8) * 2 * E * sizeof(float);
 }
 
-extern "C" int ffsr_bn_stats(const float* x, int G, long R, int C, double* sum, double* sumsq, cudaStream_t stream) {
-  FFSR_REQUIRE(x && sum && sumsq && G > 0 && R > 0 && C > 0 && G <= 65535, FFSR_ERR_ARG, "bn_stats: bad argument");
-  dim3 block;
-  int CT;
-  colsum_geom(C, block, CT);
-  long blocks = 148 * 4 / ((long)ceil_div(C, CT) * G);
-  if (blocks < 1) blocks = 1;
-  long rpb = (R + blocks - 1) / blocks;
-  if (rpb < 64) rpb = 64;
-  dim3 grid(ceil_div(R, rpb), ceil_div(C, CT), G);
-  k_bn_stats<<<grid, block, 2 * 256 * sizeof(double), stream>>>(x, R, C, rpb, sum, sumsq);
-  return ffsr_check_launch("bn_stats");
+extern "C" int ffsr_layernorm_backward(const float* x, const float* dy, long rows, int E, const float* w, float* dx,
+                                       float* dw, float* db, void* ws, size_t ws_bytes, cudaStream_t stream) {
+  FFSR_REQUIRE(x && dy && w && dx && dw && db && ws && rows > 0, FFSR_ERR_ARG, "layernorm_backward: null pointer");
+  FFSR_REQUIRE(E % 32 == 0 && E >= 32 && E <= 256, FFSR_ERR_ARG, "layernorm_backward: E must be a multiple of 32 in [32,256]");
+  FFSR_REQUIRE(ws_bytes >= ffsr_layernorm_backward_workspace_bytes(rows, E), FFSR_ERR_ARG, "layernorm_backward: workspace too small");
+  const int grid = (int)min(LN_MAX_BLOCKS, (rows + 7) / 8);
+  float* part = (float*)ws;
+  k_layernorm_bwd<<<grid, 256, 8 * 2 * E * sizeof(float), stream>>>(x, dy, rows, E, w, dx, part);
+  const int rc = ffsr_check_launch("layernorm_backward");
+  if (rc) return rc;
+  launch_sum_slots<float>(part, grid, 2L * E, dw, stream, db, E);
+  return ffsr_check_launch("layernorm_backward_reduce");
+}
+
+extern "C" size_t ffsr_bn_stats_workspace_bytes(int G, long R, int C) {
+  if (G <= 0 || R <= 0 || C <= 0) return 0;
+  dim3 block, grid;
+  long rpb;
+  bn_geom(G, R, C, block, grid, rpb);
+  return (size_t)grid.x * 2 * G * C * sizeof(double);
+}
+
+extern "C" int ffsr_bn_stats(const float* x, int G, long R, int C, double* sum, double* sumsq, void* ws, size_t ws_bytes,
+                             cudaStream_t stream) {
+  FFSR_REQUIRE(x && sum && sumsq && ws && G > 0 && R > 0 && C > 0 && G <= 65535, FFSR_ERR_ARG, "bn_stats: bad argument");
+  FFSR_REQUIRE(ws_bytes >= ffsr_bn_stats_workspace_bytes(G, R, C), FFSR_ERR_ARG, "bn_stats: workspace too small");
+  dim3 block, grid;
+  long rpb;
+  bn_geom(G, R, C, block, grid, rpb);
+  double* part = (double*)ws;
+  k_bn_stats<<<grid, block, 2 * 256 * sizeof(double), stream>>>(x, R, C, rpb, part);
+  const int rc = ffsr_check_launch("bn_stats");
+  if (rc) return rc;
+  launch_sum_slots<double>(part, (int)grid.x, 2L * G * C, sum, stream, sumsq, (long)G * C);
+  return ffsr_check_launch("bn_stats_reduce");
 }
 
 extern "C" int ffsr_bn_apply(const float* x, int G, long R, int C, const float* mean, const float* rstd, const float* w,
@@ -1132,21 +1229,29 @@ extern "C" int ffsr_bn_apply(const float* x, int G, long R, int C, const float* 
   return ffsr_check_launch("bn_apply");
 }
 
+extern "C" size_t ffsr_bn_backward_workspace_bytes(int G, long R, int C) {
+  if (G <= 0 || R <= 0 || C <= 0) return 0;
+  dim3 block, grid;
+  long rpb;
+  bn_geom(G, R, C, block, grid, rpb);
+  return (size_t)grid.x * 2 * G * C * sizeof(float);
+}
+
 extern "C" int ffsr_bn_backward(const float* x, const float* dy, int G, long R, int C, const float* mean,
-                                const float* rstd, const float* w, float* sdy, float* sdyx, float* dx,
-                                cudaStream_t stream) {
-  FFSR_REQUIRE(x && dy && mean && rstd && w && sdy && sdyx && dx && G > 0 && R > 0 && C > 0 && G <= 65535, FFSR_ERR_ARG,
+                                const float* rstd, const float* w, float* sdy, float* sdyx, float* dx, void* ws,
+                                size_t ws_bytes, cudaStream_t stream) {
+  FFSR_REQUIRE(x && dy && mean && rstd && w && sdy && sdyx && dx && ws && G > 0 && R > 0 && C > 0 && G <= 65535, FFSR_ERR_ARG,
                "bn_backward: bad argument");
-  dim3 block;
-  int CT;
-  colsum_geom(C, block, CT);
-  long blocks = 148 * 4 / ((long)ceil_div(C, CT) * G);
-  if (blocks < 1) blocks = 1;
-  long rpb = (R + blocks - 1) / blocks;
-  if (rpb < 64) rpb = 64;
-  dim3 grid(ceil_div(R, rpb), ceil_div(C, CT), G);
-  k_bn_bwd_reduce<<<grid, block, 2 * 256 * sizeof(float), stream>>>(x, dy, R, C, rpb, mean, rstd, sdy, sdyx);
+  FFSR_REQUIRE(ws_bytes >= ffsr_bn_backward_workspace_bytes(G, R, C), FFSR_ERR_ARG, "bn_backward: workspace too small");
+  dim3 block, grid;
+  long rpb;
+  bn_geom(G, R, C, block, grid, rpb);
+  float* part = (float*)ws;
+  k_bn_bwd_reduce<<<grid, block, 2 * 256 * sizeof(float), stream>>>(x, dy, R, C, rpb, mean, rstd, part);
   int rc = ffsr_check_launch("bn_backward_reduce");
+  if (rc) return rc;
+  launch_sum_slots<float>(part, (int)grid.x, 2L * G * C, sdy, stream, sdyx, (long)G * C);
+  rc = ffsr_check_launch("bn_backward_sum");
   if (rc) return rc;
   FFSR_REQUIRE(C % 4 == 0, FFSR_ERR_ARG, "bn_backward: C must be a multiple of 4");
   const long total = (long)G * R * (C / 4);
@@ -1246,7 +1351,6 @@ extern "C" int ffsr_bilinear_forward(const void* src, int N, int h, int w, int C
 extern "C" int ffsr_bilinear_backward(const void* gout, int N, int H, int W, int C, void* gin, int h, int w, int dtype,
                                       cudaStream_t stream) {
   FFSR_REQUIRE(gout && gin && N > 0 && h > 0 && w > 0 && H > 0 && W > 0 && C > 0, FFSR_ERR_ARG, "bilinear_backward: bad argument");
-  FFSR_REQUIRE((long)H <= 6L * h + 6 && (long)W <= 6L * w + 6, FFSR_ERR_ARG, "bilinear_backward: upscaling factors above 6 are not built");
   return launch_bilinear<true>(gout, N, h, w, C, gin, H, W, dtype, stream);
 }
 
@@ -1304,23 +1408,36 @@ extern "C" int ffsr_axpby_forward(const void* a, const void* b, const void* c, l
   return ffsr_check_launch("axpby_forward");
 }
 
+extern "C" size_t ffsr_axpby_backward_workspace_bytes(long NP, int C) {
+  (void)NP; (void)C;
+  return (size_t)AXPBY_MAX_BLOCKS * 2 * sizeof(float);
+}
+
 extern "C" int ffsr_axpby_backward(const void* g, const void* b, const void* c, long c_pitch, const float* s1, const float* s2,
-                                   long NP, int C, void* db, void* dc, float* ds, int dtype, cudaStream_t stream) {
-  FFSR_REQUIRE(g && b && s1 && db && ds && NP > 0 && C > 0 && (!c || (s2 && dc)), FFSR_ERR_ARG, "axpby_backward: bad argument");
+                                   long NP, int C, void* db, void* dc, float* ds, void* ws, size_t ws_bytes, int dtype,
+                                   cudaStream_t stream) {
+  FFSR_REQUIRE(g && b && s1 && db && ds && ws && NP > 0 && C > 0 && (!c || (s2 && dc)), FFSR_ERR_ARG, "axpby_backward: bad argument");
+  FFSR_REQUIRE(ws_bytes >= ffsr_axpby_backward_workspace_bytes(NP, C), FFSR_ERR_ARG, "axpby_backward: workspace too small");
+  float* part = (float*)ws;
+  const int L = c ? 2 : 1;
+  int grid;
   auto al16 = [](const void* p) { return ((uintptr_t)p % 16) == 0; };
   const int esz = dtype == FFSR_DT_BF16 ? 2 : 4;
   if (C % 8 == 0 && al16(g) && al16(b) && al16(db) && (!c || (al16(c) && al16(dc) && (c_pitch * esz) % 16 == 0))) {
     const long total8 = NP * (C / 8);
-    const int grid8 = (int)min((long)148 * 8, (total8 + 255) / 256);
+    grid = (int)min(AXPBY_MAX_BLOCKS, (total8 + 255) / 256);
     if (dtype == FFSR_DT_BF16)
-      k_axpby_bwd8<__nv_bfloat16><<<grid8, 256, 0, stream>>>((const __nv_bfloat16*)g, (const __nv_bfloat16*)b, (const __nv_bfloat16*)c, c_pitch, s1, s2, NP, C, (__nv_bfloat16*)db, (__nv_bfloat16*)dc, ds);
-    else k_axpby_bwd8<float><<<grid8, 256, 0, stream>>>((const float*)g, (const float*)b, (const float*)c, c_pitch, s1, s2, NP, C, (float*)db, (float*)dc, ds);
-    return ffsr_check_launch("axpby_backward");
+      k_axpby_bwd8<__nv_bfloat16><<<grid, 256, 0, stream>>>((const __nv_bfloat16*)g, (const __nv_bfloat16*)b, (const __nv_bfloat16*)c, c_pitch, s1, s2, NP, C, (__nv_bfloat16*)db, (__nv_bfloat16*)dc, part);
+    else k_axpby_bwd8<float><<<grid, 256, 0, stream>>>((const float*)g, (const float*)b, (const float*)c, c_pitch, s1, s2, NP, C, (float*)db, (float*)dc, part);
+  } else {
+    const long total = NP * C;
+    grid = (int)min(AXPBY_MAX_BLOCKS, (total + 255) / 256);
+    if (dtype == FFSR_DT_BF16)
+      k_axpby_bwd<__nv_bfloat16><<<grid, 256, 0, stream>>>((const __nv_bfloat16*)g, (const __nv_bfloat16*)b, (const __nv_bfloat16*)c, c_pitch, s1, s2, NP, C, (__nv_bfloat16*)db, (__nv_bfloat16*)dc, part);
+    else k_axpby_bwd<float><<<grid, 256, 0, stream>>>((const float*)g, (const float*)b, (const float*)c, c_pitch, s1, s2, NP, C, (float*)db, (float*)dc, part);
   }
-  const long total = NP * C;
-  const int grid = (int)min((long)148 * 8, (total + 255) / 256);
-  if (dtype == FFSR_DT_BF16)
-    k_axpby_bwd<__nv_bfloat16><<<grid, 256, 0, stream>>>((const __nv_bfloat16*)g, (const __nv_bfloat16*)b, (const __nv_bfloat16*)c, c_pitch, s1, s2, NP, C, (__nv_bfloat16*)db, (__nv_bfloat16*)dc, ds);
-  else k_axpby_bwd<float><<<grid, 256, 0, stream>>>((const float*)g, (const float*)b, (const float*)c, c_pitch, s1, s2, NP, C, (float*)db, (float*)dc, ds);
-  return ffsr_check_launch("axpby_backward");
+  const int rc = ffsr_check_launch("axpby_backward");
+  if (rc) return rc;
+  launch_sum_slots<float>(part, grid, L, ds, stream);
+  return ffsr_check_launch("axpby_backward_reduce");
 }

@@ -406,11 +406,17 @@ k_wgrad_tc1c(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CU
   }
 }
 
-// dw[tap][ci][co] += sum_p ws[p][tap][ci][co]
-__global__ void __launch_bounds__(256) k_wgrad_reduce(const float* __restrict__ ws, int P, int taps, int Cin, int Cout,
-                                                      int cin_pad, int cout_pad, float* __restrict__ dw) {
+// dw[tap][ci][co] += sum_p ws[p][tap][ci][co] in blocks [0, dw_blocks); the blocks after them finish the bias sums
+constexpr int WR_THREADS = 1024;
+__global__ void __launch_bounds__(WR_THREADS) k_wgrad_reduce(const float* __restrict__ ws, int P, int taps, int Cin, int Cout,
+                                                             int cin_pad, int cout_pad, float* __restrict__ dw,
+                                                             long dw_blocks, const SlotSum<float> bias) {
+  if ((long)blockIdx.x >= dw_blocks) {
+    sum_slots_chunk(bias, blockIdx.x - dw_blocks);
+    return;
+  }
   const long total = (long)taps * Cin * Cout;
-  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += dw_blocks * blockDim.x) {
     const int co = (int)(i % Cout);
     const int ci = (int)((i / Cout) % Cin);
     const int tap = (int)(i / ((long)Cout * Cin));
@@ -480,8 +486,27 @@ WgPlan wg_plan(int N, int H, int W, int Cin, int Cout, int ks) {
 
 extern "C" size_t ffsr_conv2d_wgrad_tc_workspace_bytes(int N, int H, int W, int Cin, int Cout, int ksize) {
   const WgPlan pl = wg_plan(N, H, W, Cin, Cout, ksize);
-  return (size_t)pl.P * ksize * ksize * pl.cin_pad * pl.cout_pad * sizeof(float);
+  return ws_align((size_t)pl.P * ksize * ksize * pl.cin_pad * pl.cout_pad * sizeof(float)) +
+         ffsr_colsum_workspace_bytes(N, H, W, Cout);
 }
+
+namespace {
+// bias column-sum partials (after the weight-gradient partials in ws), then ONE launch reduces both
+int wgrad_tc_finish(const ffsr_wgrad_params& p, const WgPlan& pl, int taps, void* ws, cudaStream_t stream) {
+  SlotSum<float> bias{};
+  if (p.dbias) {
+    float* bpart = (float*)((char*)ws + ws_align((size_t)pl.P * taps * pl.cin_pad * pl.cout_pad * sizeof(float)));
+    int nb;
+    const int rc = colsum_partials(p.dy, p.dy_dtype, p.N, p.H, p.W, p.Cout, p.dy_sN, p.dy_sY, p.dy_sX, bpart, &nb, stream);
+    if (rc) return rc;
+    bias = slot_sum<float>(bpart, nb, p.Cout, p.dbias);
+  }
+  const long dw_blocks = ((long)taps * p.Cin * p.Cout + WR_THREADS - 1) / WR_THREADS;
+  k_wgrad_reduce<<<(unsigned)(dw_blocks + slot_sum_blocks(bias)), WR_THREADS, 0, stream>>>(
+      (const float*)ws, pl.P, taps, p.Cin, p.Cout, pl.cin_pad, pl.cout_pad, p.dw, dw_blocks, bias);
+  return ffsr_check_launch("conv2d_wgrad_reduce");
+}
+}  // namespace
 
 // x, dy: bf16 channels-last with 16-byte-multiple strides (pad the channel pitch to a multiple of 8)
 extern "C" int ffsr_conv2d_wgrad_tc(const ffsr_wgrad_params* pp, void* ws, size_t ws_bytes, cudaStream_t stream) {
@@ -543,12 +568,7 @@ extern "C" int ffsr_conv2d_wgrad_tc(const ffsr_wgrad_params* pp, void* ws, size_
     k_wgrad_tc1c<<<grid1, WT_THREADS, smem1, stream>>>(tX, tD, a1);
     int rc1 = ffsr_check_launch("conv2d_wgrad_tc1c");
     if (rc1) return rc1;
-    const long total1 = 9L * p.Cin * p.Cout;
-    k_wgrad_reduce<<<(int)((total1 + 255) / 256), 256, 0, stream>>>(a1.ws, pl.P, 9, p.Cin, p.Cout, pl.cin_pad, pl.cout_pad, p.dw);
-    rc1 = ffsr_check_launch("conv2d_wgrad_reduce");
-    if (rc1) return rc1;
-    if (p.dbias) return ffsr_colsum(p.dy, p.dy_dtype, p.N, p.H, p.W, p.Cout, p.dy_sN, p.dy_sY, p.dy_sX, p.dbias, stream);
-    return FFSR_OK;
+    return wgrad_tc_finish(p, pl, 9, ws, stream);
   }
   CUtensorMap tmX, tmD;
   {
@@ -596,11 +616,5 @@ extern "C" int ffsr_conv2d_wgrad_tc(const ffsr_wgrad_params* pp, void* ws, size_
   k_wgrad_tc<<<grid, WT_THREADS, smem_bytes, stream>>>(tmX, tmD, a);
   int rc = ffsr_check_launch("conv2d_wgrad_tc");
   if (rc) return rc;
-  const long total = (long)p.ksize * p.ksize * p.Cin * p.Cout;
-  k_wgrad_reduce<<<(int)((total + 255) / 256), 256, 0, stream>>>(a.ws, pl.P, p.ksize * p.ksize, p.Cin, p.Cout, pl.cin_pad,
-                                                                 pl.cout_pad, p.dw);
-  rc = ffsr_check_launch("conv2d_wgrad_reduce");
-  if (rc) return rc;
-  if (p.dbias) return ffsr_colsum(p.dy, p.dy_dtype, p.N, p.H, p.W, p.Cout, p.dy_sN, p.dy_sY, p.dy_sX, p.dbias, stream);
-  return FFSR_OK;
+  return wgrad_tc_finish(p, pl, p.ksize * p.ksize, ws, stream);
 }

@@ -62,7 +62,10 @@ class _FusedLosses(torch.autograd.Function):
         S = _S(p)
         with torch.cuda.device(dev):
             if w_l1 > 0:
-                K.check(lib.ffsr_loss_l1(p.data_ptr(), t.data_ptr(), n, w_l1 / n, sums.data_ptr(), dpred.data_ptr(), S), "loss_l1")
+                nb = lib.ffsr_loss_l1_workspace_bytes(n)
+                ws = torch.empty(nb, device=dev, dtype=torch.uint8)
+                K.check(lib.ffsr_loss_l1(p.data_ptr(), t.data_ptr(), n, w_l1 / n, sums.data_ptr(), ws.data_ptr(), nb,
+                                         dpred.data_ptr(), S), "loss_l1")
             if w_swt > 0:
                 nb = lib.ffsr_loss_swt_workspace_bytes(P, H, W)
                 ws = torch.empty(nb, device=dev, dtype=torch.uint8)

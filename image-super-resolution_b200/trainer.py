@@ -105,6 +105,7 @@ class FusedAdamW(torch.optim.Optimizer):
         self.ema = self.bucket.flat.clone() if ema_decay is not None else None
         dev = self.bucket.flat.device
         self._gsq = torch.zeros(1, device=dev, dtype=torch.float64)
+        self._gsq_ws = torch.empty(self.lib.ffsr_sumsq_workspace_bytes(self.bucket.numel), device=dev, dtype=torch.uint8)
         # step counter and learning rate live on the device so that a CUDA-graph replay sees fresh values
         self._step_dev = torch.zeros(1, device=dev, dtype=torch.int32)
         self._lr_dev = torch.full((1,), float(lr), device=dev, dtype=torch.float32)
@@ -174,7 +175,8 @@ class FusedAdamW(torch.optim.Optimizer):
             gsq = None
             if self.max_grad_norm > 0:
                 self._gsq.zero_()
-                K.check(self.lib.ffsr_sumsq(self.grads.data_ptr(), n, self._gsq.data_ptr(), S), "sumsq")
+                K.check(self.lib.ffsr_sumsq(self.grads.data_ptr(), n, self._gsq.data_ptr(), self._gsq_ws.data_ptr(),
+                                            self._gsq_ws.numel(), S), "sumsq")
                 gsq = self._gsq.data_ptr()
             K.check(self.lib.ffsr_adamw_ema_step(
                 self.bucket.flat.data_ptr(), self.grads.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(),
@@ -283,14 +285,22 @@ class FusionTrainer:
     backward, gradient all-reduce, clip + AdamW + EMA, BatchNorm buffer sync -- is captured once into a CUDA
     graph and replayed from static input buffers: the ~2,000 kernel launches of a step cost one graph launch
     instead of ~80 us of Python / driver time each.  The values that change between steps (optimizer step
-    count, learning rate, dropout seed) are device-side scalars.  A change of input shapes re-captures."""
+    count, learning rate, dropout seed) are device-side scalars.  A change of input shapes re-captures.
+
+    Reproducibility: every reduction of the step runs in a fixed order (no floating-point atomics) and the dropout
+    seeds come from torch's CPU generator plus a device counter that construction resets, so two trainers built
+    after the same ``torch.manual_seed`` (before the model, and on the same GPU, precision mode and inputs) give
+    bitwise-identical losses, gradients, parameters, optimizer / EMA state and BatchNorm buffers, eager or
+    graph-replayed, with or without ``torch.use_deterministic_algorithms(True)``."""
 
     def __init__(self, model, criterion, lr: float = 2e-4, betas=(0.9, 0.999), eps: float = 1e-8,
                  weight_decay: float = 1e-4, max_grad_norm: float = 1.0, ema_decay: Optional[float] = 0.999,
                  cuda_graph: bool = True, graph_warmup: int = 3):
+        from .training import seed_counter
         self.model, self.criterion = model, criterion
         self.names = [n for n, p in model.named_parameters() if p.requires_grad]
         self.optimizer = FusedAdamW(model.parameters(), lr, betas, eps, weight_decay, max_grad_norm, ema_decay)
+        seed_counter(self.optimizer.bucket.flat.device).zero_()     # dropout masks start over with each trainer
         if _world() > 1:                      # BatchNorm statistics / counters start from rank 0's too (parameters: FusedAdamW)
             for n, b in model.named_buffers():
                 if n.endswith(("running_mean", "running_var", "num_batches_tracked")):

@@ -35,7 +35,6 @@ import os
 from typing import Dict, List, Optional
 
 import torch
-import torch.nn.functional as F
 
 from . import _cabi as K
 
@@ -102,6 +101,12 @@ def _zeros(shape, dev, dtype=torch.float32):
 
 def _dt(t):
     return K.DT_BF16 if t.dtype == torch.bfloat16 else K.DT_F32
+
+
+def _ws(nbytes: int, dev) -> torch.Tensor:
+    """Workspace for the per-block partial sums of a reduction kernel (fixed-order, atomic-free: the training step is
+    bitwise reproducible).  The kernels write every byte they read, so it needs no initialisation."""
+    return torch.empty(max(int(nbytes), 16), device=dev, dtype=torch.uint8)
 
 
 # --------------------------------------------------------------------------------------
@@ -173,7 +178,9 @@ class _Conv2d(torch.autograd.Function):
             p.N, p.H, p.W, p.Cin, p.Cout, p.ksize = N, H, W, ci, co, kh
             p.dw = dwp.data_ptr()
             p.dbias = dbp.data_ptr() if dbp is not None else None
-            _ck(_lib().ffsr_conv2d_wgrad(C.byref(p), _S(x)), "conv2d_wgrad")
+            lib = _lib()
+            ws = _ws(lib.ffsr_conv2d_wgrad_workspace_bytes(N, H, W, ci, co, kh), x.device)
+            _ck(lib.ffsr_conv2d_wgrad(C.byref(p), ws.data_ptr(), ws.numel(), _S(x)), "conv2d_wgrad")
             dw = dwp.view(kh, kw, ci, co).permute(3, 2, 0, 1)
             db = dbp
         return dx, dw, db
@@ -298,7 +305,7 @@ def _wgrad_tc(xb, gb, ci, co, ks, has_bias):
     p.dw = dwp.data_ptr()
     p.dbias = dbp.data_ptr() if dbp is not None else None
     nb = lib.ffsr_conv2d_wgrad_tc_workspace_bytes(N, H, W, ci, co, ks)
-    ws = torch.empty(nb, device=xb.device, dtype=torch.uint8)
+    ws = _ws(nb, xb.device)
     _ck(lib.ffsr_conv2d_wgrad_tc(C.byref(p), ws.data_ptr(), nb, _S(xb)), "conv2d_wgrad_tc")
     return dwp, dbp
 
@@ -530,9 +537,12 @@ class _Axpby(torch.autograd.Function):
         db = torch.empty_like(b)
         dc = torch.empty_like(b) if ctx.has_c else None
         ds = _zeros((2,), b.device)
-        _ck(_lib().ffsr_axpby_backward(g.data_ptr(), b.data_ptr(), c.data_ptr() if ctx.has_c else None, ctx.c_pitch,
-                                       s1c.data_ptr(), s2c.data_ptr() if ctx.has_c else None, N * H * W, Cc, db.data_ptr(),
-                                       dc.data_ptr() if dc is not None else None, ds.data_ptr(), _dt(b), _S(b)), "axpby_backward")
+        lib = _lib()
+        ws = _ws(lib.ffsr_axpby_backward_workspace_bytes(N * H * W, Cc), b.device)
+        _ck(lib.ffsr_axpby_backward(g.data_ptr(), b.data_ptr(), c.data_ptr() if ctx.has_c else None, ctx.c_pitch,
+                                    s1c.data_ptr(), s2c.data_ptr() if ctx.has_c else None, N * H * W, Cc, db.data_ptr(),
+                                    dc.data_ptr() if dc is not None else None, ds.data_ptr(), ws.data_ptr(), ws.numel(),
+                                    _dt(b), _S(b)), "axpby_backward")
         return g, db, ds[0].reshape(()), dc, (ds[1].reshape(()) if ctx.has_c else None)
 
 
@@ -553,7 +563,9 @@ class _BatchNormTrain(torch.autograd.Function):
         dev = x.device
         s = _zeros((2, G, Cc), dev, torch.float64)
         lib = _lib()
-        _ck(lib.ffsr_bn_stats(x.data_ptr(), G, R, Cc, s[0].data_ptr(), s[1].data_ptr(), _S(x)), "bn_stats")
+        ws = _ws(lib.ffsr_bn_stats_workspace_bytes(G, R, Cc), dev)
+        _ck(lib.ffsr_bn_stats(x.data_ptr(), G, R, Cc, s[0].data_ptr(), s[1].data_ptr(), ws.data_ptr(), ws.numel(), _S(x)),
+            "bn_stats")
         mean64 = s[0] / R
         var64 = (s[1] / R - mean64 * mean64).clamp_(min=0.0)
         mean = mean64.float()
@@ -577,9 +589,11 @@ class _BatchNormTrain(torch.autograd.Function):
         gy = _cl(gy)
         red = _zeros((2, G, Cc), x.device)
         dx = torch.empty_like(x)
-        _ck(_lib().ffsr_bn_backward(x.data_ptr(), gy.data_ptr(), G, R, Cc, mean.data_ptr(), rstd.data_ptr(),
-                                    w.data_ptr(), red[0].data_ptr(), red[1].data_ptr(), dx.data_ptr(), _S(x)),
-            "bn_backward")
+        lib = _lib()
+        ws = _ws(lib.ffsr_bn_backward_workspace_bytes(G, R, Cc), x.device)
+        _ck(lib.ffsr_bn_backward(x.data_ptr(), gy.data_ptr(), G, R, Cc, mean.data_ptr(), rstd.data_ptr(),
+                                 w.data_ptr(), red[0].data_ptr(), red[1].data_ptr(), dx.data_ptr(), ws.data_ptr(), ws.numel(),
+                                 _S(x)), "bn_backward")
         return dx, red[1].sum(0), red[0].sum(0), None
 
 
@@ -637,8 +651,11 @@ class _LayerNorm(torch.autograd.Function):
         gy = _cl(gy)
         dx = torch.empty_like(x)
         dwb = _zeros((2, E), x.device)
-        _ck(_lib().ffsr_layernorm_backward(x.data_ptr(), gy.data_ptr(), N * H * W, E, w.data_ptr(), dx.data_ptr(),
-                                           dwb[0].data_ptr(), dwb[1].data_ptr(), _S(x)), "layernorm_backward")
+        lib = _lib()
+        ws = _ws(lib.ffsr_layernorm_backward_workspace_bytes(N * H * W, E), x.device)
+        _ck(lib.ffsr_layernorm_backward(x.data_ptr(), gy.data_ptr(), N * H * W, E, w.data_ptr(), dx.data_ptr(),
+                                        dwb[0].data_ptr(), dwb[1].data_ptr(), ws.data_ptr(), ws.numel(), _S(x)),
+            "layernorm_backward")
         return dx, dwb[0], dwb[1]
 
 
@@ -745,7 +762,9 @@ class _DwStage(torch.autograd.Function):
             _ck(lib.ffsr_dwconv_stage(gy.data_ptr(), N, H, W, Cc, kind, wf.data_ptr(), ones.data_ptr(), zeros.data_ptr(),
                                       dx.data_ptr(), _S(x)), "dwconv_stage(bwd)")
         dw = _zeros((Cc, weight.numel() // Cc), x.device)
-        _ck(lib.ffsr_dwconv_wgrad(x.data_ptr(), gy.data_ptr(), N, H, W, Cc, kind, dw.data_ptr(), _S(x)), "dwconv_wgrad")
+        ws = _ws(lib.ffsr_dwconv_wgrad_workspace_bytes(N, H, W, Cc, kind), x.device)
+        _ck(lib.ffsr_dwconv_wgrad(x.data_ptr(), gy.data_ptr(), N, H, W, Cc, kind, dw.data_ptr(), ws.data_ptr(), ws.numel(),
+                                  _S(x)), "dwconv_wgrad")
         return dx, dw.view(weight.shape), None
 
 
@@ -835,7 +854,8 @@ def _phase2_train(m, lr):
     The DCT and DWT analysis run on the library kernels with unit scales (the input needs no
     gradient, so they are constants of the graph) and are scaled by the learnable factors here;
     the FFT low-pass and the gradient of its learnable mask run on the library's dense-DFT kernels
-    (ffsr_fft_lowpass / ffsr_fft_lowpass_backward); only the 64x64 -> HxWf mask resize + sigmoid are tensor ops."""
+    (ffsr_fft_lowpass / ffsr_fft_lowpass_backward); the 64x64 -> HxWf mask resize runs on the bilinear node, the sigmoid is a
+    tensor op."""
     lib = _lib()
     fd = m.freq_decomp
     B, _, H, W = lr.shape
@@ -863,7 +883,9 @@ def _phase2_train(m, lr):
     scale7 = torch.cat([fd.dct.band_scale, fd.dwt.subband_scale])
     b7 = raw[:, :7] * scale7[None, :, None, None, None]
     Wf = W // 2 + 1
-    msk = F.interpolate(fd.fft.freq_mask_logits, size=(H, Wf), mode="bilinear", align_corners=False)   # [1,1,64,64] -> tiny
+    # [1,1,64,64] -> [1,1,H,Wf] on the library's bilinear node: its adjoint is a gather (no atomics), so the mask
+    # gradient is reproducible and the step runs under torch.use_deterministic_algorithms(True)
+    msk = _bilinear(fd.fft.freq_mask_logits, (H, Wf))
     msk = torch.sigmoid(msk * fd.fft.temperature.clamp(min=1.0))
     low = _FFTLowpass.apply(lr, msk)                                       # irfft2(rfft2(lr) * mask)
     low_s = low * fd.fft.band_scale[0]

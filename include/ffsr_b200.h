@@ -289,11 +289,18 @@ typedef struct ffsr_wgrad_params {
   float* dw;    /* [k*k][Cin][Cout] fp32, ACCUMULATED */
   float* dbias; /* [Cout] fp32, ACCUMULATED, or NULL */
 } ffsr_wgrad_params;
-int ffsr_conv2d_wgrad(const ffsr_wgrad_params* p, cudaStream_t stream);
+/* Reproducibility: every reduction of the training path below (weight / bias / scalar gradients, normalisation
+ * statistics, loss sums, gradient norm) partitions its work by shape alone, writes one partial per block into the
+ * caller's workspace `ws` (ws_bytes >= the matching *_workspace_bytes query; no initialisation needed) and adds
+ * the partials to the output in a fixed order: no floating-point atomics, so results are bitwise reproducible
+ * for the same shapes on the same GPU.  A workspace may be reused by calls ordered on one stream. */
+size_t ffsr_conv2d_wgrad_workspace_bytes(int N, int H, int W, int Cin, int Cout, int ksize);
+int ffsr_conv2d_wgrad(const ffsr_wgrad_params* p, void* ws, size_t ws_bytes, cudaStream_t stream);
 size_t ffsr_wgrad_params_size(void);
 /* out[c] += sum over (n,y,x) of a channels-last tensor (bias / scale gradients) */
+size_t ffsr_colsum_workspace_bytes(int N, int H, int W, int C);
 int ffsr_colsum(const void* v, int dtype, int N, int H, int W, int C, long long sN, long long sY, long long sX,
-                float* out, cudaStream_t stream);
+                float* out, void* ws, size_t ws_bytes, cudaStream_t stream);
 
 /* nn.GELU / nn.ReLU / nn.Sigmoid forward on contiguous data and backward on the saved
  * pre-activation: dx = dy * act'(x) */
@@ -301,8 +308,9 @@ int ffsr_act_forward(const void* x, void* y, long n, int act, int dtype, cudaStr
 int ffsr_act_backward(const void* x, const void* dy, void* dx, long n, int act, int dtype, cudaStream_t stream);
 
 /* nn.LayerNorm backward (large_kernel_attention.py:223, 389, 392); dw/db ACCUMULATED */
+size_t ffsr_layernorm_backward_workspace_bytes(long rows, int E);
 int ffsr_layernorm_backward(const float* x, const float* dy, long rows, int E, const float* w, float* dx, float* dw,
-                            float* db, cudaStream_t stream);
+                            float* db, void* ws, size_t ws_bytes, cudaStream_t stream);
 
 /* nn.BatchNorm2d in train mode (large_kernel_attention.py:84,128,131) on channels-last data
  * viewed as [G][R][C]: G independent statistic groups (one LKABlock call each), R rows per group.
@@ -310,11 +318,14 @@ int ffsr_layernorm_backward(const float* x, const float* dy, long rows, int E, c
  *   ffsr_bn_apply:    y = (x - mean[g][c]) * rstd[g][c] * w[c] + b[c]
  *   ffsr_bn_backward: sdy[g][c] += sum dy, sdyx[g][c] += sum dy*xhat (ACCUMULATED), then
  *                     dx = w*rstd*(dy - sdy/R - xhat*sdyx/R) */
-int ffsr_bn_stats(const float* x, int G, long R, int C, double* sum, double* sumsq, cudaStream_t stream);
+size_t ffsr_bn_stats_workspace_bytes(int G, long R, int C);
+int ffsr_bn_stats(const float* x, int G, long R, int C, double* sum, double* sumsq, void* ws, size_t ws_bytes,
+                  cudaStream_t stream);
 int ffsr_bn_apply(const float* x, int G, long R, int C, const float* mean, const float* rstd, const float* w,
                   const float* b, float* y, cudaStream_t stream);
+size_t ffsr_bn_backward_workspace_bytes(int G, long R, int C);
 int ffsr_bn_backward(const float* x, const float* dy, int G, long R, int C, const float* mean, const float* rstd,
-                     const float* w, float* sdy, float* sdyx, float* dx, cudaStream_t stream);
+                     const float* w, float* sdy, float* sdyx, float* dx, void* ws, size_t ws_bytes, cudaStream_t stream);
 
 /* nn.MultiheadAttention core in train mode (T = 4 or 9 tokens per LR pixel, head_dim 16,
  * attention-probability dropout): probs[B][HW][E/16][T][T] saved for the backward; the dropout
@@ -332,20 +343,23 @@ int ffsr_token_attention_backward(const float* qkv, const float* probs, const fl
  * and their weight gradients dw[C][taps] (ACCUMULATED).  large_kernel_attention.py:98-100 */
 int ffsr_dwconv_stage(const float* in, int N, int H, int W, int C, int kind, const float* w, const float* bn_k,
                       const float* bn_d, float* out, cudaStream_t stream);
-int ffsr_dwconv_wgrad(const float* in, const float* g, int N, int H, int W, int C, int kind, float* dw,
-                      cudaStream_t stream);
+size_t ffsr_dwconv_wgrad_workspace_bytes(int N, int H, int W, int C, int kind);
+int ffsr_dwconv_wgrad(const float* in, const float* g, int N, int H, int W, int C, int kind, float* dw, void* ws,
+                      size_t ws_bytes, cudaStream_t stream);
 
 /* ---- fused training losses (forward value + gradient w.r.t. pred in one pass) --------------
  * pred / target / dpred: [P][H][W] fp32 planes (P = B*C of an NCHW-contiguous tensor).
  * Each call ADDS its partial sums into the fp64 accumulators and ADDS gscale * dLoss/dPred into
- * dpred (the caller zeroes both); gscale = loss weight / element count (see losses.py).
+ * dpred (the caller zeroes both); gscale = loss weight / element count (see losses.py).  The partial sums
+ * go through the workspace (size queries below) and are added in a fixed order.
  *   ffsr_loss_l1    L1Loss        src/losses/perceptual_loss.py:86-104      sum[0] = sum |p-t|
  *   ffsr_loss_swt   SWTLoss       :661-733, 797-813   sums8 = sum|cA|,|cH|,|cV|,|cD| for level 0 then level 1
  *   ffsr_loss_ssim  SSIMLoss      :225-291            sum[0] = sum of the SSIM map
  *   ffsr_loss_fft   FFTLoss       :533-598            sums2 = sum w*||P|-|T||, sum w*|angle P - angle T|
  *                   (H, W must factor into 2,3,5,7: training patches are 256 / 384) */
-int ffsr_loss_l1(const float* pred, const float* target, long n, float gscale, double* sum, float* dpred,
-                 cudaStream_t stream);
+size_t ffsr_loss_l1_workspace_bytes(long n);
+int ffsr_loss_l1(const float* pred, const float* target, long n, float gscale, double* sum, void* ws, size_t ws_bytes,
+                 float* dpred, cudaStream_t stream);
 size_t ffsr_loss_swt_workspace_bytes(int P, int H, int W);
 int ffsr_loss_swt(const float* pred, const float* target, int P, int H, int W, float gscale, double* sums8, void* ws,
                   size_t ws_bytes, float* dpred, cudaStream_t stream);
@@ -363,7 +377,8 @@ int ffsr_loss_fft(const float* pred, const float* target, int P, int H, int W, f
  *   (train.py:847-853); ema = decay*ema + (1-decay)*p (checkpoint_manager.py:352-359; ema may be NULL).
  *   step_dev / lr_dev (optional device scalars): effective step = step + *step_dev, lr = *lr_dev -- the values
  *   that change between replays of a CUDA-graph-captured training step. */
-int ffsr_sumsq(const float* g, long n, double* out, cudaStream_t stream);
+size_t ffsr_sumsq_workspace_bytes(long n);
+int ffsr_sumsq(const float* g, long n, double* out, void* ws, size_t ws_bytes, cudaStream_t stream);
 int ffsr_adamw_ema_step(float* p, const float* g, float* m, float* v, float* ema, long n, float lr, float beta1,
                         float beta2, float eps, float weight_decay, int step, const int* step_dev, const float* lr_dev,
                         const double* gsumsq, float grad_scale, float max_norm, float ema_decay, cudaStream_t stream);
@@ -376,11 +391,12 @@ int ffsr_adamw_ema_step(float* p, const float* g, float* m, float* v, float* ema
  *   results in `ws` (ffsr_conv2d_wgrad_tc_workspace_bytes) reduced deterministically into dw. */
 int ffsr_to_bf16_nhwc(const void* src, int src_dtype, long long sN, long long sY, long long sX, long long sC, int N,
                       int H, int W, int C, int Cpad, void* dst, cudaStream_t stream);
-size_t ffsr_conv2d_wgrad_tc_workspace_bytes(int N, int H, int W, int Cin, int Cout, int ksize);
+size_t ffsr_conv2d_wgrad_tc_workspace_bytes(int N, int H, int W, int Cin, int Cout, int ksize);   /* covers the bias sums */
 int ffsr_conv2d_wgrad_tc(const ffsr_wgrad_params* p, void* ws, size_t ws_bytes, cudaStream_t stream);
 
 /* F.interpolate(mode="bilinear", align_corners=False) on dense channels-last tensors ([N][h][w][C] -> [N][H][W][C])
- * and its adjoint (gradient w.r.t. the source); any C, fp32 or bf16 (fp32 arithmetic).
+ * and its adjoint (gradient w.r.t. the source, a gather with no atomics); any C, any scale factor, fp32 or bf16
+ * (fp32 arithmetic).
  * hierarchical_fusion.py:156-186, enhanced_fusion_v2.py:735-791, edge_enhancement.py:208-250 */
 int ffsr_bilinear_forward(const void* src, int N, int h, int w, int C, void* dst, int H, int W, int dtype,
                           cudaStream_t stream);
@@ -399,8 +415,9 @@ int ffsr_gate_mul_backward(const void* y, const float* g, const void* gout, long
                            cudaStream_t stream);
 int ffsr_axpby_forward(const void* a, const void* b, const void* c, long c_pitch, const float* s1, const float* s2, long NP,
                        int C, void* out, int dtype, cudaStream_t stream);
+size_t ffsr_axpby_backward_workspace_bytes(long NP, int C);
 int ffsr_axpby_backward(const void* g, const void* b, const void* c, long c_pitch, const float* s1, const float* s2, long NP,
-                        int C, void* db, void* dc, float* ds, int dtype, cudaStream_t stream);
+                        int C, void* db, void* dc, float* ds, void* ws, size_t ws_bytes, int dtype, cudaStream_t stream);
 
 /* Train mode of FFTDecomposition (multi_domain_frequency.py:352-385): low = irfft2(mask * rfft2(x), ortho) with the
  * sigmoid mask [H][W/2+1] supplied by the caller, and d(loss)/d(mask) from d(loss)/d(low) (sum over batch and
