@@ -181,6 +181,7 @@ PROTOTYPES = {
     "ffsr_sumsq_workspace_bytes": (_SZ, [_L]),
     "ffsr_sumsq": (_I, [_P, _L, _P, _P, _SZ, _P]),
     "ffsr_adamw_ema_step": (_I, [_P, _P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _I, _P, _P, _P, _F, _F, _F, _P]),
+    "ffsr_sum_slots_ordered": (_I, [_P, _I, _L, _L, _P, _P]),
 }
 
 _lib = None

@@ -442,11 +442,7 @@ def epoch_batches(total: int, batch_size: int, shuffle: bool, seed: int, epoch: 
                   drop_last: bool = True) -> List[List[int]]:
     """Index batches of one epoch for one rank: a permutation shared by all ranks (seeded by ``seed + epoch``), every
     world-th index from position ``rank``, cut into batches.  Ranks never share an index within an epoch."""
-    if shuffle:
-        g = torch.Generator().manual_seed(seed + epoch)
-        order = torch.randperm(total, generator=g).tolist()
-    else:
-        order = list(range(total))
+    order = _epoch_order(total, shuffle, seed, epoch)
     if world > 1:
         # every rank must run the SAME number of steps: each step is a collective (gradient all-reduce, BatchNorm buffer
         # sync), so a rank with one batch more would wait in NCCL for ever at the end of the epoch.  With drop_last the
@@ -462,6 +458,42 @@ def epoch_batches(total: int, batch_size: int, shuffle: bool, seed: int, epoch: 
     if out and drop_last and len(out[-1]) < batch_size:
         out.pop()
     return out
+
+
+def _epoch_order(total: int, shuffle: bool, seed: int, epoch: int) -> List[int]:
+    if shuffle:
+        g = torch.Generator().manual_seed(seed + epoch)
+        return torch.randperm(total, generator=g).tolist()
+    return list(range(total))
+
+
+def world_invariant_batches(total: int, batch_size: int, shuffle: bool, seed: int, epoch: int, rank: int = 0,
+                            world: int = 1, drop_last: bool = True) -> List[Tuple[List[int], List[int]]]:
+    """(positions, sample indices) of one rank's batches in the world-invariant layout: at step t rank r takes
+    positions [t*world*B + r*B, t*world*B + (r+1)*B) of the epoch permutation shared by all ranks, which is cut to a
+    multiple of world*B (drop_last) or padded by wrapping around.  With world*B fixed, a position lands on the same
+    step and, cut into micro-batches of b = B/k, in the same global micro-batch (r*k + j) for every world size."""
+    order = _epoch_order(total, shuffle, seed, epoch)
+    span = world * batch_size
+    if drop_last:
+        order = order[:len(order) // span * span]
+    elif order:
+        target = -(-len(order) // span) * span
+        order = (order * -(-target // len(order)))[:target]
+    out = []
+    for t in range(len(order) // span):
+        pos = list(range(t * span + rank * batch_size, t * span + (rank + 1) * batch_size))
+        out.append((pos, [order[p] for p in pos]))
+    return out
+
+
+def augment_code(seed: int, epoch: int, position: int) -> int:
+    """Dihedral code of the sample at ``position`` of the epoch permutation, drawn (the reference's three draws, in its
+    order) from a generator keyed by (seed, epoch, position) alone: the same on whichever rank loads the sample."""
+    rng = random.Random(f"ffsr-augment:{seed}:{epoch}:{position}")
+    hflip = rng.random() < 0.5
+    vflip = rng.random() < 0.5
+    return dihedral_code(hflip, vflip, rng.randint(0, 3))
 
 
 def batches_per_epoch(total: int, batch_size: int, world: int = 1, drop_last: bool = True) -> int:
@@ -484,12 +516,18 @@ class DeviceBatchLoader:
 
     ``rng``: a ``random.Random`` (default seeded from ``seed``) from which the augmentation of every sample is drawn in
     the reference's order, so a run seeded like ``random.seed(s)`` reproduces the reference's augmentations.
-    Under ``world > 1`` rank r takes every world-th index of the (shared-seed) epoch permutation."""
+    Under ``world > 1`` rank r takes every world-th index of the (shared-seed) epoch permutation.
+
+    ``world_invariant=True``: rank r's batch at step t is the contiguous block of positions
+    [t*world*B + r*B, t*world*B + (r+1)*B) of the shared permutation, and each sample's augmentation is drawn from a
+    generator keyed by (seed, epoch, position) (``world_invariant_batches``, ``augment_code``).  For a fixed world*B,
+    every micro-batch of a step then gets the same samples and flips for any world size: the loader of
+    ``FusionTrainer(world_invariant=True)``.  ``rng`` is not used in this mode."""
 
     def __init__(self, shard: str, batch_size: int, device, augment: bool = True, shuffle: bool = True,
                  drop_last: bool = True, load_features: bool = True, repeat_factor: int = 1, rank: int = 0, world: int = 1,
                  seed: int = 0, depth: int = 2, copy_threads: int = 4, rng: Optional[random.Random] = None,
-                 out_dtype: torch.dtype = torch.float32, reuse_buffers: bool = True):
+                 out_dtype: torch.dtype = torch.float32, reuse_buffers: bool = True, world_invariant: bool = False):
         from . import _cabi as K
         self.K = K
         self.lib = K.load()                                   # raises FusionLibraryError when the library is missing
@@ -504,6 +542,7 @@ class DeviceBatchLoader:
         self.B, self.augment, self.shuffle, self.drop_last = int(batch_size), augment, shuffle, drop_last
         self.load_features = load_features and self.cache.header["load_features"]
         self.repeat_factor, self.rank, self.world, self.seed = repeat_factor, rank, world, seed
+        self.world_invariant = bool(world_invariant)
         self.depth = max(2, int(depth))
         self.rng = rng if rng is not None else random.Random(seed * 1000003 + rank)
         self.out_dtype = out_dtype
@@ -520,7 +559,11 @@ class DeviceBatchLoader:
         self.launches = 0
 
     def __len__(self) -> int:
-        return batches_per_epoch(self.cache.count * self.repeat_factor, self.B, self.world, self.drop_last)
+        total = self.cache.count * self.repeat_factor
+        if self.world_invariant:
+            span = self.world * self.B
+            return total // span if self.drop_last else -(-total // span)
+        return batches_per_epoch(total, self.B, self.world, self.drop_last)
 
     def set_epoch(self, epoch: int) -> None:
         self.epoch = int(epoch)
@@ -534,7 +577,7 @@ class DeviceBatchLoader:
                             "outs": {}} for _ in range(self.depth + 1)]
         return self._slots[k % len(self._slots)]
 
-    def _produce(self, k: int, idxs: List[int]) -> dict:
+    def _produce(self, k: int, idxs: List[int], positions: Optional[List[int]] = None, epoch: int = 0) -> dict:
         K, cache = self.K, self.cache
         n = len(idxs)
         recs = [i % cache.count for i in idxs]
@@ -544,7 +587,10 @@ class DeviceBatchLoader:
             slot["ev"].synchronize()                          # the H2D that last used this staging buffer has finished
         host = slot["host"].numpy()
         codes = np.zeros(self.B, dtype=np.int32)
-        if self.augment:
+        if self.augment and positions is not None:
+            for j in range(n):
+                codes[j] = augment_code(self.seed, epoch, positions[j])
+        elif self.augment:
             for j in range(n):
                 hflip = self.rng.random() < 0.5
                 vflip = self.rng.random() < 0.5
@@ -615,12 +661,18 @@ class DeviceBatchLoader:
         out["_event"], out["_tensors"], out["_slot"] = ev, tensors, slot
         return out
 
-    def _batches(self) -> List[List[int]]:
-        return epoch_batches(self.cache.count * self.repeat_factor, self.B, self.shuffle, self.seed, self.epoch, self.rank,
-                             self.world, self.drop_last)
+    def _batches(self) -> List[Tuple[Optional[List[int]], List[int]]]:
+        """(positions or None, sample indices) per batch of the current epoch."""
+        total = self.cache.count * self.repeat_factor
+        if self.world_invariant:
+            return world_invariant_batches(total, self.B, self.shuffle, self.seed, self.epoch, self.rank, self.world,
+                                           self.drop_last)
+        return [(None, b) for b in epoch_batches(total, self.B, self.shuffle, self.seed, self.epoch, self.rank,
+                                                 self.world, self.drop_last)]
 
     def __iter__(self) -> Iterator[dict]:
         batches = self._batches()
+        epoch = self.epoch
         self.epoch += 1
         q: "queue.Queue" = queue.Queue(maxsize=self.depth - 1)
         stop = threading.Event()
@@ -628,10 +680,10 @@ class DeviceBatchLoader:
         def worker():
             try:
                 with torch.cuda.device(self.device):
-                    for k, idxs in enumerate(batches):
+                    for k, (pos, idxs) in enumerate(batches):
                         if stop.is_set():
                             return
-                        q.put(self._produce(k, idxs))
+                        q.put(self._produce(k, idxs, pos, epoch))
                 q.put(None)
             except BaseException as exc:                      # surface loader errors in the consumer
                 q.put(exc)

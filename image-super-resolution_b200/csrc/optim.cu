@@ -5,6 +5,8 @@
 // The reference runs these as ~600 small ATen launches per step (198 tensors x 3); here it is one
 // reduction + one elementwise pass: 20 B read + 16 B written per parameter.  No host sync: the clip
 // coefficient is derived on the device from the squared-norm accumulator.
+#include <type_traits>
+
 #include "common.cuh"
 #include "../../include/ffsr_b200.h"
 
@@ -59,7 +61,55 @@ __global__ void __launch_bounds__(256) k_adamw_ema(float* __restrict__ p, const 
     if (ema) ema[i] = ema_decay * ema[i] + (1.0f - ema_decay) * pi;
   }
 }
+
+// out[i] = (...((s_0[i] + s_1[i]) + s_2[i]) ... + s_{M-1}[i]) with s_m = slots + m * pitch: one thread owns VEC
+// consecutive entries and adds the M slots in slot order, one fp32 rounding per add (__fadd_rn is never contracted
+// into an FMA), so each entry depends on its M inputs only -- not on the grid, the block size or which path ran.
+// The world-invariant training step sums its per-micro-batch gradient rows with it.
+template <int VEC>
+__global__ void __launch_bounds__(256) k_sum_slots_ordered(const float* __restrict__ slots, int M, long n, long pitch,
+                                                           float* __restrict__ out) {
+  using V = typename std::conditional<VEC == 4, float4, float>::type;
+  const long nv = n / VEC, pv = pitch / VEC;
+  const V* __restrict__ s = reinterpret_cast<const V*>(slots);
+  V* __restrict__ o = reinterpret_cast<V*>(out);
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long)gridDim.x * blockDim.x) {
+    V a = s[i];
+#pragma unroll 4
+    for (int m = 1; m < M; ++m) {
+      const V b = s[(long)m * pv + i];
+      if constexpr (VEC == 4) {
+        a.x = __fadd_rn(a.x, b.x);
+        a.y = __fadd_rn(a.y, b.y);
+        a.z = __fadd_rn(a.z, b.z);
+        a.w = __fadd_rn(a.w, b.w);
+      } else {
+        a = __fadd_rn(a, b);
+      }
+    }
+    o[i] = a;
+  }
+  if (VEC > 1 && blockIdx.x == 0 && threadIdx.x < n - nv * VEC) {   // the last n % VEC entries
+    const long i = nv * VEC + threadIdx.x;
+    float a = slots[i];
+    for (int m = 1; m < M; ++m) a = __fadd_rn(a, slots[(long)m * pitch + i]);
+    out[i] = a;
+  }
+}
 }  // namespace
+
+extern "C" int ffsr_sum_slots_ordered(const float* slots, int M, long n, long pitch, float* out, cudaStream_t stream) {
+  FFSR_REQUIRE(slots && out && M >= 1 && n >= 1 && pitch >= n, FFSR_ERR_ARG, "sum_slots_ordered: bad argument");
+  FFSR_REQUIRE(out + n <= slots || out >= slots + (long)(M - 1) * pitch + n, FFSR_ERR_ARG,
+               "sum_slots_ordered: out overlaps the slots");
+  // 16-byte loads and stores when every slot row and the output start on a 16-byte boundary
+  const bool vec = ((uintptr_t)slots % 16 == 0) && ((uintptr_t)out % 16 == 0) && (pitch % 4 == 0);
+  const long items = vec ? n / 4 : n;
+  const int grid = (int)(items <= 0 ? 1 : ((items + 255) / 256 < 148L * 8 ? (items + 255) / 256 : 148L * 8));
+  if (vec) k_sum_slots_ordered<4><<<grid, 256, 0, stream>>>(slots, M, n, pitch, out);
+  else k_sum_slots_ordered<1><<<grid, 256, 0, stream>>>(slots, M, n, pitch, out);
+  return ffsr_check_launch("sum_slots_ordered");
+}
 
 static inline int sumsq_grid(long n) { return (int)((n + 255) / 256 < 148L * 4 ? (n + 255) / 256 : 148L * 4); }
 

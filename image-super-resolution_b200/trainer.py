@@ -5,8 +5,19 @@ Mirrors the reference's cached training loop (``train.py:300-357``: forward_with
 clamp -> criterion -> backward -> clip_grad_norm_(1.0) -> AdamW.step -> EMA.update) with the
 per-tensor ATen loops replaced by two kernels over a flat bucket (``csrc/optim.cu``) and, under
 ``torchrun``, one ``ncclAllReduce`` of the 1,433,217-float gradient bucket over NVLink/NVSwitch
-(SURVEY §8e: the reference has no DDP; an N-rank step equals its own ``accumulation_steps=N`` run over
-the same N micro-batches, including per-micro-batch BatchNorm statistics).
+(SURVEY §8e: the reference has no DDP).  ``FusionTrainer(accumulation_steps=k)`` runs k micro-batches per rank and
+step, accumulating their gradients into the bucket as ``train.py:331-357`` does.  In this default mode an N-rank step
+equals its own ``accumulation_steps=N`` run only up to rounding: the all-reduce's ring order depends on N, and the
+ranks' BatchNorm running statistics are averaged EMAs.
+
+``world_invariant=True`` makes the step bitwise independent of N for a fixed sequence of M = N*k micro-batches of b
+patches: every micro-batch's gradient, BatchNorm records and loss terms go into a row of their own, ONE all-gather puts
+all M rows on every rank in micro-batch order, and every rank sums them in that order (``ffsr_sum_slots_ordered``),
+folds the BatchNorm records of all M micro-batches in one closed form and applies the optimizer with grad_scale 1/M.
+Dropout seeds are a hash of (run base, global micro-batch, call).  With the same build, GPU model, precision mode,
+``torch.manual_seed``, data and step sequence, losses, gradients, parameters, optimizer / EMA state and BatchNorm
+buffers match bit for bit for every N dividing M (feed it from ``DeviceBatchLoader(world_invariant=True)``).  With one
+micro-batch per step it is exactly the default step.
 
 ``FusedAdamW`` is a ``torch.optim.Optimizer`` so LR schedulers and ``optimizer.state_dict()`` keep
 working in an unchanged ``train.py``; parameters stay ordinary leaf ``nn.Parameter``s whose storage
@@ -111,11 +122,20 @@ class FusedAdamW(torch.optim.Optimizer):
         self._lr_dev = torch.full((1,), float(lr), device=dev, dtype=torch.float32)
         self._lr_host = float(lr)
         self.steps = 0
+        # micro-batch gradients each rank sums into `grads` per step (FusionTrainer's accumulation_steps): step()
+        # scales the all-reduced bucket by 1 / (world * micro_batches)
+        self.micro_batches = 1
+        self._grad_count = 1
         for i, p in enumerate(params):
             p.data = self.bucket.view(i)                       # same values, storage now inside the bucket
-            o = self.bucket.offsets[i]
-            p.grad = self.grads[o:o + p.numel()].view(p.shape)  # autograd accumulates in place into the bucket
+        self.attach_grads(self.grads)                          # autograd accumulates in place into the bucket
         self.sync_from_rank0()
+
+    def attach_grads(self, flat: torch.Tensor) -> None:
+        """Point every parameter's ``.grad`` at its slice of ``flat`` (a buffer laid out like the bucket)."""
+        for i, p in enumerate(self._params):
+            o = self.bucket.offsets[i]
+            p.grad = flat[o:o + p.numel()].view(p.shape)
 
     @torch.no_grad()
     def sync_from_rank0(self) -> None:
@@ -157,10 +177,18 @@ class FusedAdamW(torch.optim.Optimizer):
     def step(self, closure=None):
         loss = closure() if closure is not None else None
         self._gather_stray_grads()
-        g = self.param_groups[0]
         world = _world()
         if world > 1:
             dist.all_reduce(self.grads, op=dist.ReduceOp.SUM)   # ONE collective: the flat 5.7 MB gradient bucket
+        self.apply_summed(world * self.micro_batches)
+        return loss
+
+    @torch.no_grad()
+    def apply_summed(self, count: int) -> None:
+        """Clip + AdamW + EMA from ``grads`` holding the sum of ``count`` micro-batch gradients, each of its own mean
+        loss: the update uses their mean (grad_scale = 1 / count).  No collective."""
+        g = self.param_groups[0]
+        self._grad_count = count
         dev = self.bucket.flat.device
         capturing = torch.cuda.is_current_stream_capturing()
         if not capturing:                    # a capture records the step without running it (the replay loop counts it)
@@ -182,10 +210,9 @@ class FusedAdamW(torch.optim.Optimizer):
                 self.bucket.flat.data_ptr(), self.grads.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(),
                 self.ema.data_ptr() if self.ema is not None else None, n, float(g["lr"]), float(g["betas"][0]),
                 float(g["betas"][1]), float(g["eps"]), float(g["weight_decay"]), 0, self._step_dev.data_ptr(),
-                self._lr_dev.data_ptr(), gsq, 1.0 / world, self.max_grad_norm, float(self.ema_decay or 0.0), S),
+                self._lr_dev.data_ptr(), gsq, 1.0 / count, self.max_grad_norm, float(self.ema_decay or 0.0), S),
                 "adamw_ema_step")
         self.bump_versions()      # the kernel wrote through raw pointers: tell the version-keyed weight caches (pipeline.py)
-        return loss
 
     # -- checkpointing (train.py saves optimizer.state_dict(): src/utils/checkpoint_manager.py:120-160) --------
     def state_dict(self):
@@ -252,7 +279,7 @@ class FusedAdamW(torch.optim.Optimizer):
 
     def grad_norm(self) -> torch.Tensor:
         """Global gradient norm seen by the last step (device scalar, no sync)."""
-        return self._gsq.sqrt() / _world()
+        return self._gsq.sqrt() / self._grad_count
 
     @torch.no_grad()
     def swap_ema(self) -> None:
@@ -291,20 +318,52 @@ class FusionTrainer:
     seeds come from torch's CPU generator plus a device counter that construction resets, so two trainers built
     after the same ``torch.manual_seed`` (before the model, and on the same GPU, precision mode and inputs) give
     bitwise-identical losses, gradients, parameters, optimizer / EMA state and BatchNorm buffers, eager or
-    graph-replayed, with or without ``torch.use_deterministic_algorithms(True)``."""
+    graph-replayed, with or without ``torch.use_deterministic_algorithms(True)``.
+
+    ``accumulation_steps=k``: ``step()`` takes the rank's k*b patches and runs them as k contiguous micro-batches along
+    dim 0; the returned loss and components are their mean.  ``world_invariant=True`` (module docstring): the same
+    results for every world size N dividing M = N*k; ``global_micro_batches=M`` instead of k sets M directly and
+    raises ``ValueError`` when N does not divide it."""
 
     def __init__(self, model, criterion, lr: float = 2e-4, betas=(0.9, 0.999), eps: float = 1e-8,
                  weight_decay: float = 1e-4, max_grad_norm: float = 1.0, ema_decay: Optional[float] = 0.999,
-                 cuda_graph: bool = True, graph_warmup: int = 3):
-        from .training import seed_counter
+                 cuda_graph: bool = True, graph_warmup: int = 3, accumulation_steps: int = 1,
+                 world_invariant: bool = False, global_micro_batches: Optional[int] = None):
+        from .training import _draw_seed, seed_counter
+        world = _world()
+        if global_micro_batches is not None:
+            if not world_invariant:
+                raise ValueError("global_micro_batches needs world_invariant=True")
+            if accumulation_steps != 1:
+                raise ValueError("give accumulation_steps (per rank) or global_micro_batches, not both")
+            if global_micro_batches < 1 or global_micro_batches % world:
+                raise ValueError(f"global_micro_batches={global_micro_batches} is not a positive multiple of the "
+                                 f"world size {world}")
+            accumulation_steps = global_micro_batches // world
+        if accumulation_steps < 1:
+            raise ValueError(f"accumulation_steps must be >= 1, got {accumulation_steps}")
         self.model, self.criterion = model, criterion
         self.names = [n for n, p in model.named_parameters() if p.requires_grad]
         self.optimizer = FusedAdamW(model.parameters(), lr, betas, eps, weight_decay, max_grad_norm, ema_decay)
-        seed_counter(self.optimizer.bucket.flat.device).zero_()     # dropout masks start over with each trainer
-        if _world() > 1:                      # BatchNorm statistics / counters start from rank 0's too (parameters: FusedAdamW)
+        dev = self.optimizer.bucket.flat.device
+        seed_counter(dev).zero_()                                   # dropout masks start over with each trainer
+        if world > 1:                         # BatchNorm statistics / counters start from rank 0's too (parameters: FusedAdamW)
             for n, b in model.named_buffers():
                 if n.endswith(("running_mean", "running_var", "num_batches_tracked")):
                     dist.broadcast(b, src=0)
+        self.accumulation_steps = int(accumulation_steps)
+        self.world_invariant = bool(world_invariant)
+        self.optimizer.micro_batches = 1 if self.world_invariant else self.accumulation_steps
+        # world-invariant mode: dropout seeds hash (base, global micro-batch, call) with ONE base per run, rank 0's.
+        # A step of one micro-batch keeps the default per-call draws, so it is exactly the default step.
+        self._seed_base = None
+        if self.world_invariant and world * self.accumulation_steps > 1:
+            base = torch.tensor([_draw_seed()], dtype=torch.int64, device=dev)
+            if world > 1:
+                dist.broadcast(base, src=0)
+            self._seed_base = int(base.item())
+        self._layout = None
+        self._rows = self._rows_all = None
         self.optimizer.zero_grad()
         self.cuda_graph = cuda_graph
         self.graph_warmup = graph_warmup
@@ -313,16 +372,120 @@ class FusionTrainer:
         self._static = None
         self._sig = None
 
+    def _split(self, lr_img, expert_imgs, expert_feats, hr_img):
+        """The rank's batch as accumulation_steps contiguous micro-batches along dim 0."""
+        k = self.accumulation_steps
+        if k == 1:
+            return [(lr_img, expert_imgs, expert_feats, hr_img)]
+        B = lr_img.shape[0]
+        if B % k:
+            raise ValueError(f"a batch of {B} patches does not split into accumulation_steps={k} micro-batches")
+        b = B // k
+
+        def cut(j):
+            return (lr_img[j * b:(j + 1) * b], {n: v[j * b:(j + 1) * b] for n, v in expert_imgs.items()},
+                    {n: v[j * b:(j + 1) * b] for n, v in expert_feats.items()} if expert_feats else expert_feats,
+                    hr_img[j * b:(j + 1) * b])
+        return [cut(j) for j in range(k)]
+
     def _step_body(self, lr_img, expert_imgs, expert_feats, hr_img):
         from .training import seed_counter
-        sr = self.model.forward_with_precomputed(lr_img, expert_imgs, expert_feats).clamp(0, 1)   # train.py:326
-        loss, comps = self.criterion(sr, hr_img, return_components=True)
-        loss.backward()
+        micro = self._split(lr_img, expert_imgs, expert_feats, hr_img)
+        if self.world_invariant:
+            world = _world()
+            rows = self._local_rows(micro, (dist.get_rank() if world > 1 else 0) * len(micro))
+            if world > 1:                     # ONE collective; rank order is global micro-batch order; moves bits only
+                if self._rows_all is None or self._rows_all.shape[0] != world * rows.shape[0]:
+                    self._rows_all = rows.new_empty((world * rows.shape[0], rows.shape[1]))
+                dist.all_gather_into_tensor(self._rows_all, rows)
+                rows = self._rows_all
+            return self._finish(rows)
+        out = []
+        for lr_j, imgs_j, feats_j, hr_j in micro:      # train.py:331-357: backward per micro-batch into one bucket
+            sr = self.model.forward_with_precomputed(lr_j, imgs_j, feats_j).clamp(0, 1)   # train.py:326
+            loss, comps = self.criterion(sr, hr_j, return_components=True)
+            loss.backward()
+            out.append((loss, comps))
         self.optimizer.step()
         sync_bn_buffers(self.model)
         self.optimizer.zero_grad()
         seed_counter(lr_img.device).add_(1)
-        return loss.detach(), {k: v.detach() for k, v in comps.items()}
+        if len(out) == 1:
+            loss, comps = out[0]
+            return loss.detach(), {k: v.detach() for k, v in comps.items()}
+        k = len(out)
+        return (sum(l.detach() for l, _ in out) / k,
+                {n: sum(c[n].detach() for _, c in out) / k for n in out[0][1]})
+
+    # ---- world-invariant step: local pass -> all-gather -> finish ---------------------------------------------
+    def _local_rows(self, micro_batches, first_index: int) -> torch.Tensor:
+        """Forward + backward of the rank's micro-batches, which are global micro-batches first_index, first_index+1,
+        ...  Row j of the returned [k, L] buffer holds micro-batch j's gradient bucket (of its own mean loss,
+        unscaled), then its BatchNorm records (per BN call, in call order: mean[G,C], biased var[G,C]), then its
+        loss and loss components.  Nothing is reduced here."""
+        from .training import micro_batch
+        opt = self.optimizer
+        rows = None
+        for j, (lr_j, imgs_j, feats_j, hr_j) in enumerate(micro_batches):
+            with micro_batch(first_index + j, self._seed_base) as mb:
+                sr = self.model.forward_with_precomputed(lr_j, imgs_j, feats_j).clamp(0, 1)   # train.py:326
+            loss, comps = self.criterion(sr, hr_j, return_components=True)
+            if j == 0:
+                rows = self._row_buffer(mb.records, comps, len(micro_batches))
+            lay = self._layout
+            if [(id(r[0]),) + tuple(r[1].shape) + (r[3],) for r in mb.records] != lay["key"] or list(comps) != lay["comps"]:
+                raise RuntimeError("world-invariant step: micro-batches of one step differ in their BatchNorm calls or "
+                                   "loss components")
+            row = rows[j]
+            parts = [t.reshape(-1) for r in mb.records for t in (r[1], r[2])]
+            parts += [loss.detach().float().reshape(1)] + [comps[n].detach().float().reshape(1) for n in lay["comps"]]
+            torch.cat(parts, out=row[lay["nb"]:lay["end"]])
+            opt.attach_grads(row)             # backward accumulates into the zeroed row j
+            loss.backward()
+        return rows
+
+    def _row_buffer(self, records, comps, k: int) -> torch.Tensor:
+        """The zeroed [k, L] row buffer; its layout follows the BN calls and loss components of the first micro-batch."""
+        key = [(id(r[0]),) + tuple(r[1].shape) + (r[3],) for r in records]
+        if self._layout is None or self._layout["key"] != key or self._layout["comps"] != list(comps) \
+                or self._rows.shape[0] != k:
+            nb = self.optimizer.bucket.numel
+            bn, off = [], nb
+            for bnm, mean, _var, n in records:
+                G, Cc = mean.shape
+                bn.append((bnm, G, Cc, n, off))
+                off += 2 * G * Cc
+            loss_off = off
+            end = loss_off + 1 + len(comps)
+            L = (end + 63) // 64 * 64                 # rows start on 256-byte boundaries: 16-byte loads in the sum
+            self._layout = {"key": key, "comps": list(comps), "nb": nb, "bn": bn, "loss_off": loss_off, "end": end}
+            dev = self.optimizer.grads.device
+            self._rows = torch.zeros((k, L), device=dev, dtype=torch.float32)
+            self._loss_sum = torch.zeros(1 + len(comps), device=dev, dtype=torch.float32)
+            return self._rows
+        return self._rows.zero_()
+
+    def _finish(self, rows: torch.Tensor):
+        """The step from the gathered rows [M, L] of all M global micro-batches, identical on every rank: gradient
+        bucket and loss terms summed in micro-batch order (ffsr_sum_slots_ordered), the BatchNorm records of all M
+        micro-batches folded in one closed form, then clip + AdamW + EMA with grad_scale = 1 / M."""
+        from .training import fold_running_stats, seed_counter
+        opt, lay = self.optimizer, self._layout
+        M, L = rows.shape
+        ncomp = lay["end"] - lay["loss_off"]
+        with torch.cuda.device(rows.device):
+            S = C.c_void_p(torch.cuda.current_stream(rows.device).cuda_stream)
+            K.check(opt.lib.ffsr_sum_slots_ordered(rows.data_ptr(), M, lay["nb"], L, opt.grads.data_ptr(), S),
+                    "sum_slots_ordered")
+            K.check(opt.lib.ffsr_sum_slots_ordered(rows.data_ptr() + 4 * lay["loss_off"], M, ncomp, L,
+                                                   self._loss_sum.data_ptr(), S), "sum_slots_ordered")
+        vals = self._loss_sum / M
+        fold_running_stats([(bn, rows[i, o:o + G * Cc].view(G, Cc), rows[i, o + G * Cc:o + 2 * G * Cc].view(G, Cc), n)
+                            for i in range(M) for bn, G, Cc, n, o in lay["bn"]])
+        opt.attach_grads(opt.grads)
+        opt.apply_summed(M)
+        seed_counter(rows.device).add_(1)
+        return vals[0], {n: vals[1 + i] for i, n in enumerate(lay["comps"])}
 
     def _signature(self, lr_img, expert_imgs, expert_feats, hr_img):
         """Everything a capture bakes in: input shapes / dtypes, and the host scalars and Python control flow of the step --
@@ -335,7 +498,8 @@ class FusionTrainer:
                 tuple(sorted((k, tuple(v.shape), v.dtype) for k, v in f.items())), tuple(hr_img.shape),
                 cw, bool(getattr(crit, "use_swt", True)), bool(getattr(crit, "use_fft", True)),
                 float(g["weight_decay"]), tuple(float(b) for b in g["betas"]), float(g["eps"]),
-                float(self.optimizer.max_grad_norm), self.optimizer.ema_decay, getattr(self.model, "precision", None))
+                float(self.optimizer.max_grad_norm), self.optimizer.ema_decay, getattr(self.model, "precision", None),
+                self.accumulation_steps)
 
     def _capture(self, lr_img, expert_imgs, expert_feats, hr_img):
         self._static = (lr_img.clone(), {k: v.clone() for k, v in expert_imgs.items()},

@@ -30,6 +30,7 @@ the library works in.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import os
 from typing import Dict, List, Optional
@@ -610,7 +611,11 @@ def batchnorm_train(x, bn: torch.nn.BatchNorm2d, G: int, stats_sink: list):
 def fold_running_stats(records):
     """nn.BatchNorm2d side effect (momentum 0.1, unbiased variance, counter += 1 per call),
     applied for the G sequential LKABlock calls of one forward.  records: [(bn, mean[G,C], var[G,C], n)]
-    in call order per BN module (large_kernel_attention.py:84,128,131)."""
+    in call order per BN module (large_kernel_attention.py:84,128,131).
+
+    The records of M micro-batches, concatenated in micro-batch order, fold in one call: each module's G' = M*G
+    groups go through the same closed form and ``num_batches_tracked`` grows by M*G, as M sequential forwards would
+    leave it.  With one micro-batch this is the per-forward fold."""
     by_mod: Dict[int, list] = {}
     for bn, mean, var, n in records:
         by_mod.setdefault(id(bn), [bn, [], [], n])
@@ -704,6 +709,53 @@ def _draw_seed() -> int:
     return int(torch.randint(0, 2 ** 62, (1,)).item())
 
 
+_M64 = (1 << 64) - 1
+
+
+def _mix64(x: int) -> int:
+    """splitmix64 finaliser: a bijection of 64-bit integers."""
+    x = (x + 0x9E3779B97F4A7C15) & _M64
+    x = ((x ^ (x >> 30)) * 0xBF58476D1CE4E5B9) & _M64
+    x = ((x ^ (x >> 27)) * 0x94D049BB133111EB) & _M64
+    return x ^ (x >> 31)
+
+
+def dropout_seed(base: int, index: int, call: int) -> int:
+    """Host seed of attention call ``call`` of global micro-batch ``index`` in a world-invariant step: a fixed hash of
+    (base, index, call) in [0, 2**62), so a micro-batch draws the same masks whichever rank runs it."""
+    return _mix64(_mix64((base & _M64) ^ _mix64(index)) ^ _mix64(call & _M64)) >> 2
+
+
+class MicroBatch:
+    """State of one micro-batch of a world-invariant training step (trainer.py), set by ``micro_batch``: its global
+    index and the step's seed base key the dropout seeds (``seed_base=None``: the default ``_draw_seed`` draws), and
+    the forward appends its BatchNorm records to ``records`` instead of folding them, so the step can fold every
+    micro-batch's records in global order."""
+
+    def __init__(self, index: int, seed_base: Optional[int]):
+        self.index, self.seed_base, self.calls, self.records = int(index), seed_base, 0, []
+
+    def seed(self) -> int:
+        if self.seed_base is None:
+            return _draw_seed()
+        self.calls += 1
+        return dropout_seed(self.seed_base, self.index, self.calls - 1)
+
+
+_MICRO: Optional[MicroBatch] = None
+
+
+@contextlib.contextmanager
+def micro_batch(index: int, seed_base: Optional[int]):
+    """``with micro_batch(i, base) as mb:`` -- train-mode forwards inside run as global micro-batch i (see MicroBatch)."""
+    global _MICRO
+    prev, _MICRO = _MICRO, MicroBatch(index, seed_base)
+    try:
+        yield _MICRO
+    finally:
+        _MICRO = prev
+
+
 _SEED_COUNTERS: Dict[str, torch.Tensor] = {}
 _CHECKED = set()
 
@@ -724,7 +776,8 @@ def mha_tokens(x, mha: torch.nn.MultiheadAttention, B: int, T: int, training: bo
     x: [B*T, E, H, W] channels-last token-major.  (large_kernel_attention.py:192-197, 294-299)"""
     qkv = conv2d(x, mha.in_proj_weight, mha.in_proj_bias, tc)
     p = float(mha.dropout) if training else 0.0
-    ctx = _TokenAttention.apply(qkv, B, T, p, _draw_seed() if p > 0 else 0, seed_counter(x.device) if p > 0 else None)
+    seed = (_MICRO.seed() if _MICRO is not None else _draw_seed()) if p > 0 else 0
+    ctx = _TokenAttention.apply(qkv, B, T, p, seed, seed_counter(x.device) if p > 0 else None)
     return conv2d(ctx, mha.out_proj.weight, mha.out_proj.bias, tc)
 
 
@@ -1140,7 +1193,10 @@ def _train_forward(m, lr, img_list, feats, want_inter):
         out = out.clamp(0, 1)
     out = out.contiguous()
     if training:
-        fold_running_stats(sink)
+        if _MICRO is not None:
+            _MICRO.records.extend(sink)
+        else:
+            fold_running_stats(sink)
     if want_inter:
         inter["raw_9_bands"] = [raw9[:, i] for i in range(9)]
         inter["guidance_bands"] = inter["raw_9_bands"][:3]

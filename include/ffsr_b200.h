@@ -376,12 +376,17 @@ int ffsr_loss_fft(const float* pred, const float* target, int P, int H, int W, f
  *   gsumsq is NULL or max_norm <= 0); torch.optim.AdamW update with bias correction for `step` (1-based)
  *   (train.py:847-853); ema = decay*ema + (1-decay)*p (checkpoint_manager.py:352-359; ema may be NULL).
  *   step_dev / lr_dev (optional device scalars): effective step = step + *step_dev, lr = *lr_dev -- the values
- *   that change between replays of a CUDA-graph-captured training step. */
+ *   that change between replays of a CUDA-graph-captured training step.
+ * ffsr_sum_slots_ordered: out[i] = (...((s_0[i] + s_1[i]) + s_2[i]) ... + s_{M-1}[i]), s_m = slots + m*pitch, i < n
+ *   (pitch >= n floats; out must not overlap the slots).  One fp32 rounding per add, in slot order: the result is
+ *   what a float32 left fold gives and depends on nothing else (grid, block size, alignment).  16-byte loads when
+ *   slots, out and pitch allow.  Sums the per-micro-batch gradient rows of the world-invariant training step. */
 size_t ffsr_sumsq_workspace_bytes(long n);
 int ffsr_sumsq(const float* g, long n, double* out, void* ws, size_t ws_bytes, cudaStream_t stream);
 int ffsr_adamw_ema_step(float* p, const float* g, float* m, float* v, float* ema, long n, float lr, float beta1,
                         float beta2, float eps, float weight_decay, int step, const int* step_dev, const float* lr_dev,
                         const double* gsumsq, float grad_scale, float max_norm, float ema_decay, cudaStream_t stream);
+int ffsr_sum_slots_ordered(const float* slots, int M, long n, long pitch, float* out, cudaStream_t stream);
 
 /* ---- bf16 / tcgen05 training path ------------------------------------------------------------
  * ffsr_to_bf16_nhwc: strided fp32/bf16 view (NCHW or NHWC) -> dense bf16 channels-last with the channel
