@@ -103,10 +103,11 @@ __global__ void __launch_bounds__(WT_THREADS) k_window_attn_tc(const __nv_bfloat
     pix[t] = yo * W + xo;
     rid[t] = shift ? (uint8_t)(wt_region(ys, H, shift) * 3 + wt_region(xs, W, shift)) : 0;
   }
-  // zero Q / K / V planes (element-wise gather: the padding channels dh..DP-1 must be zero; head-padded rows carry their zeros)
+  // zero K / V planes (element-wise gather: the padding channels dh..DP-1 must be zero; head-padded rows carry their zeros).
+  // Q is not zeroed here: the bias table overwrites its planes after every S, so each tile's Q gather writes all DP channels.
   if (!HEADPAD) {
-    uint4* z = reinterpret_cast<uint4*>(sQ);
-    const int n16 = (128 * DP * 2 + 2 * WT_N * DP * 2) / 16;
+    uint4* z = reinterpret_cast<uint4*>(sK);
+    const int n16 = (2 * WT_N * DP * 2) / 16;
     for (int i = tid; i < n16; i += WT_THREADS) z[i] = make_uint4(0u, 0u, 0u, 0u);
   }
   tc_fence_before();
@@ -190,10 +191,12 @@ __global__ void __launch_bounds__(WT_THREADS) k_window_attn_tc(const __nv_bfloat
       size_t row[8];
 #pragma unroll
       for (int u = 0; u < 8; ++u) row[u] = (img + (size_t)pix[mt * 128 + r0 + u]) * (size_t)qp + (size_t)(h * dh);
-      for (int d = lane; d < dh; d += 32) {
+      // channels dh..DP-1 are written as zeros: for dh < 16 they share planes 0 / 1 with the table of the previous tile, whose
+      // bytes can read as bf16 Inf / NaN, and Inf x the zero K padding is NaN in the MMA
+      for (int d = lane; d < DP; d += 32) {
         __nv_bfloat16 qv[8];
 #pragma unroll
-        for (int u = 0; u < 8; ++u) qv[u] = qkv[row[u] + d];
+        for (int u = 0; u < 8; ++u) qv[u] = d < dh ? qkv[row[u] + d] : __float2bfloat16_rn(0.f);
 #pragma unroll
         for (int u = 0; u < 8; ++u) *reinterpret_cast<__nv_bfloat16*>(sQ + (d >> 3) * 2048 + (r0 + u) * 16 + (d & 7) * 2) = qv[u];
       }

@@ -80,9 +80,14 @@ def test_module_mirror_has_the_reference_state_layout():
         D.DRCT(upsampler="nearest+conv")
 
 
-@pytest.mark.parametrize("precision", ["fp32", "bf16"])
-def test_drct_launch_sequence_dry_run(precision):
-    """Every line of the orchestration runs against a recording fake of the library (no compute without a GPU)."""
+@pytest.mark.parametrize("precision,ws,headpad", [pytest.param("fp32", 8, True, id="fp32"), pytest.param("bf16", 8, True, id="bf16"),
+                                                  pytest.param("fp32", 16, True, id="fp32-ws16"),
+                                                  pytest.param("bf16", 16, True, id="bf16-ws16"),
+                                                  pytest.param("bf16", 16, False, id="bf16-ws16-plain-qkv")])
+def test_drct_launch_sequence_dry_run(precision, ws, headpad):
+    """Every line of the orchestration runs against a recording fake of the library (no compute without a GPU).  bf16 mode
+    at window 16 writes head-padded qkv rows (Cout = 3 heads DP) and runs ffsr_window_attention_headpadded on exactly those
+    rows; headpad_qkv = False (FFSR_DRCT_QKV_PLAIN) runs the pitched entry point instead."""
     import ctypes as C
     import isr_b200  # noqa: F401
     from isr_b200 import drct as D
@@ -98,20 +103,65 @@ def test_drct_launch_sequence_dry_run(precision):
             f.__name__ = name
             return f
 
+        def ffsr_window_attention_head_pad(self, dh):
+            return (dh + 15) // 16 * 16
+
     n = 2
-    m = D.DRCT(img_size=16, window_size=8, depths=[6] * n, num_heads=[6] * n).eval()
+    m = D.DRCT(img_size=2 * ws, window_size=ws, depths=[6] * n, num_heads=[6] * n).eval()
     m.precision = precision
+    m.headpad_qkv = headpad
     lib = Fake()
-    y = m._run(torch.rand(1, 3, 16, 24), lib, C.c_void_p(0))
-    assert tuple(y.shape) == (1, 3, 64, 96) and tuple(m.last_feature.shape) == (1, 180, 16, 24)
+    H, W = 2 * ws, 3 * ws
+    y = m._run(torch.rand(1, 3, H, W), lib, C.c_void_p(0))
+    assert tuple(y.shape) == (1, 3, 4 * H, 4 * W) and tuple(m.last_feature.shape) == (1, 180, H, W)
     names = [c[0] for c in lib.calls]
     # bf16 mode: conv_after_body runs twice (the cached fp32 feature; x0 + conv as the bf16 input of the tcgen05 tail)
     assert names.count("ffsr_conv2d") == 1 + 25 * n + 5 + (1 if precision == "bf16" else 0)
     assert names.count("ffsr_layernorm_strided") == 1 + 10 * n + 1
-    att = "ffsr_window_attention_pitched" if precision == "bf16" else "ffsr_window_attention"
-    assert names.count(att) == 5 * n and names.count("ffsr_leaky_relu") == 4 * n + 1
+    hp = precision == "bf16" and ws == 16 and headpad
+    att = "ffsr_window_attention_headpadded" if hp else ("ffsr_window_attention_pitched" if precision == "bf16" else "ffsr_window_attention")
+    others = {"ffsr_window_attention_headpadded", "ffsr_window_attention_pitched", "ffsr_window_attention"} - {att}
+    assert names.count(att) == 5 * n and not any(names.count(o) for o in others)
+    assert names.count("ffsr_leaky_relu") == 4 * n + 1
     assert names.count("ffsr_pixel_shuffle2") == 2 and names[0] == "ffsr_rgb_shift_in" and names[-1] == "ffsr_rgb_shift_out"
-    heads = [c[1][5] if precision == "fp32" else c[1][6] for c in lib.calls if c[0] == att]
+    hi, si = (5, 7) if att != "ffsr_window_attention_pitched" else (6, 8)
+    heads = [c[1][hi] for c in lib.calls if c[0] == att]
     assert heads[:5] == [6, 4, 2, 6, 4]
-    shifts = [c[1][7] if precision == "fp32" else c[1][8] for c in lib.calls if c[0] == att]
-    assert shifts[:5] == [0, 4, 0, 4, 0]
+    shifts = [c[1][si] for c in lib.calls if c[0] == att]
+    assert shifts[:5] == [0, ws // 2] * 2 + [0]
+    if hp:                                              # the qkv conv right before each launch writes its input rows
+        for i, (name, a) in enumerate(lib.calls):
+            if name == att:
+                d, h = a[4], a[5]
+                conv = lib.calls[i - 1]
+                assert conv[0] == "ffsr_conv2d"
+                p = conv[1][0]._obj
+                assert (p.Cin, p.Cout, p.ksize) == (d, 3 * h * ((d // h + 15) // 16 * 16), 1)
+                assert p.out == a[0] and a[6] == ws and a[10] == (d + 7) // 8 * 8
+
+
+def test_headpadded_qkv_weights():
+    """bf16 mode at window 16: the packed `.attn.qkvp` Linear of DRCT._weights writes the rows [q|k|v] x heads x DP whose
+    [3][heads][:dh] slices are the module's own qkv Linear and whose padding channels are exactly 0 (the tcgen05 window
+    attention multiplies them with each other)."""
+    import isr_b200  # noqa: F401
+    from isr_b200 import drct as D
+    torch.manual_seed(0)
+    m = D.DRCT(img_size=32, window_size=16, depths=[6], num_heads=[6]).eval()
+    for mod in m.modules():                             # non-zero biases: a misplaced bias row shows too
+        if isinstance(mod, torch.nn.Linear):
+            torch.nn.init.normal_(mod.bias)
+    w = m._weights(torch.device("cpu"))
+    x = torch.randn(5, 7, 308)
+    for j in range(5):
+        sw = getattr(m.layers[0], f"swin{j + 1}")
+        d, heads = sw.dim, sw.heads
+        dh = d // heads
+        DP = (dh + 15) // 16 * 16
+        p = f"layers.0.swin{j + 1}.attn"
+        assert tuple(w[p + ".qkvp"].shape) == (1, d, 3 * heads * DP) and tuple(w[p + ".qkvp.b"].shape) == (3 * heads * DP,)
+        xd = x[..., :d].double()
+        got = (xd @ w[p + ".qkvp"][0].double() + w[p + ".qkvp.b"].double()).view(5, 7, 3, heads, DP)
+        want = torch.nn.functional.linear(xd, sw.attn.qkv.weight.detach().double(), sw.attn.qkv.bias.detach().double()).view(5, 7, 3, heads, dh)
+        assert float((got[..., :dh] - want).abs().max()) < 1e-12, (j, d, heads)
+        assert bool((got[..., dh:] == 0).all()), (j, d, heads)
