@@ -26,15 +26,21 @@
 //               tile (~2k issue cycles) hides under the MMAs of the next one.
 // Persistent: grid = min(tiles, #SMs), static round-robin over tiles.
 //
-// Three tile geometries, chosen per layer in ffsr_conv2d_tc:
+// Four tile geometries, chosen per layer in ffsr_conv2d_tc:
 //   g0   : the 8x16-pixel tile described above (1x1 layers; 3x3 layers only as a fallback);
-//   g0x2 : 16x16-pixel tiles = two M=128 MMAs per (tap, K-step) that share every STREAMED weight stage (128->128 3x3,
-//          whose nine-tap weight set does not fit beside the A stages);
+//   g0x2 : 16x16-pixel tiles = two M=128 MMAs per (tap, K-step) that share every STREAMED weight stage (3x3 layers whose
+//          nine-tap weight set does not fit beside the A stages, when g3 cannot take them);
 //   g1   : 16x8-pixel tiles fed by ONE haloed copy {64 ch, 10 px, 18 rows} per 64-channel chunk -- every other 3x3
 //          layer.  Measured: the 128-byte swizzle of tcgen05 shared-memory operands is a function of the ABSOLUTE
 //          shared-memory address, so the operand of tap (dy, dx) is the same copy at byte offset dy*1280 + dx*128
 //          (SBO = 1280, base offset 0).  These layers were bound by the L2 -> shared-memory traffic of three haloed
 //          copies per tile, not by the tensor pipe.
+//   g3   : SWAPPED operands for the streamed-weight 3x3 layers with bf16 inference outputs (128->128 refinement convs):
+//          D[cout, pixel], the weights are the M=128 operand (single-tap 16 KB stages in a ring of 8) and an 8 px x 32 row
+//          tile is the N=256 operand, fed by one haloed copy {64 ch, 10 px, 34 rows} per K chunk (ring of 2) with the
+//          g1 tap offsets.  One M128 x N256 x K16 MMA reads 12 KB of shared memory per 128 cycles where the two
+//          M128 x N128 MMAs of g0x2 read 16 KB: the refinement layers were bound by shared-memory operand bandwidth.
+//          The transposing epilogue (swapped_epilogue) has one output channel per thread.
 // Epilogue extras for the training graph: an optional bf16 copy of the pre-activation (out2) and FFSR_EPI_ACTGRAD
 // (input gradient multiplied by act'(saved pre-activation of the previous layer)).
 #include <cuda.h>
@@ -59,7 +65,7 @@ constexpr int TC_EPI_WARP0 = 1 + TC_MMA_WARPS; // first epilogue warp
 constexpr int TC_THREADS = 32 * (TC_EPI_WARP0 + TC_EPI_WARPS);
 constexpr int TC_TMEM_COLS = 512;             // whole TMEM: ring of 512/slot accumulators (1 CTA per SM)
 constexpr int TC_MAX_ACC = 12;
-constexpr int TC_MAX_ASLOTS = 4;              // geom 2: activation ring depth limit
+constexpr int TC_MAX_ASLOTS = 2;              // geom 3: activation ring depth
 
 struct TcArgs {
   int N, H, W, Cin, Cout, taps, ks;
@@ -94,9 +100,9 @@ struct TcArgs {
   int halves;        // 1: tile = 8x16 px (M=128); 2: tile = 16x16 px as two M=128 MMAs sharing every weight stage
   int acc_half;      // TMEM columns of one half accumulator (acc_slot = halves * acc_half)
   int geom;          // 0: 8x16-px tile rows, one haloed A copy per dx;  1: 16x8-px tiles, ONE haloed copy per K chunk;
-                     // 2: streamed weights, 16x16-px tiles as two 16x8 halves: ONE haloed copy {64 ch, 18 px, 18 rows} per K chunk
-                     //    in its own ring + a ring of single-tap weight stages (see the kernel)
-  int tile_h;        // output rows per tile (8 * halves, or 16 for geom 1)
+                     // 3: swapped operands (weights = M, 8x32-px tile = N = 256): ONE haloed copy {64 ch, 10 px, 34 rows} per
+                     //    K chunk in its own ring + a ring of single-tap weight stages (see the kernel)
+  int tile_h;        // output rows per tile (8 * halves, 16 for geom 1, 32 for geom 3)
   uint32_t a_step16; // geom 1: dy stride inside the haloed copy, in 16-byte units (10 px * 128 B)
   uint32_t a_desc_hi;// geom 1: A descriptor high word (SBO = haloed image-row pitch)
   int gelu_tanh;     // tanh-form GELU for bf16 outputs of inference launches (see gelu_tanh_fast)
@@ -106,8 +112,8 @@ struct TcArgs {
   int nmma;          // MMA-issuing warps (1, 2 or 3): warp 1+g issues the MMAs of tiles g, g+nmma, ... of this CTA
   int nb_fast;       // 1: the cout block varies FASTEST in the tile walk (multi-block 1x1 layers with streamed weights): the CTAs
                      //    of a wave then work on the same few pixel tiles, whose activations stay in L2 across the cout blocks
-  int a_slot;        // geom 2: bytes of one slot of the activation ring (haloed copy rounded up to 1 KB)
-  int na_slots;      // geom 2: slots of the activation ring (the weight ring has nstages slots of stage_bytes)
+  int a_slot;        // geom 3: bytes of one slot of the activation ring (haloed copy rounded up to 1 KB)
+  int na_slots;      // geom 3: slots of the activation ring (the weight ring has nstages slots of stage_bytes)
 };
 
 // ---------------------------------------------------------------------------- PTX wrappers
@@ -654,20 +660,19 @@ __device__ __forceinline__ void lean_epilogue(const TcArgs& a, uint64_t* tfull, 
     }
     const int n = ti.n;
     const int cb = ti.nb * a.nblk;                      // first output column of this cout block
-    const int x0 = (a.geom == 2 ? ti.tx * 16 : ti.tx * tw) + px;
+    const int x0 = ti.tx * tw + px;
     if (MODE == EM_RESIDUAL) {
       // the residual rows of this thread's pixels are fetched towards L1 BEFORE the wait for the accumulator: their loads sat
       // behind the TMEM load in every chunk, and a residual layer cost twice its plain twin (stage3.r2 0.25 vs r0 0.11 ms)
       for (int half = 0; half < halves; ++half) {
-        const int xx = a.geom == 2 ? x0 + half * 8 : x0;
-        const int yy = ti.ty * a.tile_h + (a.geom == 2 ? 0 : half * TC_TH) + py;
-        if (yy < a.H && xx < a.W) {
-          const long long e1 = (long long)n * a.r1_sN + (long long)yy * a.r1_sY + (long long)xx * a.r1_sX + cb + c_lo * 16;
+        const int yy = ti.ty * a.tile_h + half * TC_TH + py;
+        if (yy < a.H && x0 < a.W) {
+          const long long e1 = (long long)n * a.r1_sN + (long long)yy * a.r1_sY + (long long)x0 * a.r1_sX + cb + c_lo * 16;
           const char* p1 = reinterpret_cast<const char*>(a.r1) + e1 * (a.r1_bf16 ? 2 : 4);
           const int bytes1 = (c_hi - c_lo) * 16 * (a.r1_bf16 ? 2 : 4);
           for (int o = 0; o < bytes1; o += 128) asm volatile("prefetch.global.L1 [%0];" ::"l"(p1 + o));
           if (has_r2) {
-            const long long e2 = (long long)n * a.r2_sN + (long long)yy * a.r2_sY + (long long)xx * a.r2_sX + cb + c_lo * 16;
+            const long long e2 = (long long)n * a.r2_sN + (long long)yy * a.r2_sY + (long long)x0 * a.r2_sX + cb + c_lo * 16;
             const char* p2 = reinterpret_cast<const char*>(a.r2) + e2 * (a.r2_bf16 ? 2 : 4);
             const int bytes2 = (c_hi - c_lo) * 16 * (a.r2_bf16 ? 2 : 4);
             for (int o = 0; o < bytes2; o += 128) asm volatile("prefetch.global.L1 [%0];" ::"l"(p2 + o));
@@ -678,14 +683,13 @@ __device__ __forceinline__ void lean_epilogue(const TcArgs& a, uint64_t* tfull, 
     mbar_wait(&tfull[as], aph);
     tc_fence_after();
     for (int half = 0; half < halves; ++half) {
-      const int x = a.geom == 2 ? x0 + half * 8 : x0;   // geom 2: the halves are the left / right 8 pixels of 16 rows
-      const int y = ti.ty * a.tile_h + (a.geom == 2 ? 0 : half * TC_TH) + py;
-      const bool inside = (y < a.H) && (x < a.W);
-      const long long opix = (long long)n * a.out_sN + (long long)y * a.out_sY + (long long)x * a.out_sX + cb;
+      const int y = ti.ty * a.tile_h + half * TC_TH + py;
+      const bool inside = (y < a.H) && (x0 < a.W);
+      const long long opix = (long long)n * a.out_sN + (long long)y * a.out_sY + (long long)x0 * a.out_sX + cb;
       long long r1pix = 0, r2pix = 0;
       if (MODE == EM_RESIDUAL) {
-        r1pix = (long long)n * a.r1_sN + (long long)y * a.r1_sY + (long long)x * a.r1_sX + cb;
-        if (has_r2) r2pix = (long long)n * a.r2_sN + (long long)y * a.r2_sY + (long long)x * a.r2_sX + cb;
+        r1pix = (long long)n * a.r1_sN + (long long)y * a.r1_sY + (long long)x0 * a.r1_sX + cb;
+        if (has_r2) r2pix = (long long)n * a.r2_sN + (long long)y * a.r2_sY + (long long)x0 * a.r2_sX + cb;
       }
       const uint32_t taddr = tmem_base + ((uint32_t)(wq * 32) << 16) + (uint32_t)(as * a.acc_slot + half * a.acc_half);
       for (int c0 = c_lo; c0 < c_hi; c0 += 2) {
@@ -712,6 +716,119 @@ __device__ __forceinline__ void lean_epilogue(const TcArgs& a, uint64_t* tfull, 
   }
 }
 
+// ---------------------------------------------------------------------------- swapped epilogue (geom 3)
+// The accumulator is D[cout, pixel]: TMEM lane = output channel, column j = pixel (row j / 8, column j % 8) of the 8x32 tile.
+// Warp w reads lane quarter w % 4 (channels 32 (w%4) .. +31 of the cout block, one per thread, so the bias is one register)
+// and column quarter (w - 4) / 4 (tile rows 8 q .. 8 q + 7).  After tcgen05.ld a thread holds one channel of consecutive
+// pixels; one shfl.xor 1 per two values turns that into two adjacent channels of one pixel, so the 32 lanes of a warp store
+// two pixels x 64 contiguous bytes per 4-byte store instruction.  Element math and bf16 rounding are those of lean_chunk.
+template <int MODE, bool TANH>
+__device__ __forceinline__ void swapped_rows2(const uint32_t (&v)[16], float bv, int odd, __nv_bfloat16* __restrict__ o,
+                                              const TcArgs& a, long long r1off, long long r2off, int r0, int rows, int cols,
+                                              bool cok, float sa, float sb, bool has_r2) {
+  float f[16];
+#pragma unroll
+  for (int k = 0; k < 16; ++k) {
+    f[k] = __uint_as_float(v[k]) + bv;
+    if (MODE == EM_GELU) f[k] = TANH ? gelu_tanh_fast(f[k]) : gelu_fast(f[k]);
+    else if (MODE == EM_RELU) f[k] = fmaxf(f[k], 0.f);
+    else if (MODE == EM_SIGMOID) f[k] = sigmoid_acc(f[k]);
+  }
+#pragma unroll
+  for (int j = 0; j < 16; j += 2) {
+    // columns j, j + 1: the even lane keeps pixel j, the odd lane pixel j + 1, each for channels (ce, ce + 1)
+    const float recv = __shfl_xor_sync(0xffffffffu, odd ? f[j] : f[j + 1], 1);
+    float lo = odd ? recv : f[j], hi = odd ? f[j + 1] : recv;
+    const int r = r0 + (j >> 3), px = j & 7;
+    if (cok && r < rows && px < cols) {
+      const int oo = r * (int)a.out_sY + px * (int)a.out_sX;
+      if (MODE == EM_RESIDUAL) {
+        const int o1 = r * (int)a.r1_sY + px * (int)a.r1_sX;
+        float2 r1;
+        if (a.r1_bf16) r1 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(reinterpret_cast<const __nv_bfloat16*>(a.r1) + r1off + o1));
+        else r1 = __ldg(reinterpret_cast<const float2*>(reinterpret_cast<const float*>(a.r1) + r1off + o1));
+        lo = fmaf(sa, lo, r1.x);
+        hi = fmaf(sa, hi, r1.y);
+        if (has_r2) {
+          const int o2 = r * (int)a.r2_sY + px * (int)a.r2_sX;
+          float2 r2;
+          if (a.r2_bf16) r2 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(reinterpret_cast<const __nv_bfloat16*>(a.r2) + r2off + o2));
+          else r2 = __ldg(reinterpret_cast<const float2*>(reinterpret_cast<const float*>(a.r2) + r2off + o2));
+          lo = fmaf(sb, r2.x, lo);
+          hi = fmaf(sb, r2.y, hi);
+        }
+      }
+      __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+      *reinterpret_cast<__nv_bfloat162*>(o + oo) = h;
+    }
+  }
+}
+
+template <int MODE, bool TANH>
+__device__ __forceinline__ void swapped_epilogue(const TcArgs& a, uint64_t* tfull, uint64_t* tempty, uint32_t tmem_base, int warp,
+                                                 int lane) {
+  const int wq = warp & 3;
+  const int cq = (warp - TC_EPI_WARP0) >> 2;
+  const int odd = lane & 1;
+  float sa = 1.f, sb = 1.f;
+  if (MODE == EM_RESIDUAL) {
+    sa = a.sa * (a.sa_ptr ? a.sa_ptr[0] : 1.0f);
+    sb = a.sb * (a.sb_ptr ? a.sb_ptr[0] : 1.0f);
+  }
+  const bool has_r2 = MODE == EM_RESIDUAL && a.r2 != nullptr;
+  __nv_bfloat16* const outp = reinterpret_cast<__nv_bfloat16*>(a.out);
+  int as = 0;
+  uint32_t aph = 0;
+  TileIter ti;
+  for (ti.init(a); ti.valid(a); ti.next(a)) {
+    const int n = ti.n;
+    const int co = ti.nb * 128 + wq * 32 + lane;       // this thread's accumulator lane
+    const float bv = (a.bias != nullptr && co < a.Cout) ? __ldg(a.bias + co) : 0.f;
+    const int ce = co - odd;                            // first of the two channels this thread stores (Cout is even)
+    const bool cok = ce < a.Cout;
+    const int y0 = ti.ty * 32 + cq * 8, x0 = ti.tx * 8 + odd;
+    const int rows = a.H - y0, cols = a.W - x0;         // valid tile rows from y0 / stored columns px (+ odd) from x0
+    const long long opix = (long long)n * a.out_sN + (long long)y0 * a.out_sY + (long long)x0 * a.out_sX + ce;
+    long long r1pix = 0, r2pix = 0;
+    if (MODE == EM_RESIDUAL) {
+      r1pix = (long long)n * a.r1_sN + (long long)y0 * a.r1_sY + (long long)x0 * a.r1_sX + ce;
+      if (has_r2) r2pix = (long long)n * a.r2_sN + (long long)y0 * a.r2_sY + (long long)x0 * a.r2_sX + ce;
+      // the 64 pixels x 32 channels this warp adds are fetched towards L1 before the wait for the accumulator
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int p = lane + 32 * h, r = p >> 3, px = p & 7;
+        if (r < rows && px < a.W - ti.tx * 8 && ti.nb * 128 + wq * 32 < a.Cout) {
+          const long long e1 = (long long)n * a.r1_sN + (long long)(y0 + r) * a.r1_sY + (long long)(ti.tx * 8 + px) * a.r1_sX + ti.nb * 128 + wq * 32;
+          asm volatile("prefetch.global.L1 [%0];" ::"l"(reinterpret_cast<const char*>(a.r1) + e1 * (a.r1_bf16 ? 2 : 4)));
+          if (has_r2) {
+            const long long e2 = (long long)n * a.r2_sN + (long long)(y0 + r) * a.r2_sY + (long long)(ti.tx * 8 + px) * a.r2_sX + ti.nb * 128 + wq * 32;
+            asm volatile("prefetch.global.L1 [%0];" ::"l"(reinterpret_cast<const char*>(a.r2) + e2 * (a.r2_bf16 ? 2 : 4)));
+          }
+        }
+      }
+    }
+    mbar_wait(&tfull[as], aph);
+    tc_fence_after();
+    const uint32_t taddr = tmem_base + ((uint32_t)(wq * 32) << 16) + (uint32_t)(as * a.acc_slot + cq * 64);
+#pragma unroll 1
+    for (int h = 0; h < 2; ++h) {                       // 32 columns = 4 tile rows per pass
+      uint32_t v0[16], v1[16];
+      tmem_ld16(taddr + (uint32_t)(h * 32), v0);
+      tmem_ld16(taddr + (uint32_t)(h * 32 + 16), v1);
+      tmem_wait_ld(v0);
+      tmem_wait_ld(v1);
+      if (h == 1) {                                     // every column of this warp is in registers: free the accumulator
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&tempty[as]);
+      }
+      swapped_rows2<MODE, TANH>(v0, bv, odd, outp + opix, a, r1pix, r2pix, 4 * h, rows, cols, cok, sa, sb, has_r2);
+      swapped_rows2<MODE, TANH>(v1, bv, odd, outp + opix, a, r1pix, r2pix, 4 * h + 2, rows, cols, cok, sa, sb, has_r2);
+    }
+    if (++as == a.nacc) { as = 0; aph ^= 1; }
+  }
+}
+
 // ---------------------------------------------------------------------------- the kernel
 __global__ void __launch_bounds__(TC_THREADS, 1)
 k_conv_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const TcArgs a) {
@@ -724,7 +841,7 @@ k_conv_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
   uint64_t* tempty = bars + 2 * TC_MAX_STAGES + TC_MAX_ACC;    // [TC_MAX_ACC]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * TC_MAX_STAGES + 2 * TC_MAX_ACC);
   uint64_t* bfull = bars + 2 * TC_MAX_STAGES + 2 * TC_MAX_ACC + 1;   // resident-weights barrier
-  uint64_t* afull = bfull + 1;                                       // geom 2: activation ring [TC_MAX_ASLOTS]
+  uint64_t* afull = bfull + 1;                                       // geom 3: activation ring [TC_MAX_ASLOTS]
   uint64_t* aempty = afull + TC_MAX_ASLOTS;
   float* sbias = reinterpret_cast<float*>(smem + TC_BIAS_OFF);       // lean epilogue: bias of every output column
   uint8_t* bres = smem + TC_SMEM_HDR;                                // resident weights (may be empty)
@@ -766,7 +883,7 @@ k_conv_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
       int cur_g = -1, cur_nb = -1, last_s = 0;
       uint32_t last_ph = 0;
       bool have_last = false;
-      int as_ = 0;                                   // geom 2: activation ring position
+      int as_ = 0;                                   // geom 3: activation ring position
       uint32_t aph_ = 0;
       uint8_t* const wring = stages + a.na_slots * a.a_slot;
       TileIter ti;
@@ -783,22 +900,20 @@ k_conv_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
           cur_g = g;
           cur_nb = nb;
         }
-        if (a.geom == 2) {
-          // Streamed weights with a deep pipeline: the 128->128 layers used 86 KB stages (one haloed copy per dx + the
-          // three dy taps of the weights), i.e. a ring of TWO -- every stage load was exposed behind ~1,500 cycles of
-          // MMAs (ncu: tensor pipe 59 % active).  Here the activations of a K chunk are ONE haloed copy
-          // {64 ch, 18 px, 18 rows} (41 KB instead of 3 x 36 KB) in their own ring, and the weights stream through a ring
-          // of single-tap 16 KB stages (8 deep = ~4,000 cycles of MMAs ahead).
+        if (a.geom == 3) {
+          // Streamed weights with a deep pipeline: the activations of a K chunk are ONE haloed copy {64 ch, 10 px, 34 rows}
+          // (43.5 KB) in their own ring, and the weights stream through a ring of single-tap 16 KB stages (8 deep =
+          // ~8,000 cycles of MMAs ahead).
           for (int ch = 0; ch < a.nchunks; ++ch) {
             mbar_wait(&aempty[as_], aph_ ^ 1);
             mbar_expect_tx_e(&afull[as_], (uint32_t)a.a_bytes);
-            tma_load_4d(stages + as_ * a.a_slot, &tmA, &afull[as_], ch * 64, tx * 16 - pad, ty * 16 - pad, n);
+            tma_load_4d(stages + as_ * a.a_slot, &tmA, &afull[as_], ch * 64, tx * 8 - 1, ty * 32 - 1, n);
             if (++as_ == a.na_slots) { as_ = 0; aph_ ^= 1; }
             for (int dxi = 0; dxi < 3; ++dxi)
               for (int dyi = 0; dyi < 3; ++dyi) {
                 mbar_wait(&empty[s], ph ^ 1);
                 mbar_expect_tx_e(&full[s], (uint32_t)a.b_bytes);
-                tma_load_5d(wring + s * a.stage_bytes, &tmB, &full[s], ch * 64, nb * a.nblk, dxi, dyi, g);
+                tma_load_5d(wring + s * a.stage_bytes, &tmB, &full[s], ch * 64, nb * 128, dxi, dyi, g);
                 if (++s == a.nstages) { s = 0; ph ^= 1; }
               }
           }
@@ -837,7 +952,8 @@ k_conv_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
     const int g = warp - 1;
     if (g < a.nmma) {
     const int nmma = a.nmma;
-    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(a.nblk >> 3) << 17) | ((128u >> 4) << 24);
+    const uint32_t umma_n = a.geom == 3 ? 256u : (uint32_t)a.nblk;   // geom 3: N = the 256 pixels of a tile
+    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((umma_n >> 3) << 17) | ((128u >> 4) << 24);
     const int k0 = g * kiters;
     int s = k0 % a.nstages;
     uint32_t ph = (uint32_t)((k0 / a.nstages) & 1);
@@ -849,8 +965,8 @@ k_conv_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
     const uint32_t b_step = (uint32_t)(a.nblk * 128) >> 4;
     const int last_chunk_it = a.geom ? a.nchunks - 1 : (a.nchunks - 1) * a.ks;   // stages of the last (possibly partial) K chunk
     const int skip = (nmma - 1) * kiters;
-    int g2_as = 0;                                  // geom 2: activation ring position
-    uint32_t g2_aph = 0;
+    int g3_as = 0;                                  // geom 3: activation ring position
+    uint32_t g3_aph = 0;
     TileIter ti;
     ti.init(a);                                     // tile coordinates matter only for weight-set changes (nmma == 1)
     for (int q = 0; q < g; ++q) ti.next(a);
@@ -868,37 +984,35 @@ k_conv_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
       mbar_wait(&tempty[as], aph ^ 1);
       tc_fence_after();
       const uint32_t tmem_d = tmem_base + (uint32_t)(as * a.acc_slot);
-      if (a.geom == 2) {
-        // nmma == 1.  Per K chunk: wait for the haloed copy; per tap: wait for its weight stage, issue the K steps of both
-        // 16x8 halves (left half: pixels 0..7 of each row, right half: 8..15 = the same copy 8 pixels further on),
-        // release the weight stage; after the ninth tap release the copy.
+      if (a.geom == 3) {
+        // nmma == 1.  Per K chunk: wait for the haloed copy; per tap: wait for its weight stage, issue its K steps as
+        // D[cout, pixel] += W_tap[cout, k] * X[pixel shifted by the tap, k] (A = the weight stage, SBO = 1024; B = the copy
+        // at byte offset dy*1280 + dx*128, SBO = 1280), release the weight stage; after the ninth tap release the copy.
+        // Chunk -> dx -> dy -> K step is the issue order of the g0x2 geometry this one replaced.
         const uint32_t wring_u32 = stages_u32 + (uint32_t)(a.na_slots * a.a_slot);
         for (int ch = 0; ch < a.nchunks; ++ch) {
-          mbar_wait(&afull[g2_as], g2_aph);
+          mbar_wait(&afull[g3_as], g3_aph);
           tc_fence_after();
-          const uint32_t a_addr = stages_u32 + (uint32_t)(g2_as * a.a_slot);
+          const uint32_t x_addr = stages_u32 + (uint32_t)(g3_as * a.a_slot);
           const int ksteps = (ch == a.nchunks - 1) ? a.ksteps_last : 4;
           for (int dxi = 0; dxi < 3; ++dxi)
             for (int dyi = 0; dyi < 3; ++dyi) {
               mbar_wait(&full[s], ph);
               tc_fence_after();
-              const uint32_t bl = desc_lo(wring_u32 + (uint32_t)(s * a.stage_bytes));
+              const uint32_t wl = desc_lo(wring_u32 + (uint32_t)(s * a.stage_bytes));
+              const uint32_t xl = desc_lo(x_addr + (uint32_t)dyi * (a.a_step16 << 4) + 128u * (uint32_t)dxi);
               const uint32_t acc0 = (ch > 0 || dxi > 0 || dyi > 0) ? 1u : 0u;
-              for (int half = 0; half < 2; ++half) {
-                const uint32_t al = desc_lo(a_addr + (uint32_t)dyi * (a.a_step16 << 4) + 128u * (uint32_t)(dxi + 8 * half));
-                const uint32_t td = tmem_d + (uint32_t)(half * a.acc_half);
-                switch (ksteps) {
-                  case 4: umma_tap1c_k4(td, al, bl, idesc, acc0, a.a_desc_hi, TC_DESC_HI); break;
-                  case 3: umma_tap1c_k3(td, al, bl, idesc, acc0, a.a_desc_hi, TC_DESC_HI); break;
-                  case 2: umma_tap1c_k2(td, al, bl, idesc, acc0, a.a_desc_hi, TC_DESC_HI); break;
-                  default: umma_tap1c_k1(td, al, bl, idesc, acc0, a.a_desc_hi, TC_DESC_HI); break;
-                }
+              switch (ksteps) {
+                case 4: umma_tap1c_k4(tmem_d, wl, xl, idesc, acc0, TC_DESC_HI, a.a_desc_hi); break;
+                case 3: umma_tap1c_k3(tmem_d, wl, xl, idesc, acc0, TC_DESC_HI, a.a_desc_hi); break;
+                case 2: umma_tap1c_k2(tmem_d, wl, xl, idesc, acc0, TC_DESC_HI, a.a_desc_hi); break;
+                default: umma_tap1c_k1(tmem_d, wl, xl, idesc, acc0, TC_DESC_HI, a.a_desc_hi); break;
               }
               umma_commit(&empty[s]);
               if (++s == a.nstages) { s = 0; ph ^= 1; }
             }
-          umma_commit(&aempty[g2_as]);
-          if (++g2_as == a.na_slots) { g2_as = 0; g2_aph ^= 1; }
+          umma_commit(&aempty[g3_as]);
+          if (++g3_as == a.na_slots) { g3_as = 0; g3_aph ^= 1; }
         }
         umma_commit(&tfull[as]);
         as += nmma;
@@ -973,7 +1087,18 @@ k_conv_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
                      : (a.epi == FFSR_EPI_RESIDUAL ? EM_RESIDUAL : (a.epi == FFSR_EPI_ACTGRAD ? EM_ACTGRAD : a.act));
     // one specialised loop per (epilogue mode, output type): no per-element switches, and the
     // plain modes do not carry the residual registers
-    if (a.lean) {
+    if (a.geom == 3) {
+      switch (mode) {
+        case EM_GELU:
+          if (a.gelu_tanh) swapped_epilogue<EM_GELU, true>(a, tfull, tempty, tmem_base, warp, lane);
+          else swapped_epilogue<EM_GELU, false>(a, tfull, tempty, tmem_base, warp, lane);
+          break;
+        case EM_RELU: swapped_epilogue<EM_RELU, false>(a, tfull, tempty, tmem_base, warp, lane); break;
+        case EM_SIGMOID: swapped_epilogue<EM_SIGMOID, false>(a, tfull, tempty, tmem_base, warp, lane); break;
+        case EM_RESIDUAL: swapped_epilogue<EM_RESIDUAL, false>(a, tfull, tempty, tmem_base, warp, lane); break;
+        default: swapped_epilogue<EM_NONE, false>(a, tfull, tempty, tmem_base, warp, lane); break;
+      }
+    } else if (a.lean) {
       switch (mode) {
         case EM_GELU:
           if (a.gelu_tanh) lean_epilogue<EM_GELU, true>(a, tfull, tempty, tmem_base, warp, lane, sbias);
@@ -1084,19 +1209,21 @@ int ffsr_conv2d_tc(const ffsr_conv_params* pp, cudaStream_t stream) {
     if (p.ksize == 3 && halves == 1 && nch0 * p.ksize * bb + 3 * A1C_STAGE <= avail0 && p.H >= 8 && getenv("FFSR_TC_GEOM0") == nullptr)
       geom = 1;
   }
-  // Streamed-weight 3x3 layers served by the lean epilogue (bf16 inference outputs): dual-ring geometry, see the kernel
-  constexpr int A2_BYTES = 18 * 18 * 128, A2_SLOT = (A2_BYTES + 1023) / 1024 * 1024;
-  if (halves == 2 && geom == 0 && p.ksize == 3 && getenv("FFSR_TC_GEOM2_OFF") == nullptr && getenv("FFSR_TC_LEAN0") == nullptr) {
+  // Streamed-weight 3x3 layers with bf16 inference outputs: swapped operands (weights = M, 8x32-px tiles = N = 256), see the
+  // kernel.  Cout <= 64 (nblk 64) stays on g0x2: an M = 128 MMA would spend half its work on zero weight rows.  Images of
+  // fewer than 32 rows stay there too: most of a 256-pixel tile would be padding.
+  constexpr int A3_BYTES = 34 * 10 * 128, A3_SLOT = (A3_BYTES + 1023) / 1024 * 1024;
+  if (halves == 2 && geom == 0 && p.ksize == 3 && getenv("FFSR_TC_LEAN0") == nullptr) {
     const bool mode_ok = p.epi == FFSR_EPI_PLAIN || (p.epi == FFSR_EPI_RESIDUAL && p.act == ACT_NONE);
     const bool out_ok = p.out_dtype == FFSR_DT_BF16 && p.out2 == nullptr && p.groups == 1 && p.Cout % 8 == 0 && ((uintptr_t)p.out % 16) == 0 &&
-                        p.out_sX % 8 == 0 && p.out_sY % 8 == 0 && p.out_sN % 8 == 0 && cout_pad <= TC_BIAS_MAX && (nblk % 64) == 0;
+                        p.out_sX % 8 == 0 && p.out_sY % 8 == 0 && p.out_sN % 8 == 0 && nblk == 128;
     bool res_ok = true;
     if (p.epi == FFSR_EPI_RESIDUAL) {
       const int r1q = p.r1_dtype == FFSR_DT_BF16 ? 8 : 4, r2q = p.r2_dtype == FFSR_DT_BF16 ? 8 : 4;
       res_ok = p.r1 != nullptr && ((uintptr_t)p.r1 % 16) == 0 && p.r1_sX % r1q == 0 && p.r1_sY % r1q == 0 && p.r1_sN % r1q == 0 &&
                (p.r2 == nullptr || (((uintptr_t)p.r2 % 16) == 0 && p.r2_sX % r2q == 0 && p.r2_sY % r2q == 0 && p.r2_sN % r2q == 0));
     }
-    if (mode_ok && out_ok && res_ok && p.W >= 18 && p.H >= 18) geom = 2;
+    if (mode_ok && out_ok && res_ok && p.H >= 32) geom = 3;
   }
   CUtensorMap tmA, tmB;
   {
@@ -1104,7 +1231,7 @@ int ffsr_conv2d_tc(const ffsr_conv_params* pp, cudaStream_t stream) {
     cuuint64_t strides[3] = {(cuuint64_t)p.in_sX * 2, (cuuint64_t)p.in_sY * 2, (cuuint64_t)p.in_sN * 2};
     cuuint32_t box[4] = {64, TC_TW, (cuuint32_t)(TC_TH * halves + 2 * (p.ksize / 2)), 1};
     if (geom == 1) { box[1] = 10; box[2] = 18; }
-    if (geom == 2) { box[1] = 18; box[2] = 18; }
+    if (geom == 3) { box[1] = 10; box[2] = 34; }
     cuuint32_t es[4] = {1, 1, 1, 1};
     CUresult r = enc(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p.in), dims, strides, box, es,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -1116,7 +1243,7 @@ int ffsr_conv2d_tc(const ffsr_conv_params* pp, cudaStream_t stream) {
     const cuuint64_t tap_bytes = (cuuint64_t)cin_pad * cout_pad * 2;
     cuuint64_t dims[5] = {(cuuint64_t)cin_pad, (cuuint64_t)cout_pad, (cuuint64_t)p.ksize, (cuuint64_t)p.ksize, (cuuint64_t)p.groups};
     cuuint64_t strides[4] = {(cuuint64_t)cin_pad * 2, tap_bytes, tap_bytes * p.ksize, tap_bytes * taps};
-    cuuint32_t box[5] = {64, (cuuint32_t)nblk, 1, (cuuint32_t)(geom == 2 ? 1 : p.ksize), 1};
+    cuuint32_t box[5] = {64, (cuuint32_t)nblk, 1, (cuuint32_t)(geom == 3 ? 1 : p.ksize), 1};
     cuuint32_t es[5] = {1, 1, 1, 1, 1};
     CUresult r = enc(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<float*>(p.w), dims, strides, box, es,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -1153,36 +1280,27 @@ int ffsr_conv2d_tc(const ffsr_conv_params* pp, cudaStream_t stream) {
   int smem_bytes = 1024 + TC_SMEM_HDR + a.bres_bytes + a.nstages * a.stage_bytes;
   a.a_slot = 0;
   a.na_slots = 0;
-  if (geom == 2) {
-    a.tile_h = 16;
-    a.a_step16 = (18u * 128u) >> 4;
-    a.a_desc_hi = ((18u * 128u) >> 4) | (1u << 14) | (2u << 29);
-    a.a_bytes = A2_BYTES;
-    a.a_slot = A2_SLOT;
-    a.na_slots = 2;
+  if (geom == 3) {
+    a.tile_h = 32;
+    a.a_bytes = A3_BYTES;
+    a.a_slot = A3_SLOT;
+    a.na_slots = TC_MAX_ASLOTS;
     a.b_bytes = nblk * 128;                                    // one tap of one K chunk
     a.b_resident = 0;
     a.bres_bytes = 0;
     a.stage_bytes = a.b_bytes;
     a.nstages = (smem_avail - a.na_slots * a.a_slot) / a.stage_bytes;
     if (a.nstages > TC_MAX_STAGES) a.nstages = TC_MAX_STAGES;
-    if (const char* e = getenv("FFSR_TC_G2_ASLOTS")) {         // experiment: deeper activation ring, shallower weight ring
-      const int v = atoi(e);
-      if (v >= 1 && v <= TC_MAX_ASLOTS && (smem_avail - v * a.a_slot) / a.stage_bytes >= 2) {
-        a.na_slots = v;
-        a.nstages = (smem_avail - v * a.a_slot) / a.stage_bytes;
-        if (a.nstages > TC_MAX_STAGES) a.nstages = TC_MAX_STAGES;
-      }
-    }
     smem_bytes = 1024 + TC_SMEM_HDR + a.na_slots * a.a_slot + a.nstages * a.stage_bytes;
   }
   a.acc_half = nblk <= 32 ? 32 : (nblk <= 64 ? 64 : 128);
-  a.acc_slot = a.acc_half * halves;
+  if (geom == 3) { a.halves = 1; a.acc_half = 256; }         // one accumulator: 128 lanes (couts) x 256 columns (pixels)
+  a.acc_slot = a.acc_half * a.halves;
   a.nacc = TC_TMEM_COLS / a.acc_slot;
   if (a.nacc > TC_MAX_ACC) a.nacc = TC_MAX_ACC;
   a.groups = p.groups;
   a.epi_own = 0;
-  a.tiles_x = ceil_div(p.W, geom == 1 ? 8 : TC_TW);
+  a.tiles_x = ceil_div(p.W, geom == 1 || geom == 3 ? 8 : TC_TW);
   a.tiles_y = ceil_div(p.H, a.tile_h);
   a.total_tiles = (long long)a.tiles_x * a.tiles_y * p.N * a.n_nblocks;
   a.out = p.out; a.out_sN = p.out_sN; a.out_sY = p.out_sY; a.out_sX = p.out_sX;
@@ -1225,7 +1343,7 @@ int ffsr_conv2d_tc(const ffsr_conv_params* pp, cudaStream_t stream) {
     if (a.lean) a.epi_own = (!own_off && own_lean) ? 1 : 0;
     if (a.lean && !a.epi_own && !split_lean) a.lean = 0;
   }
-  FFSR_REQUIRE(geom != 2 || a.lean, FFSR_ERR_ARG, "conv2d(tc): internal: dual-ring geometry without the lean epilogue");
+  if (geom == 3) { a.lean = 0; a.epi_own = 0; }               // geom 3 has its own epilogue (swapped_epilogue)
   // several MMA-issuing warps for launches whose tiles are a few small MMAs (issue-bound, see the kernel): needs one weight
   // set for the whole launch and an accumulator ring that is a multiple of the warp count (3 warps: ring of 6)
   {
