@@ -78,7 +78,7 @@ PROTOTYPES = {
     "ffsr_fft_twiddles": (_I, [_I, _P, _P]),
     "ffsr_fft_workspace_bytes": (_SZ, [_I, _I, _I]),
     "ffsr_fft_bands": (_I, [_P, _I, _I, _I, _P, _I, _P, _P, _P, _P, _P, _SZ, _P, _P]),
-    "ffsr_crossband_attention": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _I, _P, _I, _P, _P]),
+    "ffsr_crossband_attention": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, _I, _P, _I, _P, _P]),
     "ffsr_crossband_out": (_I, [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "ffsr_lka_depthwise": (_I, [_P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _I, _P]),
     "ffsr_lka_tail_weight_bytes": (_SZ, []),

@@ -1185,7 +1185,7 @@ int ffsr_conv2d_tc(const ffsr_conv_params* pp, cudaStream_t stream) {
   // weights the whole activation tensor was re-read from HBM once per block (6 x 88 MB for a 244 -> 768 Linear: the launch sat on
   // the HBM roof of that schedule, 150 us for 12 GFLOP).  Here the cout block varies fastest, the weights stream beside the
   // activations and 16x16-pixel tiles share every weight stage between two M = 128 MMAs.
-  const bool gemm_mode = p.ksize == 1 && cout_pad / nblk > 1 && p.groups == 1 && getenv("FFSR_TC_GEMM_MODE_OFF") == nullptr;
+  const bool gemm_mode = p.ksize == 1 && cout_pad / nblk > 1 && p.groups == 1;
   int halves = 1;
   if (gemm_mode && p.H >= 16 && nblk * 2 * 2 <= TC_TMEM_COLS) halves = 2;
   {
@@ -1206,25 +1206,24 @@ int ffsr_conv2d_tc(const ffsr_conv_params* pp, cudaStream_t stream) {
     const int nch0 = (p.Cin + 63) / 64;
     const int bb = p.ksize * nblk * 128;
     const int avail0 = TC_SMEM_MAX - 1024 - TC_SMEM_HDR;
-    if (p.ksize == 3 && halves == 1 && nch0 * p.ksize * bb + 3 * A1C_STAGE <= avail0 && p.H >= 8 && getenv("FFSR_TC_GEOM0") == nullptr)
+    if (p.ksize == 3 && halves == 1 && nch0 * p.ksize * bb + 3 * A1C_STAGE <= avail0 && p.H >= 8)
       geom = 1;
   }
   // Streamed-weight 3x3 layers with bf16 inference outputs: swapped operands (weights = M, 8x32-px tiles = N = 256), see the
   // kernel.  Cout <= 64 (nblk 64) stays on g0x2: an M = 128 MMA would spend half its work on zero weight rows.  Images of
   // fewer than 32 rows stay there too: most of a 256-pixel tile would be padding.
   constexpr int A3_BYTES = 34 * 10 * 128, A3_SLOT = (A3_BYTES + 1023) / 1024 * 1024;
-  if (halves == 2 && geom == 0 && p.ksize == 3 && getenv("FFSR_TC_LEAN0") == nullptr) {
-    const bool mode_ok = p.epi == FFSR_EPI_PLAIN || (p.epi == FFSR_EPI_RESIDUAL && p.act == ACT_NONE);
-    const bool out_ok = p.out_dtype == FFSR_DT_BF16 && p.out2 == nullptr && p.groups == 1 && p.Cout % 8 == 0 && ((uintptr_t)p.out % 16) == 0 &&
-                        p.out_sX % 8 == 0 && p.out_sY % 8 == 0 && p.out_sN % 8 == 0 && nblk == 128;
-    bool res_ok = true;
-    if (p.epi == FFSR_EPI_RESIDUAL) {
-      const int r1q = p.r1_dtype == FFSR_DT_BF16 ? 8 : 4, r2q = p.r2_dtype == FFSR_DT_BF16 ? 8 : 4;
-      res_ok = p.r1 != nullptr && ((uintptr_t)p.r1 % 16) == 0 && p.r1_sX % r1q == 0 && p.r1_sY % r1q == 0 && p.r1_sN % r1q == 0 &&
-               (p.r2 == nullptr || (((uintptr_t)p.r2 % 16) == 0 && p.r2_sX % r2q == 0 && p.r2_sY % r2q == 0 && p.r2_sN % r2q == 0));
-    }
-    if (mode_ok && out_ok && res_ok && p.H >= 32) geom = 3;
+  // Outputs that both 16-byte-group epilogues (the lean one and geom 3's) can store: bf16, plain or residual without an
+  // activation, aligned rows, residual inputs aligned to their own 16-byte groups.
+  bool lean_ok = (p.epi == FFSR_EPI_PLAIN || (p.epi == FFSR_EPI_RESIDUAL && p.act == ACT_NONE)) && p.out_dtype == FFSR_DT_BF16 &&
+                 p.out2 == nullptr && p.groups == 1 && p.Cout % 8 == 0 && ((uintptr_t)p.out % 16) == 0 && p.out_sX % 8 == 0 &&
+                 p.out_sY % 8 == 0 && p.out_sN % 8 == 0;
+  if (lean_ok && p.epi == FFSR_EPI_RESIDUAL) {
+    const int r1q = p.r1_dtype == FFSR_DT_BF16 ? 8 : 4, r2q = p.r2_dtype == FFSR_DT_BF16 ? 8 : 4;
+    lean_ok = p.r1 != nullptr && ((uintptr_t)p.r1 % 16) == 0 && p.r1_sX % r1q == 0 && p.r1_sY % r1q == 0 && p.r1_sN % r1q == 0 &&
+              (p.r2 == nullptr || (((uintptr_t)p.r2 % 16) == 0 && p.r2_sX % r2q == 0 && p.r2_sY % r2q == 0 && p.r2_sN % r2q == 0));
   }
+  if (halves == 2 && geom == 0 && p.ksize == 3 && lean_ok && nblk == 128 && p.H >= 32) geom = 3;
   CUtensorMap tmA, tmB;
   {
     cuuint64_t dims[4] = {(cuuint64_t)p.Cin, (cuuint64_t)p.W, (cuuint64_t)p.H, (cuuint64_t)p.N};
@@ -1320,35 +1319,22 @@ int ffsr_conv2d_tc(const ffsr_conv_params* pp, cudaStream_t stream) {
   }
   const int grid = (int)(a.total_tiles < num_sms ? a.total_tiles : num_sms);
   // tile-per-group epilogue: needs >= 8 accumulators in flight (N <= 64, single-half tiles) and enough tiles per CTA
-  static const bool own_off = getenv("FFSR_TC_EPI_OWN0") != nullptr;
   static const bool erf_forced = getenv("FFSR_TC_GELU_ERF") != nullptr;
   a.gelu_tanh = (!erf_forced && p.out2 == nullptr) ? 1 : 0;
   const bool own_force = getenv("FFSR_TC_EPI_OWN_FORCE") != nullptr;     // tests: small images take the own path too (read per call)
-  const bool lean_off = getenv("FFSR_TC_LEAN0") != nullptr;
-  a.epi_own = (!own_off && halves == 1 && a.nacc >= 8 && (own_force || a.total_tiles >= 8LL * grid)) ? 1 : 0;
+  a.epi_own = (halves == 1 && a.nacc >= 8 && (own_force || a.total_tiles >= 8LL * grid)) ? 1 : 0;
   {
     // lean epilogue: bf16 inference outputs in 16-byte groups; own mode also for 128-column single-half tiles (4 accumulators)
-    const bool mode_ok = p.epi == FFSR_EPI_PLAIN || (p.epi == FFSR_EPI_RESIDUAL && p.act == ACT_NONE);
-    const bool out_ok = a.out_bf16 && p.out2 == nullptr && p.groups == 1 && p.Cout % 8 == 0 && ((uintptr_t)p.out % 16) == 0 &&
-                        p.out_sX % 8 == 0 && p.out_sY % 8 == 0 && p.out_sN % 8 == 0 && a.n_nblocks * a.nblk <= TC_BIAS_MAX;
-    bool res_ok = true;
-    if (p.epi == FFSR_EPI_RESIDUAL) {
-      const int r1q = p.r1_dtype == FFSR_DT_BF16 ? 8 : 4, r2q = p.r2_dtype == FFSR_DT_BF16 ? 8 : 4;
-      res_ok = p.r1 != nullptr && ((uintptr_t)p.r1 % 16) == 0 && p.r1_sX % r1q == 0 && p.r1_sY % r1q == 0 && p.r1_sN % r1q == 0 &&
-               (p.r2 == nullptr || (((uintptr_t)p.r2 % 16) == 0 && p.r2_sX % r2q == 0 && p.r2_sY % r2q == 0 && p.r2_sN % r2q == 0));
-    }
     const bool own_lean = halves == 1 && a.nacc >= 4 && (own_force || a.total_tiles >= 8LL * grid);
     const bool split_lean = (a.nblk % 64) == 0;
-    a.lean = (!lean_off && mode_ok && out_ok && res_ok && (own_lean || split_lean)) ? 1 : 0;
-    if (a.lean) a.epi_own = (!own_off && own_lean) ? 1 : 0;
+    a.lean = (lean_ok && a.n_nblocks * a.nblk <= TC_BIAS_MAX && (own_lean || split_lean)) ? 1 : 0;
+    if (a.lean) a.epi_own = own_lean ? 1 : 0;
     if (a.lean && !a.epi_own && !split_lean) a.lean = 0;
   }
   if (geom == 3) { a.lean = 0; a.epi_own = 0; }               // geom 3 has its own epilogue (swapped_epilogue)
   // several MMA-issuing warps for launches whose tiles are a few small MMAs (issue-bound, see the kernel): needs one weight
   // set for the whole launch and an accumulator ring that is a multiple of the warp count (3 warps: ring of 6)
   {
-    int want = TC_MMA_WARPS;
-    if (const char* e = getenv("FFSR_TC_NMMA")) want = atoi(e);
     a.nmma = 1;
     // Every barrier wait is by PARITY, which tells a phase only from its neighbours: whoever waits for use k of a pipeline
     // stage must KNOW that use k - nstages has completed.  With one issuer that is its own previous wait.  With several, a
@@ -1358,9 +1344,8 @@ int ffsr_conv2d_tc(const ffsr_conv_params* pp, cudaStream_t stream) {
     // So the ring is trimmed to a multiple of nmma * (stages per tile): tile q and tile q + ring / kiters then use the same
     // stages AND belong to the same warp, and every wait follows that warp's own wait for the previous phase.
     const int kiters = geom ? a.nchunks : p.ksize * a.nchunks;
-    if (const char* e = getenv("FFSR_TC_NSTAGES")) { const int v = atoi(e); if (v >= 1 && v <= a.nstages) a.nstages = v; }   // debug
-    if (want > 1 && (p.flags & FFSR_CONV_MULTI_ISSUE) && a.b_resident && p.groups == 1 && a.n_nblocks == 1 && halves == 1) {
-      int n = want >= 3 ? 3 : 2;
+    if ((p.flags & FFSR_CONV_MULTI_ISSUE) && a.b_resident && p.groups == 1 && a.n_nblocks == 1 && halves == 1) {
+      int n = TC_MMA_WARPS >= 3 ? 3 : TC_MMA_WARPS;
       while (n > 1 && n * kiters > a.nstages) --n;
       // The accumulator ring must likewise be a multiple of the issuing warps (a slot always belongs to the same warp) AND,
       // with tile ownership in the epilogue, of the four epilogue warp groups (a group waits for its tile's accumulator by

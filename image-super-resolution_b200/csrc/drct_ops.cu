@@ -4,7 +4,6 @@
 //
 // STATUS: exercised on a B200 through `isr_b200.drct.DRCT.forward` (parity <= 1e-4 against the reference class's output,
 // tests/test_gpu_drct.py); simple grid-stride kernels, not yet timed against the HBM roof.
-#include <stdlib.h>
 #include "common.cuh"
 #include "../../include/ffsr_b200.h"
 
@@ -160,7 +159,7 @@ extern "C" int ffsr_layernorm_strided(const void* x, long rows, int C, long x_pi
   if (ib && ob) k_layernorm_strided<__nv_bfloat16, __nv_bfloat16><<<grid, 256, 0, stream>>>((const __nv_bfloat16*)x, rows, C, x_pitch, w, b, (__nv_bfloat16*)y, y_pitch);
   else if (ib) k_layernorm_strided<__nv_bfloat16, float><<<grid, 256, 0, stream>>>((const __nv_bfloat16*)x, rows, C, x_pitch, w, b, (float*)y, y_pitch);
   else if (ob && (C & 3) == 0 && (x_pitch & 3) == 0 && (y_pitch & 3) == 0 && ((uintptr_t)x & 15) == 0 && ((uintptr_t)y & 7) == 0 &&
-           ((uintptr_t)w & 15) == 0 && ((uintptr_t)b & 15) == 0 && getenv("FFSR_LN_SCALAR") == nullptr)
+           ((uintptr_t)w & 15) == 0 && ((uintptr_t)b & 15) == 0)
     k_layernorm_strided_v4<<<grid, 256, 0, stream>>>((const float*)x, rows, C, x_pitch, w, b, (__nv_bfloat16*)y, y_pitch);
   else if (ob) k_layernorm_strided<float, __nv_bfloat16><<<grid, 256, 0, stream>>>((const float*)x, rows, C, x_pitch, w, b, (__nv_bfloat16*)y, y_pitch);
   else k_layernorm_strided<float, float><<<grid, 256, 0, stream>>>((const float*)x, rows, C, x_pitch, w, b, (float*)y, y_pitch);

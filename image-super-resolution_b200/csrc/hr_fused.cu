@@ -2,7 +2,6 @@
 // per pixel x 4-channel group, coalesced planar reads, channels-last vector writes).
 // Each kernel cites the reference op sequence it replaces in include/ffsr_b200.h.
 #include <type_traits>
-#include <stdlib.h>
 #include "common.cuh"
 #include "../../include/ffsr_b200.h"
 
@@ -479,9 +478,8 @@ extern "C" int ffsr_resize_nhwc(const void* src, int N, int h, int w, int C, lon
   const int esz = dtype == FFSR_DT_BF16 ? 2 : 4;
   FFSR_REQUIRE(((uintptr_t)src % (4 * esz)) == 0 && ((uintptr_t)dst % (4 * esz)) == 0 && src_sX % 4 == 0 && dst_sX % 4 == 0,
                FFSR_ERR_ALIGN, "resize_nhwc: vector alignment");
-  static const bool up_v1 = getenv("FFSR_UPSAMPLE_V1") != nullptr;
   if (dtype == FFSR_DT_BF16 && C % 8 == 0 && ((uintptr_t)src % 16) == 0 && ((uintptr_t)dst % 16) == 0 && src_sX % 8 == 0 &&
-      dst_sX % 8 == 0 && h <= 65535 && N <= 65535 && !up_v1 && ((H == 2 * h && W == 2 * w) || (H == 4 * h && W == 4 * w))) {
+      dst_sX % 8 == 0 && h <= 65535 && N <= 65535 && ((H == 2 * h && W == 2 * w) || (H == 4 * h && W == 4 * w))) {
     dim3 grid(ceil_div((long)w * (C / 8), 256), h, N);
     if (H == 2 * h)
       k_upsample_int<2, false><<<grid, 256, 0, stream>>>((const __nv_bfloat16*)src, nullptr, h, w, C / 8, src_sX, nullptr, 0, (__nv_bfloat16*)dst, dst_sX);
@@ -505,12 +503,12 @@ extern "C" int ffsr_resize_nhwc(const void* src, int N, int h, int w, int C, lon
 }
 
 // ------------------------------------------------------------------------------------------
-// SpatialGate: y = x * sigmoid(w2 . gelu(W1 x + b1) + b2), one thread per pixel
+// SpatialGate: y = x * sigmoid(w2 . gelu(W1 x + b1) + b2), fp32 rows, one thread per pixel
 // ------------------------------------------------------------------------------------------
-template <typename T, int C>
-__global__ void __launch_bounds__(128) k_spatial_gate(const T* __restrict__ x, long pixels, const float* __restrict__ w1,
+template <int C>
+__global__ void __launch_bounds__(128) k_spatial_gate(const float* __restrict__ x, long pixels, const float* __restrict__ w1,
                                                       const float* __restrict__ b1, const float* __restrict__ w2,
-                                                      const float* __restrict__ b2, T* __restrict__ y) {
+                                                      const float* __restrict__ b2, float* __restrict__ y) {
   constexpr int HID = C / 4;
   __shared__ __align__(16) float sw1[HID][C];
   __shared__ float sb1[HID], sw2[HID];
@@ -522,7 +520,7 @@ __global__ void __launch_bounds__(128) k_spatial_gate(const T* __restrict__ x, l
   float v[C];
 #pragma unroll
   for (int c = 0; c < C; c += 4) {
-    const float4 t = load_vec4<T>(x + p * C + c);
+    const float4 t = load_vec4<float>(x + p * C + c);
     v[c] = t.x; v[c + 1] = t.y; v[c + 2] = t.z; v[c + 3] = t.w;
   }
   float z = b2[0];
@@ -534,15 +532,15 @@ __global__ void __launch_bounds__(128) k_spatial_gate(const T* __restrict__ x, l
       const float4 w4 = *reinterpret_cast<const float4*>(&sw1[h][c]);
       a = fmaf(w4.x, v[c], a); a = fmaf(w4.y, v[c + 1], a); a = fmaf(w4.z, v[c + 2], a); a = fmaf(w4.w, v[c + 3], a);
     }
-    z = fmaf(sw2[h], gelu_sel<!std::is_same<T, float>::value>(a), z);
+    z = fmaf(sw2[h], gelu_sel<false>(a), z);
   }
   const float g = sigmoid_acc(z);
 #pragma unroll
-  for (int c = 0; c < C; c += 4) store_vec4<T>(y + p * C + c, v[c] * g, v[c + 1] * g, v[c + 2] * g, v[c + 3] * g);
+  for (int c = 0; c < C; c += 4) store_vec4<float>(y + p * C + c, v[c] * g, v[c + 1] * g, v[c + 2] * g, v[c + 3] * g);
 }
 
 // bf16 rows, TPP = C / CH lanes per pixel with CH channels each, the lane's slice of W1 (HID x CH = 64 floats) in REGISTERS
-// for the whole grid-stride loop.  ncu of the one-thread-per-pixel kernel above: 65 % of the issue cycles without an eligible warp,
+// for the whole grid-stride loop.  ncu of a one-thread-per-pixel bf16 kernel: 65 % of the issue cycles without an eligible warp,
 // short-scoreboard stalls on the 64 shared-memory weight loads per pixel (weights of all C channels cannot live in one thread's
 // registers).  The HID partial sums are combined by a transposing butterfly: at each of the log2(TPP) steps a lane hands half of
 // its values to its partner, so it ends with HID / TPP complete hidden units (HID - HID / TPP shuffles in total instead of
@@ -637,9 +635,7 @@ extern "C" int ffsr_spatial_gate(const void* x, long pixels, int C, const float*
   FFSR_REQUIRE(x && y && w1 && b1 && w2 && b2, FFSR_ERR_ARG, "spatial_gate: null pointer");
   FFSR_REQUIRE(C == 64 || C == 32, FFSR_ERR_ARG, "spatial_gate: C must be 32 or 64");
   FFSR_REQUIRE(((uintptr_t)x % 16) == 0 && ((uintptr_t)y % 16) == 0, FFSR_ERR_ALIGN, "spatial_gate: 16B alignment");
-  const int grid = ceil_div(pixels, 128);
-  static const bool v1 = getenv("FFSR_SPATIAL_GATE_V1") != nullptr;
-  if (dtype == FFSR_DT_BF16 && !v1) {
+  if (dtype == FFSR_DT_BF16) {
     static int num_sms = 0;
     if (!num_sms) {
       int dev = 0;
@@ -653,13 +649,9 @@ extern "C" int ffsr_spatial_gate(const void* x, long pixels, int C, const float*
     else k_spatial_gate_rows<32, 8><<<g2, 256, 0, stream>>>((const __nv_bfloat16*)x, pixels, w1, b1, w2, b2, (__nv_bfloat16*)y);
     return ffsr_check_launch("spatial_gate");
   }
-  if (dtype == FFSR_DT_BF16) {
-    if (C == 64) k_spatial_gate<__nv_bfloat16, 64><<<grid, 128, 0, stream>>>((const __nv_bfloat16*)x, pixels, w1, b1, w2, b2, (__nv_bfloat16*)y);
-    else k_spatial_gate<__nv_bfloat16, 32><<<grid, 128, 0, stream>>>((const __nv_bfloat16*)x, pixels, w1, b1, w2, b2, (__nv_bfloat16*)y);
-  } else {
-    if (C == 64) k_spatial_gate<float, 64><<<grid, 128, 0, stream>>>((const float*)x, pixels, w1, b1, w2, b2, (float*)y);
-    else k_spatial_gate<float, 32><<<grid, 128, 0, stream>>>((const float*)x, pixels, w1, b1, w2, b2, (float*)y);
-  }
+  const int grid = ceil_div(pixels, 128);
+  if (C == 64) k_spatial_gate<64><<<grid, 128, 0, stream>>>((const float*)x, pixels, w1, b1, w2, b2, (float*)y);
+  else k_spatial_gate<32><<<grid, 128, 0, stream>>>((const float*)x, pixels, w1, b1, w2, b2, (float*)y);
   return ffsr_check_launch("spatial_gate");
 }
 
@@ -1028,8 +1020,7 @@ extern "C" int ffsr_edge_attn_upsample(const void* o, int o_dtype, const float* 
                "edge_attn_upsample: alignment");
   const long total = (long)N * H * W * (C / 4);
   FFSR_REQUIRE(o_dtype == FFSR_DT_F32 || dtype == FFSR_DT_BF16, FFSR_ERR_ARG, "edge_attn_upsample: bf16 input needs bf16 output");
-  static const bool up_v1 = getenv("FFSR_UPSAMPLE_V1") != nullptr;
-  if (o_dtype == FFSR_DT_BF16 && C % 8 == 0 && ((uintptr_t)dst % 16) == 0 && dst_sX % 8 == 0 && h <= 65535 && N <= 65535 && !up_v1 &&
+  if (o_dtype == FFSR_DT_BF16 && C % 8 == 0 && ((uintptr_t)dst % 16) == 0 && dst_sX % 8 == 0 && h <= 65535 && N <= 65535 &&
       ((H == 2 * h && W == 2 * w) || (H == 4 * h && W == 4 * w))) {
     dim3 grid(ceil_div((long)w * (C / 8), 256), h, N);
     if (H == 2 * h)

@@ -7,12 +7,10 @@
 // (three separately padded convs != one 25x25 conv at the borders; SURVEY §7 hard part 5).
 // HBM/L1-bound: each thread owns one channel and a short run of outputs along the conv
 // axis, keeps the sliding window in registers, and warps read 32 consecutive channels.
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace {
 constexpr int R5 = 4;    // 4x4 output patch per thread for the 5x5 (8x8 input window in registers)
-constexpr int R21 = 16;  // outputs per thread along the conv axis for the 21-tap passes
 }
 
 // BN is folded to y = x*k + d (eval: running stats; train: batch stats computed upstream).
@@ -93,80 +91,11 @@ __global__ void __launch_bounds__(256) k_lka_dw5(const TI* __restrict__ x, int H
       if (y0 + a < H && x0 + b < W) out[(((long)n * H + y0 + a) * W + x0 + b) * C + c] = acc[a][b];
 }
 
-// AXIS = 0: taps along W (1x21); AXIS = 1: taps along H (21x1)
-template <int AXIS, typename TO, int CT = 0>
-__global__ void __launch_bounds__(256) k_lka_dw21(const float* __restrict__ in, int H, int W, int C_rt,
-                                                  const float* __restrict__ w21, TO* __restrict__ out) {
-  const int C = CT > 0 ? CT : C_rt;
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  const int n = blockIdx.z;
-  int y, x;
-  if (AXIS == 0) {
-    const int runs = (W + R21 - 1) / R21;
-    const int idx = blockIdx.y * blockDim.y + threadIdx.y;    // over H * runs
-    y = idx / runs;
-    x = (idx % runs) * R21;
-    if (y >= H) return;
-  } else {
-    const int runs = (H + R21 - 1) / R21;
-    const int idx = blockIdx.y * blockDim.y + threadIdx.y;    // over runs * W
-    y = (idx / W) * R21;
-    x = idx % W;
-    if (idx >= runs * W) return;
-  }
-  if (c >= C) return;
-  float w[21];
-#pragma unroll
-  for (int i = 0; i < 21; ++i) w[i] = w21[c * 21 + i];
-  const float* img = in + (long)n * H * W * C;
-  TO* oimg = out + (long)n * H * W * C;
-  float v[R21 + 20];
-  // The kernel is instruction-issue bound (ncu: 74 % issue slots busy at 25 % of HBM), so runs that do not touch
-  // the border take a path without per-load bounds tests and with 32-bit strided offsets.
-  const int stride = (AXIS == 0) ? C : W * C;
-  const bool interior = (AXIS == 0) ? (x >= 10 && x + R21 + 10 <= W) : (y >= 10 && y + R21 + 10 <= H);
-  if (interior) {
-    const float* p = img + ((AXIS == 0) ? ((long)y * W + (x - 10)) : ((long)(y - 10) * W + x)) * C + c;
-#pragma unroll
-    for (int i = 0; i < R21 + 20; ++i) v[i] = p[i * stride];
-    TO* o = oimg + ((long)y * W + x) * C + c;
-#pragma unroll
-    for (int r = 0; r < R21; ++r) {
-      float acc = 0.f;
-#pragma unroll
-      for (int t = 0; t < 21; ++t) acc = fmaf(w[t], v[r + t], acc);
-      o[r * stride] = from_f32<TO>(acc);
-    }
-    return;
-  }
-#pragma unroll
-  for (int i = 0; i < R21 + 20; ++i) {
-    if (AXIS == 0) {
-      const int xx = x + i - 10;
-      v[i] = (xx >= 0 && xx < W) ? img[((long)y * W + xx) * C + c] : 0.f;
-    } else {
-      const int yy = y + i - 10;
-      v[i] = (yy >= 0 && yy < H) ? img[((long)yy * W + x) * C + c] : 0.f;
-    }
-  }
-#pragma unroll
-  for (int r = 0; r < R21; ++r) {
-    float acc = 0.f;
-#pragma unroll
-    for (int t = 0; t < 21; ++t) acc = fmaf(w[t], v[r + t], acc);
-    if (AXIS == 0) {
-      if (x + r < W) oimg[((long)y * W + x + r) * C + c] = from_f32<TO>(acc);
-    } else {
-      if (y + r < H) oimg[((long)(y + r) * W + x) * C + c] = from_f32<TO>(acc);
-    }
-  }
-}
-
-// Rolling-window 21-tap pass: a thread owns one channel and a STRIP of up to `strip` outputs along the conv axis and walks it
-// in chunks of 16.  The 36-value window stays in registers; each chunk loads only its 16 new values, and loads them one
-// chunk AHEAD, so their latency hides behind the 336 FMAs of the current chunk (the one-shot kernel above loads 36 values per
-// 16 outputs and then waits: ncu showed 44 % of the issue cycles without an eligible warp at 29 % occupancy).
-// Tap order of every output is t = 0..20 as above: results are bit-identical to k_lka_dw21.
+// Rolling-window 21-tap pass, AXIS = 0: taps along W (1x21); AXIS = 1: taps along H (21x1).  A thread owns one channel and a
+// STRIP of up to `strip` outputs along the conv axis and walks it in chunks of 16.  The 36-value window stays in registers;
+// each chunk loads only its 16 new values, and loads them one chunk AHEAD, so their latency hides behind the 336 FMAs of the
+// current chunk (a one-shot kernel that loaded 36 values per 16 outputs and then waited had 44 % of the issue cycles without
+// an eligible warp at 29 % occupancy in ncu).  Every output sums its taps in the order t = 0..20.
 template <int AXIS, typename TO, int CT>
 __global__ void __launch_bounds__(256) k_lka_dw21_roll(const float* __restrict__ in, int H, int W, int C_rt, const float* __restrict__ w21,
                                                        TO* __restrict__ out, int strip, int nstrips) {
@@ -229,6 +158,15 @@ __global__ void __launch_bounds__(256) k_lka_dw21_roll(const float* __restrict__
   }
 }
 
+// A line of L outputs of the rolling-window passes as `n` strips of `len` <= 256 outputs (a multiple of 16)
+struct DwStrips {
+  int n, len;
+};
+static DwStrips dw_strips(int L) {
+  const int n = ceil_div(L, 256);
+  return {n, ceil_div(ceil_div(L, n), 16) * 16};
+}
+
 // x: [N][H][W][C] -> out: [N][H][W][C]; tmp1/tmp2: same-size scratch (tmp2 may alias out? no: distinct)
 static int lka_depthwise_impl(const void* x, int x_dtype, int N, int H, int W, int C, const float* bn_k, const float* bn_d,
                               const float* w5, const float* wh, const float* wv, float* tmp1, float* tmp2, void* out,
@@ -256,30 +194,17 @@ static int lka_depthwise_impl(const void* x, int x_dtype, int N, int H, int W, i
   const int ty = 256 / cx;
   const dim3 block(cx, ty);
   const dim3 g5(C / cx, ceil_div((long)ceil_div(H, R5) * ceil_div(W, R5), ty), N);
-  const dim3 gh(C / cx, ceil_div((long)H * ceil_div(W, R21), ty), N);
-  const dim3 gv(C / cx, ceil_div((long)ceil_div(H, R21) * W, ty), N);
   typedef __nv_bfloat16 bf;
-  // rolling-window 21-tap passes: strips of <= `target` outputs (a multiple of 16) along the conv axis
-  static const int target = getenv("FFSR_DW_STRIP") ? atoi(getenv("FFSR_DW_STRIP")) : 256;
-  const bool roll = target > 0;
-  const int tg = target > 0 ? target : 128;
-  const int nsw = ceil_div(W, tg), sw = ceil_div(ceil_div(W, nsw), 16) * 16;
-  const int nsh = ceil_div(H, tg), sh = ceil_div(ceil_div(H, nsh), 16) * 16;
-  const dim3 rh(C / cx, ceil_div((long)H * nsw, ty), N);
-  const dim3 rv(C / cx, ceil_div((long)W * nsh, ty), N);
-#define FFSR_DW_CHAIN(CT)                                                                                              \
-  {                                                                                                                    \
-    if (x_dtype == 1) k_lka_dw5<bf, CT><<<g5, block, 0, stream>>>((const bf*)x, H, W, C, bn_k, bn_d, w5, tmp1); \
-    else k_lka_dw5<float, CT><<<g5, block, 0, stream>>>((const float*)x, H, W, C, bn_k, bn_d, w5, tmp1);               \
-    if (!roll) {                                                                                                       \
-      k_lka_dw21<0, float, CT><<<gh, block, 0, stream>>>(tmp1, H, W, C, wh, tmp2);                                     \
-      if (out_dtype == 1) k_lka_dw21<1, bf, CT><<<gv, block, 0, stream>>>(tmp2, H, W, C, wv, (bf*)out);                \
-      else k_lka_dw21<1, float, CT><<<gv, block, 0, stream>>>(tmp2, H, W, C, wv, (float*)out);                         \
-    } else {                                                                                                           \
-      k_lka_dw21_roll<0, float, CT><<<rh, block, 0, stream>>>(tmp1, H, W, C, wh, tmp2, sw, nsw);                       \
-      if (out_dtype == 1) k_lka_dw21_roll<1, bf, CT><<<rv, block, 0, stream>>>(tmp2, H, W, C, wv, (bf*)out, sh, nsh);  \
-      else k_lka_dw21_roll<1, float, CT><<<rv, block, 0, stream>>>(tmp2, H, W, C, wv, (float*)out, sh, nsh);           \
-    }                                                                                                                  \
+  const DwStrips sw = dw_strips(W), sh = dw_strips(H);
+  const dim3 rh(C / cx, ceil_div((long)H * sw.n, ty), N);
+  const dim3 rv(C / cx, ceil_div((long)W * sh.n, ty), N);
+#define FFSR_DW_CHAIN(CT)                                                                                                    \
+  {                                                                                                                          \
+    if (x_dtype == 1) k_lka_dw5<bf, CT><<<g5, block, 0, stream>>>((const bf*)x, H, W, C, bn_k, bn_d, w5, tmp1);             \
+    else k_lka_dw5<float, CT><<<g5, block, 0, stream>>>((const float*)x, H, W, C, bn_k, bn_d, w5, tmp1);                     \
+    k_lka_dw21_roll<0, float, CT><<<rh, block, 0, stream>>>(tmp1, H, W, C, wh, tmp2, sw.len, sw.n);                          \
+    if (out_dtype == 1) k_lka_dw21_roll<1, bf, CT><<<rv, block, 0, stream>>>(tmp2, H, W, C, wv, (bf*)out, sh.len, sh.n);     \
+    else k_lka_dw21_roll<1, float, CT><<<rv, block, 0, stream>>>(tmp2, H, W, C, wv, (float*)out, sh.len, sh.n);              \
   }
   if (C == 128) FFSR_DW_CHAIN(128) else if (C == 64) FFSR_DW_CHAIN(64) else FFSR_DW_CHAIN(0)
 #undef FFSR_DW_CHAIN
@@ -306,18 +231,18 @@ extern "C" int ffsr_dwconv_stage(const float* in, int N, int H, int W, int C, in
     dim3 grid(C / cx, ceil_div((long)ceil_div(H, R5) * ceil_div(W, R5), ty), N);
     k_lka_dw5<float><<<grid, block, 0, stream>>>(in, H, W, C, bn_k, bn_d, w, out);
   } else {
-    // the rolling-window passes of the inference chain (bit-identical, see k_lka_dw21_roll); strips of <= 256 outputs
-    const int L = kind == 1 ? W : H, lines = kind == 1 ? H : W;
-    const int ns = ceil_div(L, 256), strip = ceil_div(ceil_div(L, ns), 16) * 16;
-    dim3 grid(C / cx, ceil_div((long)lines * ns, ty), N);
+    // the rolling-window passes of the inference chain, cut into the same strips
+    const int lines = kind == 1 ? H : W;
+    const DwStrips st = dw_strips(kind == 1 ? W : H);
+    dim3 grid(C / cx, ceil_div((long)lines * st.n, ty), N);
     if (kind == 1) {
-      if (C == 128) k_lka_dw21_roll<0, float, 128><<<grid, block, 0, stream>>>(in, H, W, C, w, out, strip, ns);
-      else if (C == 64) k_lka_dw21_roll<0, float, 64><<<grid, block, 0, stream>>>(in, H, W, C, w, out, strip, ns);
-      else k_lka_dw21_roll<0, float, 0><<<grid, block, 0, stream>>>(in, H, W, C, w, out, strip, ns);
+      if (C == 128) k_lka_dw21_roll<0, float, 128><<<grid, block, 0, stream>>>(in, H, W, C, w, out, st.len, st.n);
+      else if (C == 64) k_lka_dw21_roll<0, float, 64><<<grid, block, 0, stream>>>(in, H, W, C, w, out, st.len, st.n);
+      else k_lka_dw21_roll<0, float, 0><<<grid, block, 0, stream>>>(in, H, W, C, w, out, st.len, st.n);
     } else {
-      if (C == 128) k_lka_dw21_roll<1, float, 128><<<grid, block, 0, stream>>>(in, H, W, C, w, out, strip, ns);
-      else if (C == 64) k_lka_dw21_roll<1, float, 64><<<grid, block, 0, stream>>>(in, H, W, C, w, out, strip, ns);
-      else k_lka_dw21_roll<1, float, 0><<<grid, block, 0, stream>>>(in, H, W, C, w, out, strip, ns);
+      if (C == 128) k_lka_dw21_roll<1, float, 128><<<grid, block, 0, stream>>>(in, H, W, C, w, out, st.len, st.n);
+      else if (C == 64) k_lka_dw21_roll<1, float, 64><<<grid, block, 0, stream>>>(in, H, W, C, w, out, st.len, st.n);
+      else k_lka_dw21_roll<1, float, 0><<<grid, block, 0, stream>>>(in, H, W, C, w, out, st.len, st.n);
     }
   }
   return ffsr_check_launch("dwconv_stage");

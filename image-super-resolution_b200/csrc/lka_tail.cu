@@ -10,8 +10,9 @@
 // dropped terms are below 2^-24 of the result, i.e. below the rounding of an fp32 FMA chain.
 //   operands : no-swizzle K-major planes (tc_ptx.cuh): activations [split][kg][row] = 16 B, weights [split][kg][n] = 16 B, all
 //              three weight matrices resident (120 KB); the 128-wide hidden layer is consumed in two 64-channel halves.
-//   threads  : 256 = 8 warps; warp w owns TMEM lanes 32 (w % 4) .. (the tcgen05.ld rule) = token rows, and column half w / 4;
-//              warp 0 issues the MMAs (one PTX block of four K steps per split pair) between the epilogue phases.
+//   threads  : 512 = 16 warps; warp w owns TMEM lanes 32 (w % 4) .. (the tcgen05.ld rule) = token rows, and channel quarter
+//              w / 4 (16 of the 64 columns); warp 0 issues the MMAs (one PTX block of four K steps per split pair) between the
+//              epilogue phases.
 #include <cuda.h>
 #include <stdlib.h>
 #include "common.cuh"
@@ -22,7 +23,6 @@ namespace {
 using namespace tcx;
 
 constexpr int LT_C = 64, LT_HID = 128;
-constexpr int LT_THREADS = 256;
 constexpr int LT_TMEM_COLS = 256;                 // [0,64): stage 1 then stage 3; [64,192): stage 2
 constexpr int LT_W1 = 3 * LT_C * LT_C * 2;        // 24,576 B  pw        [split][kg 8][n 64][8]
 constexpr int LT_W0 = 3 * LT_HID * LT_C * 2;      // 49,152 B  ffn0      [split][kg 8][n 128][8]
@@ -73,187 +73,9 @@ __device__ __forceinline__ void lt_gemm(uint32_t tmem_d, uint32_t a32, uint32_t 
   }
 }
 
-__global__ void __launch_bounds__(LT_THREADS, 1) k_lka_tail(const float* __restrict__ xin, const float* __restrict__ ain, long rows,
-                                                            const uint8_t* __restrict__ wblob, const float* __restrict__ pblob,
-                                                            const float* __restrict__ s1p, const float* __restrict__ s2p,
-                                                            float* __restrict__ out) {
-  extern __shared__ __align__(16) uint8_t smem[];
-  uint64_t* bar = reinterpret_cast<uint64_t*>(smem);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + 8);
-  float* par = reinterpret_cast<float*>(smem + LT_S_PAR);
-  uint8_t* sW = smem + LT_S_W;
-  uint8_t* sA = smem + LT_S_A;
-  uint8_t* sH = smem + LT_S_H;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int row = (warp & 3) * 32 + lane;           // token row of the tile = TMEM lane
-  const int half = warp >> 2;                        // column half (32 of 64 columns)
-
-  for (int i = tid; i < LT_WBYTES / 16; i += LT_THREADS) reinterpret_cast<uint4*>(sW)[i] = __ldg(reinterpret_cast<const uint4*>(wblob) + i);
-  for (int i = tid; i < LT_PF; i += LT_THREADS) par[i] = __ldg(pblob + i);
-  if (tid == 0) {
-    mbar_init(bar, 1);
-    fence_barrier_init();
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(LT_TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
-  fence_proxy_async();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  const float s1 = s1p[0], s2 = s2p[0];
-  const float* b_pw = par;
-  const float* k1 = par + 64;
-  const float* d1 = par + 128;
-  const float* b0 = par + 192;
-  const float* b2 = par + 320;
-  const uint32_t w1_32 = smem_u32(sW), w0_32 = w1_32 + LT_W1, w2_32 = w0_32 + LT_W0, a32 = smem_u32(sA), h32 = smem_u32(sH);
-  const uint32_t id64 = idesc_bf16_m128(64), id128 = idesc_bf16_m128(128);
-  const uint32_t trow = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-  uint32_t phase = 0;
-  const long tiles = (rows + 127) / 128;
-
-  for (long tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-    const long r = tile * 128 + row;
-    const bool live = r < rows;
-    float x[32];
-    // ---- a -> split planes; x (this thread's 32 channels) stays in registers
-    {
-      const float4* ap = reinterpret_cast<const float4*>(ain + r * LT_C + half * 32);
-      const float4* xp = reinterpret_cast<const float4*>(xin + r * LT_C + half * 32);
-#pragma unroll
-      for (int g = 0; g < 4; ++g) {                  // 8 channels = one 16-byte cell of each split
-        float v[8];
-        const float4 p0 = live ? __ldg(ap + 2 * g) : make_float4(0.f, 0.f, 0.f, 0.f), p1 = live ? __ldg(ap + 2 * g + 1) : make_float4(0.f, 0.f, 0.f, 0.f);
-        v[0] = p0.x; v[1] = p0.y; v[2] = p0.z; v[3] = p0.w; v[4] = p1.x; v[5] = p1.y; v[6] = p1.z; v[7] = p1.w;
-        uint4 c1, c2, c3;
-        split8(v, c1, c2, c3);
-        uint8_t* cell = sA + (half * 4 + g) * 2048 + row * 16;
-        *reinterpret_cast<uint4*>(cell) = c1;
-        *reinterpret_cast<uint4*>(cell + 8 * 2048) = c2;
-        *reinterpret_cast<uint4*>(cell + 16 * 2048) = c3;
-        const float4 q0 = live ? __ldg(xp + 2 * g) : make_float4(0.f, 0.f, 0.f, 0.f), q1 = live ? __ldg(xp + 2 * g + 1) : make_float4(0.f, 0.f, 0.f, 0.f);
-        x[8 * g] = q0.x; x[8 * g + 1] = q0.y; x[8 * g + 2] = q0.z; x[8 * g + 3] = q0.w;
-        x[8 * g + 4] = q1.x; x[8 * g + 5] = q1.y; x[8 * g + 6] = q1.z; x[8 * g + 7] = q1.w;
-      }
-    }
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    // ---- stage 1: G = a . Wpw^T
-    if (warp == 0) {
-      tc_fence_after();
-      lt_gemm(tmem, a32, w1_32, 64, 8, 0, 4, id64, true);
-      umma_commit(bar);
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1;
-    tc_fence_after();
-    // ---- epilogue 1: x1 = x + s1 * (x k1 + d1) * sigmoid(G + b); x1 -> registers and split planes
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      uint32_t v[16];
-      tmem_ld16(trow + (uint32_t)(half * 32 + c * 16), v);
-      tmem_wait_ld(v);
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const int ch = half * 32 + c * 16 + i;
-        const float xr = x[c * 16 + i];
-        x[c * 16 + i] = xr + s1 * (fmaf(xr, k1[ch], d1[ch]) * sigmoid_acc(__uint_as_float(v[i]) + b_pw[ch]));
-      }
-    }
-    tc_fence_before();
-    __syncthreads();                                 // stage-1 operands and accumulator are dead
-#pragma unroll
-    for (int g = 0; g < 4; ++g) {
-      float v[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) v[i] = x[8 * g + i];
-      uint4 c1, c2, c3;
-      split8(v, c1, c2, c3);
-      uint8_t* cell = sA + (half * 4 + g) * 2048 + row * 16;
-      *reinterpret_cast<uint4*>(cell) = c1;
-      *reinterpret_cast<uint4*>(cell + 8 * 2048) = c2;
-      *reinterpret_cast<uint4*>(cell + 16 * 2048) = c3;
-    }
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    // ---- stage 2: Hd = x1 . W0^T  (128 columns at TMEM column 64)
-    if (warp == 0) {
-      tc_fence_after();
-      lt_gemm(tmem + 64, a32, w0_32, 128, 8, 0, 4, id128, true);
-      umma_commit(bar);
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1;
-    tc_fence_after();
-    // ---- stage 3 in two hidden halves: GELU(Hd + b0) -> split planes -> x2 += . W2^T
-#pragma unroll 1
-    for (int hh = 0; hh < 2; ++hh) {
-#pragma unroll
-      for (int c = 0; c < 2; ++c) {
-        uint32_t v[16];
-        tmem_ld16(trow + (uint32_t)(64 + hh * 64 + half * 32 + c * 16), v);
-        tmem_wait_ld(v);
-#pragma unroll
-        for (int g = 0; g < 2; ++g) {
-          float y[8];
-#pragma unroll
-          for (int i = 0; i < 8; ++i) y[i] = gelu_erf(__uint_as_float(v[g * 8 + i]) + b0[hh * 64 + half * 32 + c * 16 + g * 8 + i]);
-          uint4 c1, c2, c3;
-          split8(y, c1, c2, c3);
-          uint8_t* cell = sH + (half * 4 + c * 2 + g) * 2048 + row * 16;
-          *reinterpret_cast<uint4*>(cell) = c1;
-          *reinterpret_cast<uint4*>(cell + 8 * 2048) = c2;
-          *reinterpret_cast<uint4*>(cell + 16 * 2048) = c3;
-        }
-      }
-      fence_proxy_async();
-      tc_fence_before();
-      __syncthreads();
-      if (warp == 0) {
-        tc_fence_after();
-        lt_gemm(tmem, h32, w2_32, 64, 16, hh * 8, 4, id64, hh == 0);
-        umma_commit(bar);
-      }
-      mbar_wait(bar, phase);
-      phase ^= 1;
-      tc_fence_after();
-    }
-    // ---- epilogue 3: x2 = x1 + s2 * (acc + b2)
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      uint32_t v[16];
-      tmem_ld16(trow + (uint32_t)(half * 32 + c * 16), v);
-      tmem_wait_ld(v);
-      if (live) {
-        float4* op = reinterpret_cast<float4*>(out + r * LT_C + half * 32 + c * 16);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          float o[4];
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const int j = q * 4 + i;
-            o[i] = fmaf(s2, __uint_as_float(v[j]) + b2[half * 32 + c * 16 + j], x[c * 16 + j]);
-          }
-          op[q] = make_float4(o[0], o[1], o[2], o[3]);
-        }
-      }
-    }
-    tc_fence_before();
-    __syncthreads();                                 // TMEM and the planes are free for the next tile
-    tc_fence_after();
-  }
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(LT_TMEM_COLS));
-}
-
-// 512-thread version of k_lka_tail (warp w: TMEM lane group w % 4, channel quarter w / 4 = 16 of the 64 columns): half the
-// instructions per thread at four warps per scheduler, the next tile's rows prefetched into registers, and the second hidden
-// half written to the (dead) x1 planes so the two ffn2 MMA groups are issued without a wait in between.  Same products in the
-// same order as k_lka_tail: bit-identical output.
+// 512 threads rather than 256: half the instructions per thread at four warps per scheduler.  The next tile's rows are
+// prefetched into registers, and the second hidden half is written to the (dead) x1 planes so the two ffn2 MMA groups are
+// issued without a wait in between.
 __global__ void __launch_bounds__(512, 1) k_lka_tailw(const float* __restrict__ xin, const float* __restrict__ ain, long rows,
                                                       const uint8_t* __restrict__ wblob, const float* __restrict__ pblob,
                                                       const float* __restrict__ s1p, const float* __restrict__ s2p,
@@ -447,222 +269,12 @@ constexpr int LB_S_H = LB_S_A + 16 * 2048;        // hidden quarter planes [kg 8
 constexpr int LB_SMEM = LB_S_H + 8 * 2048;        // 225,280 B
 constexpr int LB_TMEM_COLS = 512;                 // [0,128): stage 1 / 3; [128,384): stage 2; [128,160): modulation layer
 
-template <bool TANH>
-__global__ void __launch_bounds__(LT_THREADS, 1) k_lka_tail128(const __nv_bfloat16* __restrict__ xin, const __nv_bfloat16* __restrict__ ain,
-                                                               int nimg, int HW, const uint8_t* __restrict__ wblob,
-                                                               const float* __restrict__ pblob, const float* __restrict__ s1p,
-                                                               const float* __restrict__ s2p, __nv_bfloat16* __restrict__ m32) {
-  extern __shared__ __align__(16) uint8_t smem[];
-  uint64_t* bar = reinterpret_cast<uint64_t*>(smem);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + 8);
-  float* par = reinterpret_cast<float*>(smem + LB_S_PAR);
-  uint8_t* sW = smem + LB_S_W;
-  uint8_t* sWM = smem + LB_S_WM;
-  uint8_t* sA = smem + LB_S_A;
-  uint8_t* sH = smem + LB_S_H;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int row = (warp & 3) * 32 + lane;
-  const int half = warp >> 2;                        // 64 of the 128 columns
-
-  for (int i = tid; i < (LB_W1 + LB_W0 + LB_W2) / 16; i += LT_THREADS) reinterpret_cast<uint4*>(sW)[i] = __ldg(reinterpret_cast<const uint4*>(wblob) + i);
-  for (int i = tid; i < LB_PF; i += LT_THREADS) par[i] = __ldg(pblob + i);
-  if (tid == 0) {
-    mbar_init(bar, 1);
-    fence_barrier_init();
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(LB_TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
-  fence_proxy_async();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  const float s1 = s1p[0], s2 = s2p[0];
-  const float* b_pw = par;
-  const float* k1 = par + 128;
-  const float* d1 = par + 256;
-  const float* b0 = par + 384;
-  const float* b2 = par + 640;
-  const float* bm = par + 768;
-  const uint32_t w1_32 = smem_u32(sW), w0_32 = w1_32 + LB_W1, w2_32 = w0_32 + LB_W0, wm_32 = smem_u32(sWM), a32 = smem_u32(sA), h32 = smem_u32(sH);
-  const uint32_t hi = desc_hi(128);
-  const uint32_t id128 = idesc_bf16_m128(128), id256 = idesc_bf16_m128(256), id32 = idesc_bf16_m128(32);
-  const uint32_t trow = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-  uint32_t phase = 0;
-  const int tpi = (HW + 127) / 128;                  // tiles per image
-  const long tiles = (long)nimg * tpi;
-  int cur_e = -1;
-
-  for (long tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-    const int n = (int)(tile / tpi), t = (int)(tile - (long)n * tpi);
-    const int e = n & 3;
-    const int pr = t * 128 + row;
-    const bool live = pr < HW;
-    const long r = (long)n * HW + (live ? pr : 0);
-    if (e != cur_e) {                                // (uniform) this expert's modulation weights; the previous tile's MMAs are done
-      for (int i = tid; i < LB_WM / 16; i += LT_THREADS)
-        reinterpret_cast<uint4*>(sWM)[i] = __ldg(reinterpret_cast<const uint4*>(wblob + LB_W1 + LB_W0 + LB_W2 + e * LB_WM) + i);
-      cur_e = e;
-    }
-    // ---- a -> planes (bf16 cells copied whole); x (64 channels of this thread) -> fp32 registers
-    float x[64];
-    {
-      const uint4* ap = reinterpret_cast<const uint4*>(ain + r * LB_C + half * 64);
-      const uint4* xp = reinterpret_cast<const uint4*>(xin + r * LB_C + half * 64);
-#pragma unroll
-      for (int g = 0; g < 8; ++g) {
-        const uint4 z = make_uint4(0u, 0u, 0u, 0u);
-        *reinterpret_cast<uint4*>(sA + (half * 8 + g) * 2048 + row * 16) = live ? __ldg(ap + g) : z;
-        const uint4 q = live ? __ldg(xp + g) : z;
-        const uint32_t w[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          const float2 f2 = unpack_bf16(w[k]);
-          x[g * 8 + 2 * k] = f2.x;
-          x[g * 8 + 2 * k + 1] = f2.y;
-        }
-      }
-    }
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    // ---- stage 1: G = a . Wpw^T (K = 128, N = 128)
-    if (warp == 0) {
-      tc_fence_after();
-      umma_taps_1x4(tmem, desc_lo(a32, 2048u), desc_lo(w1_32, 128u * 16u), id128, 0u, hi, hi, (2u * 2048u) >> 4, 2u * 128u, 0u);
-      umma_taps_1x4(tmem, desc_lo(a32 + 8u * 2048u, 2048u), desc_lo(w1_32 + 8u * 128u * 16u, 128u * 16u), id128, 1u, hi, hi, (2u * 2048u) >> 4, 2u * 128u, 0u);
-      umma_commit(bar);
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1;
-    tc_fence_after();
-    // ---- epilogue 1: x1 = x + s1 * (x k1 + d1) * sigmoid(G + b) -> registers and planes
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      uint32_t v[16];
-      tmem_ld16(trow + (uint32_t)(half * 64 + c * 16), v);
-      tmem_wait_ld(v);
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const int ch = half * 64 + c * 16 + i;
-        const float xr = x[c * 16 + i];
-        x[c * 16 + i] = xr + s1 * (fmaf(xr, k1[ch], d1[ch]) * sigmoid_acc(__uint_as_float(v[i]) + b_pw[ch]));
-      }
-    }
-    tc_fence_before();
-    __syncthreads();
-#pragma unroll
-    for (int g = 0; g < 8; ++g)
-      *reinterpret_cast<uint4*>(sA + (half * 8 + g) * 2048 + row * 16) =
-          make_uint4(pack_bf16(x[g * 8], x[g * 8 + 1]), pack_bf16(x[g * 8 + 2], x[g * 8 + 3]), pack_bf16(x[g * 8 + 4], x[g * 8 + 5]),
-                     pack_bf16(x[g * 8 + 6], x[g * 8 + 7]));
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    // ---- stage 2: Hd = x1 . W0^T (K = 128, N = 256) at TMEM column 128
-    if (warp == 0) {
-      tc_fence_after();
-      umma_taps_1x4(tmem + 128, desc_lo(a32, 2048u), desc_lo(w0_32, 256u * 16u), id256, 0u, hi, hi, (2u * 2048u) >> 4, 2u * 256u, 0u);
-      umma_taps_1x4(tmem + 128, desc_lo(a32 + 8u * 2048u, 2048u), desc_lo(w0_32 + 8u * 256u * 16u, 256u * 16u), id256, 1u, hi, hi, (2u * 2048u) >> 4, 2u * 256u, 0u);
-      umma_commit(bar);
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1;
-    tc_fence_after();
-    // ---- stage 3 in four hidden quarters of 64: GELU(Hd + b0) -> planes -> acc += . W2^T
-#pragma unroll 1
-    for (int q = 0; q < 4; ++q) {
-#pragma unroll
-      for (int c = 0; c < 2; ++c) {
-        uint32_t v[16];
-        tmem_ld16(trow + (uint32_t)(128 + q * 64 + half * 32 + c * 16), v);
-        tmem_wait_ld(v);
-        float y[16];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          const float z = __uint_as_float(v[i]) + b0[q * 64 + half * 32 + c * 16 + i];
-          y[i] = TANH ? gelu_tanh_fast(z) : gelu_erf_fast(z);
-        }
-#pragma unroll
-        for (int g = 0; g < 2; ++g)
-          *reinterpret_cast<uint4*>(sH + (half * 4 + c * 2 + g) * 2048 + row * 16) =
-              make_uint4(pack_bf16(y[g * 8], y[g * 8 + 1]), pack_bf16(y[g * 8 + 2], y[g * 8 + 3]), pack_bf16(y[g * 8 + 4], y[g * 8 + 5]),
-                         pack_bf16(y[g * 8 + 6], y[g * 8 + 7]));
-      }
-      fence_proxy_async();
-      tc_fence_before();
-      __syncthreads();
-      if (warp == 0) {
-        tc_fence_after();
-        umma_taps_1x4(tmem, desc_lo(h32, 2048u), desc_lo(w2_32 + (uint32_t)(q * 8) * 128u * 16u, 128u * 16u), id128, q == 0 ? 0u : 1u, hi, hi,
-                      (2u * 2048u) >> 4, 2u * 128u, 0u);
-        umma_commit(bar);
-      }
-      mbar_wait(bar, phase);
-      phase ^= 1;
-      tc_fence_after();
-    }
-    // ---- epilogue 3: x2 = x1 + s2 * (acc + b2) -> planes
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      uint32_t v[16];
-      tmem_ld16(trow + (uint32_t)(half * 64 + c * 16), v);
-      tmem_wait_ld(v);
-#pragma unroll
-      for (int i = 0; i < 16; ++i) x[c * 16 + i] = fmaf(s2, __uint_as_float(v[i]) + b2[half * 64 + c * 16 + i], x[c * 16 + i]);
-    }
-#pragma unroll
-    for (int g = 0; g < 8; ++g)
-      *reinterpret_cast<uint4*>(sA + (half * 8 + g) * 2048 + row * 16) =
-          make_uint4(pack_bf16(x[g * 8], x[g * 8 + 1]), pack_bf16(x[g * 8 + 2], x[g * 8 + 3]), pack_bf16(x[g * 8 + 4], x[g * 8 + 5]),
-                     pack_bf16(x[g * 8 + 6], x[g * 8 + 7]));
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    // ---- stage 4: modulation layer 0 of this expert, m32 = x2 . Wm^T (K = 128, N = 32) at TMEM column 128
-    if (warp == 0) {
-      tc_fence_after();
-      umma_taps_1x4(tmem + 128, desc_lo(a32, 2048u), desc_lo(wm_32, 32u * 16u), id32, 0u, hi, hi, (2u * 2048u) >> 4, 2u * 32u, 0u);
-      umma_taps_1x4(tmem + 128, desc_lo(a32 + 8u * 2048u, 2048u), desc_lo(wm_32 + 8u * 32u * 16u, 32u * 16u), id32, 1u, hi, hi, (2u * 2048u) >> 4, 2u * 32u, 0u);
-      umma_commit(bar);
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1;
-    tc_fence_after();
-    if (half == 0) {
-      uint32_t v0[16], v1[16];
-      tmem_ld16(trow + 128u, v0);
-      tmem_ld16(trow + 144u, v1);
-      tmem_wait_ld(v0);
-      tmem_wait_ld(v1);
-      if (live) {
-        const float* bb = bm + e * 32;
-        uint4* op = reinterpret_cast<uint4*>(m32 + r * 32);
-        op[0] = make_uint4(pack_bf16(__uint_as_float(v0[0]) + bb[0], __uint_as_float(v0[1]) + bb[1]), pack_bf16(__uint_as_float(v0[2]) + bb[2], __uint_as_float(v0[3]) + bb[3]),
-                           pack_bf16(__uint_as_float(v0[4]) + bb[4], __uint_as_float(v0[5]) + bb[5]), pack_bf16(__uint_as_float(v0[6]) + bb[6], __uint_as_float(v0[7]) + bb[7]));
-        op[1] = make_uint4(pack_bf16(__uint_as_float(v0[8]) + bb[8], __uint_as_float(v0[9]) + bb[9]), pack_bf16(__uint_as_float(v0[10]) + bb[10], __uint_as_float(v0[11]) + bb[11]),
-                           pack_bf16(__uint_as_float(v0[12]) + bb[12], __uint_as_float(v0[13]) + bb[13]), pack_bf16(__uint_as_float(v0[14]) + bb[14], __uint_as_float(v0[15]) + bb[15]));
-        op[2] = make_uint4(pack_bf16(__uint_as_float(v1[0]) + bb[16], __uint_as_float(v1[1]) + bb[17]), pack_bf16(__uint_as_float(v1[2]) + bb[18], __uint_as_float(v1[3]) + bb[19]),
-                           pack_bf16(__uint_as_float(v1[4]) + bb[20], __uint_as_float(v1[5]) + bb[21]), pack_bf16(__uint_as_float(v1[6]) + bb[22], __uint_as_float(v1[7]) + bb[23]));
-        op[3] = make_uint4(pack_bf16(__uint_as_float(v1[8]) + bb[24], __uint_as_float(v1[9]) + bb[25]), pack_bf16(__uint_as_float(v1[10]) + bb[26], __uint_as_float(v1[11]) + bb[27]),
-                           pack_bf16(__uint_as_float(v1[12]) + bb[28], __uint_as_float(v1[13]) + bb[29]), pack_bf16(__uint_as_float(v1[14]) + bb[30], __uint_as_float(v1[15]) + bb[31]));
-      }
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-  }
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(LB_TMEM_COLS));
-}
-
 // ---------------------------------------------------------------------------------------------------------------------
-// k_lka_tail128w: the same chain with 512 threads (warp w: TMEM lane group w % 4 = 32 token rows, channel quarter w / 4), the
-// next tile's rows prefetched into registers, and the four hidden quarters written alternately to sH and to the two halves
-// of the (by then dead) x1 planes, so the four ffn2 MMAs are issued back to back with the GELU epilogues instead of being
-// waited for one by one.  ncu of the 256-thread version: 3.3 k instructions per thread and tile at two warps per scheduler,
-// 75 % of the issue cycles without an eligible warp (long-scoreboard on the un-prefetched loads, MMA waits).
+// k_lka_tail128w: 512 threads (warp w: TMEM lane group w % 4 = 32 token rows, channel quarter w / 4), the next tile's rows
+// prefetched into registers, and the four hidden quarters written alternately to sH and to the two halves of the (by then
+// dead) x1 planes, so the four ffn2 MMAs are issued back to back with the GELU epilogues instead of being waited for one by
+// one.  ncu of an earlier 256-thread version: 3.3 k instructions per thread and tile at two warps per scheduler, 75 % of the
+// issue cycles without an eligible warp (long-scoreboard on the un-prefetched loads, MMA waits).
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int LW_THREADS = 512;
 
@@ -912,21 +524,11 @@ extern "C" int ffsr_lka_tail64(const float* x, const float* a, long rows, const 
     int dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaFuncSetAttribute(k_lka_tail, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_SMEM);
+    cudaFuncSetAttribute(k_lka_tailw, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_SMEM);
   }
   const long tiles = (rows + 127) / 128;
   const int grid = (int)(tiles < num_sms ? tiles : num_sms);
-  static const bool v1 = getenv("FFSR_LKA_TAIL64_V1") != nullptr;
-  if (!v1) {
-    static bool attr = false;
-    if (!attr) {
-      cudaFuncSetAttribute(k_lka_tailw, cudaFuncAttributeMaxDynamicSharedMemorySize, LT_SMEM);
-      attr = true;
-    }
-    k_lka_tailw<<<grid, 512, LT_SMEM, stream>>>(x, a, rows, (const uint8_t*)wblob, pblob, scale1, scale2, out);
-    return ffsr_check_launch("lka_tail64");
-  }
-  k_lka_tail<<<grid, LT_THREADS, LT_SMEM, stream>>>(x, a, rows, (const uint8_t*)wblob, pblob, scale1, scale2, out);
+  k_lka_tailw<<<grid, 512, LT_SMEM, stream>>>(x, a, rows, (const uint8_t*)wblob, pblob, scale1, scale2, out);
   return ffsr_check_launch("lka_tail64");
 }
 
@@ -945,32 +547,16 @@ extern "C" int ffsr_lka_tail128_mod(const void* x, const void* a, int nimg, int 
     int dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaFuncSetAttribute(k_lka_tail128<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LB_SMEM);
-    cudaFuncSetAttribute(k_lka_tail128<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, LB_SMEM);
+    cudaFuncSetAttribute(k_lka_tail128w<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LB_SMEM);
+    cudaFuncSetAttribute(k_lka_tail128w<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, LB_SMEM);
   }
   const long tiles = (long)nimg * ((HW + 127) / 128);
   const int grid = (int)(tiles < num_sms ? tiles : num_sms);
-  static const bool v1 = getenv("FFSR_LKA_TAIL128_V1") != nullptr;
-  if (!v1) {
-    static bool attr = false;
-    if (!attr) {
-      cudaFuncSetAttribute(k_lka_tail128w<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LB_SMEM);
-      cudaFuncSetAttribute(k_lka_tail128w<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, LB_SMEM);
-      attr = true;
-    }
-    if (erf_forced)
-      k_lka_tail128w<false><<<grid, LW_THREADS, LB_SMEM, stream>>>((const __nv_bfloat16*)x, (const __nv_bfloat16*)a, nimg, HW, (const uint8_t*)wblob,
-                                                                    pblob, scale1, scale2, (__nv_bfloat16*)m32);
-    else
-      k_lka_tail128w<true><<<grid, LW_THREADS, LB_SMEM, stream>>>((const __nv_bfloat16*)x, (const __nv_bfloat16*)a, nimg, HW, (const uint8_t*)wblob,
-                                                                   pblob, scale1, scale2, (__nv_bfloat16*)m32);
-    return ffsr_check_launch("lka_tail128_mod");
-  }
   if (erf_forced)
-    k_lka_tail128<false><<<grid, LT_THREADS, LB_SMEM, stream>>>((const __nv_bfloat16*)x, (const __nv_bfloat16*)a, nimg, HW, (const uint8_t*)wblob, pblob,
-                                                                scale1, scale2, (__nv_bfloat16*)m32);
+    k_lka_tail128w<false><<<grid, LW_THREADS, LB_SMEM, stream>>>((const __nv_bfloat16*)x, (const __nv_bfloat16*)a, nimg, HW, (const uint8_t*)wblob,
+                                                                  pblob, scale1, scale2, (__nv_bfloat16*)m32);
   else
-    k_lka_tail128<true><<<grid, LT_THREADS, LB_SMEM, stream>>>((const __nv_bfloat16*)x, (const __nv_bfloat16*)a, nimg, HW, (const uint8_t*)wblob, pblob,
-                                                               scale1, scale2, (__nv_bfloat16*)m32);
+    k_lka_tail128w<true><<<grid, LW_THREADS, LB_SMEM, stream>>>((const __nv_bfloat16*)x, (const __nv_bfloat16*)a, nimg, HW, (const uint8_t*)wblob,
+                                                                 pblob, scale1, scale2, (__nv_bfloat16*)m32);
   return ffsr_check_launch("lka_tail128_mod");
 }

@@ -5,217 +5,27 @@
 //   * LayerNorm rows and the 4-token x 8-head attention core used by Phase 4 (:389-392)
 //   * Phase 6 gate normalisation (DynamicExpertSelector.forward, enhanced_fusion_v2.py:462-465)
 // All fp32: routing_lr feeds the expert-selection indices that must be bit-exact.
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace {
-constexpr int CB_DIM = 64, CB_BANDS = 9, CB_HEADS = 4, CB_HD = 16;
-constexpr int CB_PX = 8;                       // LR pixels per tile
-constexpr int CB_TOK = CB_PX * CB_BANDS;       // 72 tokens per tile
-constexpr int CB_THREADS = 192;                // one thread per packed in_proj row
-constexpr int CB_QKV_LD = 3 * CB_DIM + 4;      // +4 floats: keeps rows 16B aligned, breaks bank stride
-
-struct CBSmem {
-  float in[CB_PX][28];                 // 27 band/channel values per pixel
-  float n[CB_TOK][CB_DIM];             // LayerNorm'ed tokens; later the attention context
-  float qkv[CB_TOK][CB_QKV_LD];
-  float wo[CB_DIM][CB_DIM];            // out_proj weight transposed: wo[c][o]
-  float pw[CB_DIM][4];                 // band_proj weight [o][3] + bias in slot 3
-  float lnw[CB_DIM], lnb[CB_DIM], ob[CB_DIM];
-  float fa[CB_DIM][4];                 // folded path: centred band_proj rows A[c][0..2] and centred bias c[c]
-  float rstd[CB_TOK];                  // folded path: LayerNorm 1/std per token
-};
+constexpr int CB_DIM = 64, CB_BANDS = 9, CB_HD = 16;
 }  // namespace
 
-// FOLD: band_proj -> LayerNorm -> in_proj collapsed algebraically.  A token is an affine function of the 3 band
-// values x:  t = Wp x + b;  t - mean(t) = A x + c;  LN(t) = (A x + c) * rstd * gamma + beta;  so
+// ------------------------------------------------------------------------------------
+// Cross-band attention with band_proj -> LayerNorm -> in_proj collapsed algebraically.  A token is an affine function of
+// the 3 band values x:  t = Wp x + b;  t - mean(t) = A x + c;  LN(t) = (A x + c) * rstd * gamma + beta;  so
 //   qkv = W_in LN(t) + b_in = rstd * (M x + m0) + n0,   M = W_in diag(gamma) A  [192x3],  m0 = W_in diag(gamma) c,
 //   n0 = W_in beta + b_in  (folded on the host in fp64): 4 FMAs per qkv channel instead of 64, with the variance
 // still taken from the 64 centred values themselves.  fold = [A|c : 64x4][M|m0 : 192x4][n0 : 192].
-template <bool FOLD>
-__global__ void __launch_bounds__(CB_THREADS, 2) k_crossband_attn(
-    const float* __restrict__ fold,
-    const float* __restrict__ raw9, int B, int HW,
-    const float* __restrict__ proj_w, const float* __restrict__ proj_b,
-    const float* __restrict__ ln_w, const float* __restrict__ ln_b,
-    const float* __restrict__ in_w, const float* __restrict__ in_b,
-    const float* __restrict__ out_w, const float* __restrict__ out_b,
-    int nq, float* __restrict__ tok_out) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  CBSmem& s = *reinterpret_cast<CBSmem*>(smem_raw);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-
-  // --- per-block constants -------------------------------------------------------------
-  for (int i = tid; i < CB_DIM * CB_DIM; i += CB_THREADS) {
-    const int o = i / CB_DIM, c = i % CB_DIM;
-    s.wo[c][o] = out_w[i];
-  }
-  if (tid < CB_DIM) {
-    s.pw[tid][0] = proj_w[tid * 3 + 0];
-    s.pw[tid][1] = proj_w[tid * 3 + 1];
-    s.pw[tid][2] = proj_w[tid * 3 + 2];
-    s.pw[tid][3] = proj_b[tid];
-    s.lnw[tid] = ln_w[tid];
-    s.lnb[tid] = ln_b[tid];
-    s.ob[tid] = out_b[tid];
-  }
-  float wrow[FOLD ? 4 : CB_DIM];       // this thread's in_proj row (q|k|v output channel tid), or its folded 3+1 row
-  float brow;
-  if (FOLD) {
-    const float4 v = *reinterpret_cast<const float4*>(fold + CB_DIM * 4 + (long)tid * 4);
-    wrow[0] = v.x; wrow[1] = v.y; wrow[2] = v.z; wrow[3] = v.w;
-    brow = fold[CB_DIM * 4 + 3 * CB_DIM * 4 + tid];
-    if (tid < CB_DIM) {
-      const float4 a = *reinterpret_cast<const float4*>(fold + tid * 4);
-      s.fa[tid][0] = a.x; s.fa[tid][1] = a.y; s.fa[tid][2] = a.z; s.fa[tid][3] = a.w;
-    }
-  } else {
-#pragma unroll
-    for (int c = 0; c < (FOLD ? 4 : CB_DIM); c += 4) {
-      const float4 v = *reinterpret_cast<const float4*>(in_w + (long)tid * CB_DIM + c);
-      wrow[c] = v.x; wrow[c + 1] = v.y; wrow[c + 2] = v.z; wrow[c + 3] = v.w;
-    }
-    brow = in_b[tid];
-  }
-  __syncthreads();
-
-  const int tiles_per_img = (HW + CB_PX - 1) / CB_PX;
-  const int total_tiles = B * tiles_per_img;
-  for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-    const int b = tile / tiles_per_img;
-    const int p0 = (tile % tiles_per_img) * CB_PX;
-
-    // A. gather the 27 inputs of each pixel
-    for (int i = tid; i < CB_PX * 27; i += CB_THREADS) {
-      const int px = i / 27, r = i % 27;
-      const int p = p0 + px;
-      s.in[px][r] = (p < HW) ? raw9[((long)b * 27 + r) * HW + p] : 0.f;
-    }
-    __syncthreads();
-
-    // B. band_proj (1x1, 3->64) + LayerNorm(64): one warp per token, 2 channels per lane
-    for (int tk = warp; tk < CB_TOK; tk += CB_THREADS / 32) {
-      const int px = tk / CB_BANDS, band = tk % CB_BANDS;
-      const float x0 = s.in[px][band * 3], x1 = s.in[px][band * 3 + 1], x2 = s.in[px][band * 3 + 2];
-      const int c0 = lane, c1 = lane + 32;
-      if (FOLD) {                        // only 1/std is needed: the centred values come straight from A x + c
-        const float d0 = fmaf(s.fa[c0][2], x2, fmaf(s.fa[c0][1], x1, fmaf(s.fa[c0][0], x0, s.fa[c0][3])));
-        const float d1 = fmaf(s.fa[c1][2], x2, fmaf(s.fa[c1][1], x1, fmaf(s.fa[c1][0], x0, s.fa[c1][3])));
-        float sq = d0 * d0 + d1 * d1;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
-        if (lane == 0) s.rstd[tk] = rsqrtf(sq * (1.0f / CB_DIM) + 1e-5f);
-        continue;
-      }
-      const float v0 = fmaf(s.pw[c0][2], x2, fmaf(s.pw[c0][1], x1, fmaf(s.pw[c0][0], x0, s.pw[c0][3])));
-      const float v1 = fmaf(s.pw[c1][2], x2, fmaf(s.pw[c1][1], x1, fmaf(s.pw[c1][0], x0, s.pw[c1][3])));
-      float sum = v0 + v1;
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
-      const float mean = sum * (1.0f / CB_DIM);
-      const float d0 = v0 - mean, d1 = v1 - mean;
-      float sq = d0 * d0 + d1 * d1;
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
-      const float rstd = rsqrtf(sq * (1.0f / CB_DIM) + 1e-5f);
-      s.n[tk][c0] = d0 * rstd * s.lnw[c0] + s.lnb[c0];
-      s.n[tk][c1] = d1 * rstd * s.lnw[c1] + s.lnb[c1];
-    }
-    __syncthreads();
-
-    // C. packed in_proj: thread `tid` owns output channel tid of [q|k|v]
-    for (int tk = 0; tk < CB_TOK; ++tk) {
-      // queries are only needed for the first nq bands (keys / values for all nine): the two q warps skip the rest
-      if (tid < CB_DIM && (tk % CB_BANDS) >= nq) continue;
-      if (FOLD) {
-        const int px = tk / CB_BANDS, band = tk % CB_BANDS;
-        const float x0 = s.in[px][band * 3], x1 = s.in[px][band * 3 + 1], x2 = s.in[px][band * 3 + 2];
-        const float lin = fmaf(wrow[2], x2, fmaf(wrow[1], x1, fmaf(wrow[0], x0, wrow[3])));
-        s.qkv[tk][tid] = fmaf(lin, s.rstd[tk], brow);
-        continue;
-      }
-      float acc = brow;
-      if constexpr (!FOLD) {
-        const float4* nrow = reinterpret_cast<const float4*>(&s.n[tk][0]);
-#pragma unroll
-        for (int c4 = 0; c4 < CB_DIM / 4; ++c4) {
-          const float4 v = nrow[c4];
-          acc = fmaf(v.x, wrow[4 * c4], acc);
-          acc = fmaf(v.y, wrow[4 * c4 + 1], acc);
-          acc = fmaf(v.z, wrow[4 * c4 + 2], acc);
-          acc = fmaf(v.w, wrow[4 * c4 + 3], acc);
-        }
-      }
-      s.qkv[tk][tid] = acc;
-    }
-    __syncthreads();
-
-    // D. softmax(q k^T / 4) v per (pixel, head, query band); context overwrites s.n
-    for (int it = tid; it < CB_PX * CB_HEADS * nq; it += CB_THREADS) {
-      const int qt = it % nq, h = (it / nq) % CB_HEADS, px = it / (nq * CB_HEADS);
-      const float* q = &s.qkv[px * CB_BANDS + qt][h * CB_HD];
-      float sc[CB_BANDS];
-      float mx = -INFINITY;
-#pragma unroll
-      for (int j = 0; j < CB_BANDS; ++j) {
-        const float* k = &s.qkv[px * CB_BANDS + j][CB_DIM + h * CB_HD];
-        float a = 0.f;
-#pragma unroll
-        for (int d = 0; d < CB_HD; ++d) a = fmaf(q[d], k[d], a);
-        sc[j] = a * 0.25f;
-        mx = fmaxf(mx, sc[j]);
-      }
-      float den = 0.f;
-#pragma unroll
-      for (int j = 0; j < CB_BANDS; ++j) {
-        sc[j] = expf(sc[j] - mx);
-        den += sc[j];
-      }
-      const float inv = 1.0f / den;
-      float ctx[CB_HD];
-#pragma unroll
-      for (int d = 0; d < CB_HD; ++d) ctx[d] = 0.f;
-#pragma unroll
-      for (int j = 0; j < CB_BANDS; ++j) {
-        const float* v = &s.qkv[px * CB_BANDS + j][2 * CB_DIM + h * CB_HD];
-        const float pj = sc[j] * inv;
-#pragma unroll
-        for (int d = 0; d < CB_HD; ++d) ctx[d] = fmaf(pj, v[d], ctx[d]);
-      }
-#pragma unroll
-      for (int d = 0; d < CB_HD; ++d) s.n[px * CB_BANDS + qt][h * CB_HD + d] = ctx[d];
-    }
-    __syncthreads();
-
-    // E. out_proj + residual with the (pre-LayerNorm) projected token; NHWC store
-    {
-      const int o = tid & 63, g = tid >> 6;
-      for (int ti = g; ti < CB_PX * nq; ti += 3) {
-        const int px = ti / nq, qt = ti % nq;
-        const int p = p0 + px;
-        const float* crow = &s.n[px * CB_BANDS + qt][0];
-        float acc = s.ob[o];
-#pragma unroll 16
-        for (int c = 0; c < CB_DIM; ++c) acc = fmaf(crow[c], s.wo[c][o], acc);
-        const float x0 = s.in[px][qt * 3], x1 = s.in[px][qt * 3 + 1], x2 = s.in[px][qt * 3 + 2];
-        const float res = fmaf(s.pw[o][2], x2, fmaf(s.pw[o][1], x1, fmaf(s.pw[o][0], x0, s.pw[o][3])));
-        if (p < HW) tok_out[(((long)b * nq + qt) * HW + p) * CB_DIM + o] = acc + res;
-      }
-    }
-    __syncthreads();
-  }
-}
-
-// ------------------------------------------------------------------------------------
-// Folded cross-band attention, register-blocked (replaces k_crossband_attn<true>: 0.87 ms per C3 image at ~15 % of the FMA
-// peak, bound by one shared-memory load per FMA in the attention and out_proj loops and by five block barriers per 8 pixels).
+// Register-blocked (a block-per-8-pixels version ran at 0.87 ms per C3 image, ~15 % of the FMA peak, bound by one
+// shared-memory load per FMA in the attention and out_proj loops and by five block barriers per 8 pixels).
 // A WARP owns 8 pixels per iteration and never meets a block barrier; lane = (pixel, head):
 //   * 1/std of the 9 tokens: each of a pixel's four lanes sums 16 of the 64 centred channels, two xor-shuffles combine them;
 //   * q, k, v are never stored: channel d of head h is  rstd * (M[d] . x + m0[d]) + n0[d]  (4 FMAs), computed where it is used,
 //     k / v once per pixel and head for all three query bands of a group;
 //   * softmax(q k^T / 4) v in registers, context -> a per-warp shared tile [24 tokens][64];
 //   * out_proj as a 6-token x 8-channel register tile per lane (48 FMAs per 14 vector loads), + bias + band_proj residual.
-// Summation orders of the scores (d = 0..15), the context (j = 0..8) and out_proj (c = 0..63) are those of the kernel above.
+// Scores sum over d = 0..15, the context over j = 0..8 and out_proj over c = 0..63, each in ascending order.
 // ------------------------------------------------------------------------------------
 namespace {
 constexpr int CB2_WARPS = 8, CB2_PX = 8, CB2_LD = 68;
@@ -410,45 +220,24 @@ __global__ void __launch_bounds__(CB2_WARPS * 32, 2) k_crossband_attn2(
 }
 
 extern "C" int ffsr_crossband_attention(const float* raw9, int B, int H, int W, const float* proj_w,
-                                        const float* proj_b, const float* ln_w, const float* ln_b,
-                                        const float* in_w, const float* in_b, const float* out_w,
-                                        const float* out_b, int nq, float* tok_out, int num_sms,
-                                        const float* fold, cudaStream_t stream) {
-  FFSR_REQUIRE(raw9 && proj_w && proj_b && ln_w && ln_b && in_w && in_b && out_w && out_b && tok_out, FFSR_ERR_ARG,
+                                        const float* proj_b, const float* out_w, const float* out_b, int nq,
+                                        float* tok_out, int num_sms, const float* fold, cudaStream_t stream) {
+  FFSR_REQUIRE(raw9 && proj_w && proj_b && out_w && out_b && tok_out && fold, FFSR_ERR_ARG,
                "crossband_attention: null pointer");
   FFSR_REQUIRE(B > 0 && H > 0 && W > 0 && nq >= 1 && nq <= CB_BANDS, FFSR_ERR_ARG, "crossband_attention: bad shape");
-  FFSR_REQUIRE(((uintptr_t)in_w % 16) == 0, FFSR_ERR_ALIGN, "crossband_attention: in_proj_weight must be 16B aligned");
+  FFSR_REQUIRE(((uintptr_t)fold % 16) == 0 && ((uintptr_t)tok_out % 16) == 0, FFSR_ERR_ALIGN, "crossband_attention: fold / tok_out must be 16B aligned");
   const int HW = H * W;
-  const int tiles = B * ((HW + CB_PX - 1) / CB_PX);
   static bool attr_set = false;
   if (!attr_set) {
-    cudaFuncSetAttribute(k_crossband_attn<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CBSmem));
-    cudaFuncSetAttribute(k_crossband_attn<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CBSmem));
+    cudaFuncSetAttribute(k_crossband_attn2<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CB2Smem));
+    cudaFuncSetAttribute(k_crossband_attn2<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CB2Smem));
     attr_set = true;
   }
-  const int grid = tiles < 2 * num_sms ? tiles : 2 * num_sms;
-  static const bool v1 = getenv("FFSR_CROSSBAND_V1") != nullptr;
-  if (fold && !v1) {
-    FFSR_REQUIRE(((uintptr_t)fold % 16) == 0 && ((uintptr_t)tok_out % 16) == 0, FFSR_ERR_ALIGN, "crossband_attention: fold / tok_out must be 16B aligned");
-    static bool attr2 = false;
-    if (!attr2) {
-      cudaFuncSetAttribute(k_crossband_attn2<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CB2Smem));
-      cudaFuncSetAttribute(k_crossband_attn2<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CB2Smem));
-      attr2 = true;
-    }
-    const long wtiles = (long)B * ((HW + CB2_PX - 1) / CB2_PX);
-    const long blocks = (wtiles + CB2_WARPS - 1) / CB2_WARPS;
-    const int grid2 = (int)(blocks < 2L * num_sms ? blocks : 2L * num_sms);
-    if (nq <= 3) k_crossband_attn2<1><<<grid2, CB2_WARPS * 32, sizeof(CB2Smem), stream>>>(fold, raw9, B, HW, proj_w, proj_b, out_w, out_b, nq, tok_out);
-    else k_crossband_attn2<3><<<grid2, CB2_WARPS * 32, sizeof(CB2Smem), stream>>>(fold, raw9, B, HW, proj_w, proj_b, out_w, out_b, nq, tok_out);
-  } else if (fold) {
-    FFSR_REQUIRE(((uintptr_t)fold % 16) == 0, FFSR_ERR_ALIGN, "crossband_attention: fold buffer must be 16B aligned");
-    k_crossband_attn<true><<<grid, CB_THREADS, sizeof(CBSmem), stream>>>(fold, raw9, B, HW, proj_w, proj_b, ln_w, ln_b, in_w,
-                                                                         in_b, out_w, out_b, nq, tok_out);
-  } else {
-    k_crossband_attn<false><<<grid, CB_THREADS, sizeof(CBSmem), stream>>>(nullptr, raw9, B, HW, proj_w, proj_b, ln_w, ln_b,
-                                                                          in_w, in_b, out_w, out_b, nq, tok_out);
-  }
+  const long wtiles = (long)B * ((HW + CB2_PX - 1) / CB2_PX);
+  const long blocks = (wtiles + CB2_WARPS - 1) / CB2_WARPS;
+  const int grid = (int)(blocks < 2L * num_sms ? blocks : 2L * num_sms);
+  if (nq <= 3) k_crossband_attn2<1><<<grid, CB2_WARPS * 32, sizeof(CB2Smem), stream>>>(fold, raw9, B, HW, proj_w, proj_b, out_w, out_b, nq, tok_out);
+  else k_crossband_attn2<3><<<grid, CB2_WARPS * 32, sizeof(CB2Smem), stream>>>(fold, raw9, B, HW, proj_w, proj_b, out_w, out_b, nq, tok_out);
   return ffsr_check_launch("crossband_attention");
 }
 

@@ -3,7 +3,6 @@
 // (src/models/multi_domain_frequency.py:146-196, 251-299, 352-385).
 // Output layout: raw9[B][9][3][H][W] fp32 (band-major planar), so raw9[:, i] is the
 // reference's i-th [B,3,H,W] band.  HBM-bound, tiny next to the HR phases.
-#include <stdlib.h>
 #include "common.cuh"
 
 // ------------------------------------------------------------------------------------
@@ -476,7 +475,7 @@ static void fft2_split(int N, int* n1, int* n2) {
   *n1 = best;
   *n2 = N / best;
 }
-static bool fft2_ok(int H, int W) { return H <= 2048 && W <= 2048 && getenv("FFSR_FFT_DENSE") == nullptr; }
+static bool fft2_ok(int H, int W) { return H <= 2048 && W <= 2048; }
 static size_t fft2_smem(int N) { return (size_t)(3 * FFT2_CW + 1) * N * sizeof(float2); }
 
 // low-pass of B*3 planes through the staged path; A: fp32 complex scratch [B*3][H][Wf]

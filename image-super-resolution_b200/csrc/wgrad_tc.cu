@@ -20,7 +20,6 @@
 //               into dw (deterministic, no atomics).
 //   warps     : 0 = TMA producer, 1 = MMA issuer (+ TMEM alloc), 2..5 = epilogue (TMEM lane quarters).
 #include <cuda.h>
-#include <stdlib.h>
 #include "common.cuh"
 #include "../../include/ffsr_b200.h"
 
@@ -447,7 +446,7 @@ struct WgPlan {
   int nblk, ci_blocks, co_blocks, cin_pad, cout_pad, P, tiles_x, tiles_y;
   long long total_tiles;
 };
-bool wg_single_copy(int H, int Cout, int ks) { return ks == 3 && Cout <= 32 && H >= 8 && getenv("FFSR_WGRAD_GEOM0") == nullptr; }
+bool wg_single_copy(int H, int Cout, int ks) { return ks == 3 && Cout <= 32 && H >= 8; }
 
 WgPlan wg_plan(int N, int H, int W, int Cin, int Cout, int ks) {
   WgPlan pl;

@@ -125,7 +125,6 @@ class DRCT(nn.Module):
         # the MLP hidden activations are bf16 rows padded to 8 channels and the Linears run on tcgen05; the residual stream
         # stays fp32.  Both modes are validated on B200 (tests/test_gpu_drct.py).
         self.precision = "fp32"
-        self.tail_tc = os.environ.get("FFSR_DRCT_TAIL_FP32") is None      # bf16 mode: reconstruction tail convs on tcgen05
         self.headpad_qkv = os.environ.get("FFSR_DRCT_QKV_PLAIN") is None   # bf16 mode, 16 x 16 windows: head-padded qkv rows
         self._packed: Optional[Tuple] = None
         self._ws: Dict[Tuple, torch.Tensor] = {}
@@ -272,16 +271,13 @@ class DRCT(nn.Module):
                 else:
                     qkv = self._buf("qkv", (B, H, W, pad(3 * d)), dev, adt)
                     conv(nhwc(n1), H, W, d, p + ".attn.qkv", 3 * d, 1, nhwc(qkv))
-                if headpad:
-                    pass
-                elif lp:
-                    call(lib.ffsr_window_attention_pitched, qkv.data_ptr(), pad(3 * d), B, H, W, d, sw.heads, ws, shift,
-                         w[p + ".attn.table"].data_ptr(), att.data_ptr(), pad(d), S)
-                else:
-                    call(lib.ffsr_window_attention, qkv.data_ptr(), B, H, W, d, sw.heads, ws, shift,
-                         w[p + ".attn.table"].data_ptr(), att.data_ptr(), K.DT_F32, S)
-                slim = lp and self.tail_tc                     # bf16 mode: the block's inner residual rows y1 / y2 as bf16 too
-                if slim:
+                    if lp:
+                        call(lib.ffsr_window_attention_pitched, qkv.data_ptr(), pad(3 * d), B, H, W, d, sw.heads, ws, shift,
+                             w[p + ".attn.table"].data_ptr(), att.data_ptr(), pad(d), S)
+                    else:
+                        call(lib.ffsr_window_attention, qkv.data_ptr(), B, H, W, d, sw.heads, ws, shift,
+                             w[p + ".attn.table"].data_ptr(), att.data_ptr(), K.DT_F32, S)
+                if lp:                                         # bf16 mode: the block's inner residual rows y1 / y2 as bf16 too
                     # Cout = d is 4 mod 8 for every DRCT-L width, which keeps these Linears off the 16-byte-store epilogue of
                     # k_conv_tc: their weights get four zero output rows (padded_out), the outputs land in the pad columns of the
                     # 8-channel-padded bf16 rows (never read: LayerNorm and the next Linear take d channels)
@@ -291,14 +287,14 @@ class DRCT(nn.Module):
                     y1 = self._buf("y1", (B, H, W, d), dev)
                     conv(nhwc(att), H, W, d, p + ".attn.proj", d, 1, nhwc(y1), r1=prefix(G))      # x + proj(attn)
                 n2 = n1
-                call(lib.ffsr_layernorm_strided, y1.data_ptr(), NP, d, pad(d) if slim else d, w[p + ".norm2.w"].data_ptr(),
-                     w[p + ".norm2.b"].data_ptr(), n2.data_ptr(), pad(d), ADT if slim else K.DT_F32, ADT, S)
+                call(lib.ffsr_layernorm_strided, y1.data_ptr(), NP, d, pad(d), w[p + ".norm2.w"].data_ptr(),
+                     w[p + ".norm2.b"].data_ptr(), n2.data_ptr(), pad(d), ADT, ADT, S)
                 hd = self._buf("hid", (B, H, W, pad(hid)), dev, adt)
                 conv(nhwc(n2), H, W, d, p + ".mlp.fc1", hid, 1, nhwc(hd), act=K.ACT_GELU)
                 # bf16 mode: y2 feeds only the adjust conv, so it is stored as bf16 rows (16-byte pitch) and that conv runs on tcgen05
                 # too (it was an fp32 CUDA-core GEMM: 16 of the 147 ms of a 352x512 forward)
-                y2 = self._buf("y2b", (B, H, W, pad(d)), dev, adt) if (lp and self.tail_tc) else (self._buf("y2", (B, H, W, d), dev) if lp else att)
-                if slim:
+                y2 = self._buf("y2b", (B, H, W, pad(d)), dev, adt) if lp else att
+                if lp:
                     conv(nhwc(hd), H, W, hid, padded_out(p + ".mlp.fc2", pad(d)), pad(d), 1, nhwc(y2), r1=nhwc(y1))
                 else:
                     conv(nhwc(hd), H, W, hid, p + ".mlp.fc2", d, 1, nhwc(y2), r1=nhwc(y1))         # + mlp
@@ -310,7 +306,7 @@ class DRCT(nn.Module):
                 else:                                          # x5 * 0.2 + x, in place on the first `embed_dim` channels
                     conv(nhwc(y2), H, W, d, a, E, 1, prefix(G), r1=prefix(G), sa=0.2)
 
-        if lp and self.tail_tc:
+        if lp:
             # bf16 mode: the reconstruction tail on tcgen05 as well.  Its six 3x3 convs ran as fp32 CUDA-core launches (16.6 of the
             # 147 ms of a 352x512 forward, the 64 -> 256 conv at 2x resolution alone 7.1 ms at 30 TFLOP/s).  The cached feature
             # (expert_loader hook) stays an fp32 tensor; x0 + conv_after_body(.) is a second launch of the same conv with the

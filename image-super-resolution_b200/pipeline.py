@@ -15,7 +15,6 @@ Phase map (reference file:line in include/ffsr_b200.h):
 from __future__ import annotations
 
 import ctypes as C
-import os
 from typing import Dict, List, Optional, Tuple
 
 import torch
@@ -181,16 +180,11 @@ class FusionEngine:
         # optional in-situ trace of EVERY launch: [(label, start_event, end_event), ...] (tools/trace_forward.py)
         self.trace = None
         self.overlap_routing = True    # phases 3 + 6 on a side stream, concurrent with phases 4 / 5
-        self.fold_crossband = True     # band_proj -> LayerNorm -> in_proj folded to 3+1 MACs per qkv channel
-        # bf16 mode: each edge refiner as ONE tile-resident kernel (csrc/edge_chain.cu) instead of six conv launches
-        self.edge_chain = os.environ.get("FFSR_EDGE_CHAIN0") is None
-        self.modulate_v2 = os.environ.get("FFSR_MODULATE_V1") is None   # 4 HR px x 4 experts per thread, bf16 features
-        self.p4_bf16_stream = os.environ.get("FFSR_P4_F32_STREAM") is None  # bf16 mode: Phase-4 residual stream stored as bf16
-        self.lka_tail_tc = os.environ.get("FFSR_LKA_TAIL_FFMA") is None     # fp32 LKA tail (Phase 3) on tcgen05, 3-term bf16 split
-        self.lka_tail128 = os.environ.get("FFSR_LKA_TAIL128_OFF") is None   # bf16 mode: Phase-4 LKA tail + modulation layer 0 fused
-        self.token_chain = os.environ.get("FFSR_TOKEN_CHAIN_OFF") is None   # bf16 mode: Phase-4 token pipeline as two tile-resident kernels
-        self.selector_fused = os.environ.get("FFSR_SELECTOR_LAYERS") is None   # Phase 6 as one tile-resident fp32 kernel
-        self.align_fused = os.environ.get("FFSR_ALIGN_LAYERS") is None   # bf16 mode: NCHW features -> aligned tokens in one kernel
+        # Tile-resident kernels in place of the layer-by-layer launches; tests turn them off to compare against the
+        # layer-by-layer path, which also serves fp32 mode and missing experts.
+        self.edge_chain = True       # bf16 mode: each edge refiner as ONE kernel (csrc/edge_chain.cu) instead of six conv launches
+        self.token_chain = True      # bf16 mode: Phase-4 token pipeline as two kernels (csrc/token_chain.cu)
+        self.selector_fused = True   # Phase 6 as one fp32 kernel (csrc/selector.cu)
         self._side: Dict[str, torch.cuda.Stream] = {}
 
     # ------------------------------------------------------------------ weights
@@ -253,7 +247,7 @@ class FusionEngine:
             cb = m.cross_band
             w["cb.proj_w"] = cb.band_proj.weight.detach().float().reshape(64, 3).contiguous()
             w["cb.out_w"] = cb.out_proj.weight.detach().float().reshape(3, 64).contiguous()
-            # band_proj -> LayerNorm -> in_proj folded in fp64 (see k_crossband_attn<FOLD>)
+            # band_proj -> LayerNorm -> in_proj folded in fp64 (see k_crossband_attn2)
             Wp = cb.band_proj.weight.detach().double().reshape(64, 3)
             bp = cb.band_proj.bias.detach().double()
             A_ = Wp - Wp.mean(dim=0, keepdim=True)
@@ -268,13 +262,6 @@ class FusionEngine:
             co = m.collaborative
             for n in EXPERT_ORDER:
                 conv("co.align." + n, co.align_layers[n])
-            cin_max = max(co.align_layers[n].weight.shape[1] for n in EXPERT_ORDER)
-            wa = torch.zeros(4, 1, cin_max, co.align_layers["drct"].weight.shape[0], device=dev)
-            for e, n in enumerate(EXPERT_ORDER):
-                pw_ = _pack_conv(co.align_layers[n].weight)
-                wa[e, :, :pw_.shape[1], :] = pw_
-            w["co.align.all"] = wa
-            w["co.align.all.b"] = torch.stack([co.align_layers[n].bias.detach().float() for n in EXPERT_ORDER]).contiguous()
             w["co.qkv"] = _pack_linear(co.cross_attn.in_proj_weight)
             w["co.qkv.b"] = co.cross_attn.in_proj_bias.detach().float().contiguous()
             w["co.out"] = _pack_linear(co.cross_attn.out_proj.weight)
@@ -292,7 +279,7 @@ class FusionEngine:
             w["co.m0b"] = torch.stack([co.modulation[i][0].bias.detach().float() for i in range(4)]).contiguous()
             lg = co.lka_global
             if lg.norm1.weight.shape[0] == 128 and all(tuple(co.modulation[i][0].weight.shape[:2]) == (32, 128) for i in range(4)):
-                # bf16 mode: LKA tail + modulation layer 0 as one tile-resident kernel (csrc/lka_tail.cu, k_lka_tail128)
+                # bf16 mode: LKA tail + modulation layer 0 as one tile-resident kernel (csrc/lka_tail.cu, k_lka_tail128w)
                 kb, db = self._bn_fold(lg.lka.bn)
                 k2, d2 = self._bn_fold(lg.norm2)
                 pw = lg.lka.pw_conv.weight.detach().float().reshape(128, 128) * kb[:, None]
@@ -450,7 +437,7 @@ class FusionEngine:
                    w[key + ".wv"].data_ptr(), t1.data_ptr(), t2.data_ptr(), a.data_ptr(),
                    K.DT_BF16 if lp else K.DT_F32, self._stream)
         self.launches += 2
-        if not lp and self.lka_tail_tc and (key + ".tail_w") in w and x.dtype == torch.float32:
+        if not lp and (key + ".tail_w") in w and x.dtype == torch.float32:
             x2 = self._buf(name + ".lka_x2f", x.shape, dev)
             self._call(self.lib.ffsr_lka_tail64, x.data_ptr(), a.data_ptr(), N * H * W, w[key + ".tail_w"].data_ptr(),
                        w[key + ".tail_p"].data_ptr(), self._P[blk + ".scale1"].data_ptr(), self._P[blk + ".scale2"].data_ptr(),
@@ -603,10 +590,8 @@ class FusionEngine:
         tok = self._buf("cb.tok", (B * nq, H, W, 64), dev)
         nsm = self._sm_count(dev)
         self._call(lib.ffsr_crossband_attention, raw9.data_ptr(), B, H, W, w["cb.proj_w"].data_ptr(),
-                   pp("cross_band.band_proj.bias"), pp("cross_band.norm.weight"), pp("cross_band.norm.bias"),
-                   pp("cross_band.band_attention.in_proj_weight"), pp("cross_band.band_attention.in_proj_bias"),
-                   pp("cross_band.band_attention.out_proj.weight"), pp("cross_band.band_attention.out_proj.bias"),
-                   nq, tok.data_ptr(), nsm, w["cb.fold"].data_ptr() if self.fold_crossband else None, S)
+                   pp("cross_band.band_proj.bias"), pp("cross_band.band_attention.out_proj.weight"),
+                   pp("cross_band.band_attention.out_proj.bias"), nq, tok.data_ptr(), nsm, w["cb.fold"].data_ptr(), S)
         x2 = self._lka_block("cb.lka", "cross_band.lka_block", tok, "cb%d" % nq)
         enh9 = self._buf("enh9", (B, 9, 3, H, W), dev, fresh=fr)
         routing = self._buf("routing", (B, 3, H, W), dev, fresh=fr)
@@ -668,26 +653,15 @@ class FusionEngine:
             # round trip of these [4][H][W][128] tensors, and the phase only feeds a sigmoid damped by 0.2
             cin_exp = {n: co.align_layers[n].weight.shape[1] for n in EXPERT_ORDER}
             fast_align = lp and len(have) == 4 and all(feats[n].shape[1] == cin_exp[n] for n in EXPERT_ORDER)
-            rdt = torch.bfloat16 if (fast_align and self.p4_bf16_stream) else f32
+            rdt = torch.bfloat16 if fast_align else f32
             tokens = self._buf("co.tok", (B, 4, Hq, Wq, 128), dev, dtype=rdt, zero=True)
-            if fast_align and self.align_fused and rdt == torch.bfloat16 and "co.align_w" in w:
+            if fast_align and "co.align_w" in w:
                 # NCHW fp32 features -> aligned bf16 tokens in one tile-resident kernel (csrc/token_chain.cu, k_align_tokens)
                 fl = [feats[n].detach().to(f32).contiguous() for n in EXPERT_ORDER]
                 fptr = (C.c_void_p * 4)(*[t.data_ptr() for t in fl])
                 cnum = (C.c_int * 4)(*[cin_exp[n] for n in EXPERT_ORDER])
                 self._call(lib.ffsr_align_tokens, fptr, cnum, B, Hq * Wq, w["co.align_w"].data_ptr(), w["co.align_b"].data_ptr(),
                            tokens.data_ptr(), S)
-            elif fast_align:
-                # bf16 mode: NCHW fp32 features -> one bf16 channels-last buffer, then ONE grouped tcgen05 1x1 conv
-                cmax = max(cin_exp.values())
-                cs = (cmax + 7) // 8 * 8
-                fbuf = self._buf("co.feat", (B, 4, Hq, Wq, cs), dev, dtype=torch.bfloat16, zero=True)
-                for e, n in enumerate(EXPERT_ORDER):
-                    f = feats[n].detach().to(f32).contiguous()
-                    self._call(lib.ffsr_nchw_to_nhwc_bf16, f.data_ptr(), B, cin_exp[n], Hq * Wq,
-                               fbuf.data_ptr() + e * Hq * Wq * cs * 2, 4 * Hq * Wq * cs, cs, S)
-                self.conv(nhwc(fbuf.view(B * 4, Hq, Wq, cs)), B * 4, Hq, Wq, cmax, "co.align.all", 128, 1,
-                          nhwc(tokens.view(B * 4, Hq, Wq, 128)), groups=4)
             else:
                 if len(have) < 4:
                     tokens.zero_()                              # missing expert -> zero token (:378-381)
@@ -737,8 +711,8 @@ class FusionEngine:
                 hdn = self._buf("co.h", (N4, Hq, Wq, 256), dev, dtype=adt)
                 self.conv(nhwc(n1), N4, Hq, Wq, 128, "co.f0", 256, 1, nhwc(hdn), act=K.ACT_GELU)
                 self.conv(nhwc(hdn), N4, Hq, Wq, 256, "co.f2", 128, 1, nhwc(t2), epi=K.EPI_RESIDUAL, r1=nhwc(t1))
-            m32 = self._buf("co.m32", (N4, Hq, Wq, 32), dev, dtype=adt if (self.modulate_v2 and (Hq, Wq) == (H, W)) else f32)
-            if lp and self.lka_tail128 and "co.tail_w" in w and t2.dtype == torch.bfloat16 and m32.dtype == torch.bfloat16:
+            m32 = self._buf("co.m32", (N4, Hq, Wq, 32), dev, dtype=adt if (Hq, Wq) == (H, W) else f32)
+            if lp and "co.tail_w" in w and t2.dtype == torch.bfloat16 and m32.dtype == torch.bfloat16:
                 # depthwise chain, then ONE tile-resident kernel: pw + gate, ffn0 + GELU, ffn2 + residual, modulation layer 0
                 ta = self._buf("co.lka_t1", t2.shape, dev)
                 tb = self._buf("co.lka_t2", t2.shape, dev)
@@ -763,14 +737,13 @@ class FusionEngine:
         if m32 is not None and tuple(m32.shape[1:3]) != (H, W):
             self._call(lib.ffsr_modulate_hr_sized, ptrs, m32.data_ptr(), m32.shape[1], m32.shape[2], w["co.m2"].data_ptr(),
                        w["co.m2b"].data_ptr(), B, H, W, 0 if m.training else 1, ecol.data_ptr(), cat3.data_ptr() + 64 * esz, 80, ADT, S)
-        elif m32 is not None and self.modulate_v2:
+        elif m32 is not None:
             self._call(lib.ffsr_modulate_hr_v2, ptrs, m32.data_ptr(), K.DT_BF16 if m32.dtype == torch.bfloat16 else K.DT_F32,
                        w["co.m2"].data_ptr(), w["co.m2b"].data_ptr(), B, H, W, 0 if m.training else 1, ecol.data_ptr(),
                        cat3.data_ptr() + 64 * esz, 80, ADT, S)
         else:
-            self._call(lib.ffsr_modulate_hr, ptrs, m32.data_ptr() if m32 is not None else None,
-                       w["co.m2"].data_ptr(), w["co.m2b"].data_ptr(), B, H, W, 0 if m.training else 1, ecol.data_ptr(),
-                       cat3.data_ptr() + 64 * esz, 80, ADT, S)
+            self._call(lib.ffsr_modulate_hr, ptrs, None, w["co.m2"].data_ptr(), w["co.m2b"].data_ptr(), B, H, W,
+                       0 if m.training else 1, ecol.data_ptr(), cat3.data_ptr() + 64 * esz, 80, ADT, S)
         self._call(lib.ffsr_expert_downsample, ecol.data_ptr(), B, Hh, Wh, cat2.data_ptr() + 64 * esz, 80,
                    s1in.data_ptr(), 16, ADT, S)
 

@@ -32,7 +32,6 @@ from __future__ import annotations
 
 import contextlib
 import ctypes as C
-import os
 from typing import Dict, List, Optional
 
 import torch
@@ -46,10 +45,6 @@ CL = torch.channels_last
 
 def _lib():
     return K.load()
-
-
-# tcgen05 launches of the training graph may use several MMA-issuing warps too (FFSR_TRAIN_SINGLE_ISSUE=1: single issuer)
-_CONV_FLAGS = 0 if os.environ.get("FFSR_TRAIN_SINGLE_ISSUE") else K.CONV_MULTI_ISSUE
 
 
 def _S(t: torch.Tensor):
@@ -129,7 +124,7 @@ def _launch_conv(x: torch.Tensor, wp: torch.Tensor, bias: Optional[torch.Tensor]
     p.out = out.data_ptr()
     p.out_sN, p.out_sY, p.out_sX = H * W * Cout, W * Cout, Cout
     p.act, p.epi = K.ACT_NONE, K.EPI_PLAIN
-    p.flags = _CONV_FLAGS
+    p.flags = K.CONV_MULTI_ISSUE
     p.sa = p.sb = 1.0
     p.in_dtype = p.out_dtype = p.w_dtype = K.DT_F32
     _ck(_lib().ffsr_conv2d(C.byref(p), _S(x)), "conv2d")
@@ -237,7 +232,7 @@ def _launch_conv_tc(xb: torch.Tensor, Cin: int, wtc: torch.Tensor, bias, out: to
     p.out = out.data_ptr()
     p.out_sN, p.out_sY, p.out_sX = out.stride(0), out.stride(2), out.stride(3)      # dense or padded-pitch channels-last
     p.act, p.epi = act, K.EPI_PLAIN
-    p.flags = _CONV_FLAGS
+    p.flags = K.CONV_MULTI_ISSUE    # tcgen05 launches: up to three MMA-issuing warps, as at inference
     p.sa = p.sb = 1.0
     p.in_dtype, p.w_dtype = K.DT_BF16, K.DT_BF16
     p.out_dtype = _dt(out)

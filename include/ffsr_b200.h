@@ -82,11 +82,11 @@ int ffsr_fft_bands(const float* lr, int B, int H, int W, const float* logits, in
 /* ---- Phase 3: cross-band attention -------------------------------------------------------
  * EnhancedCrossBandWithLKA.forward steps 1-2  src/models/large_kernel_attention.py:219-233
  * tok_out[B][nq][H][W][64]: attention output (+residual) of the first nq bands.
- * fold (optional, 16B aligned, [64x4 | 192x4 | 192] floats): band_proj -> LayerNorm -> in_proj collapsed on the host
+ * fold (required, 16B aligned, [64x4 | 192x4 | 192] floats): band_proj -> LayerNorm -> in_proj collapsed on the host
  * (a token is an affine function of 3 band values): A|c = centred band_proj rows / bias, M|m0 = W_in diag(gamma) [A|c],
- * n0 = W_in beta + b_in; qkv = rstd * (M x + m0) + n0 -- 16x fewer FLOPs, same result up to fp32 rounding. */
+ * n0 = W_in beta + b_in; qkv = rstd * (M x + m0) + n0 -- 16x fewer FLOPs, same result up to fp32 rounding.
+ * tok_out must be 16B aligned. */
 int ffsr_crossband_attention(const float* raw9, int B, int H, int W, const float* proj_w, const float* proj_b,
-                             const float* ln_w, const float* ln_b, const float* in_w, const float* in_b,
                              const float* out_w, const float* out_b, int nq, float* tok_out, int num_sms,
                              const float* fold, cudaStream_t stream);
 /* out_proj + band residual (:240-241) and routing_lr = bands 0+1+2 (enhanced_fusion_v2.py:713) */

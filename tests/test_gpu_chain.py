@@ -37,7 +37,7 @@ def test_edge_refiner_chain_matches_layer_by_layer(B, H, W):
     with torch.no_grad():
         m.forward_with_precomputed(lr, imgs, fts)
         eng = m._engine
-        assert eng.edge_chain, "FFSR_EDGE_CHAIN0 is set: nothing to compare"
+        assert eng.edge_chain, "the edge-chain kernel must be the default path"
         sr_chain = m.forward_with_precomputed(lr, imgs, fts).float().cpu()
         cat_chain = eng.workspace("ee.cat96").float().cpu().clone()
         eng.edge_chain = False
@@ -154,7 +154,7 @@ def test_fused_selector_matches_layer_by_layer(B, H, W):
     with torch.no_grad():
         m.forward_with_precomputed(lr, imgs, fts)
         eng = m._engine
-        assert eng.selector_fused, "FFSR_SELECTOR_LAYERS is set: nothing to compare"
+        assert eng.selector_fused, "the fused selector kernel must be the default path"
         run = lambda: m._run_pipeline(lr, [imgs[k] for k in O.EXPERT_ORDER], fts, 4 * H, 4 * W, {}, True)[1]
         a = run()
         a = {k: a[k].clone() for k in ("gates", "difficulty", "gate_logits", "active")}

@@ -122,3 +122,35 @@ def test_conv_tc_lean_epilogue_many_tiles():
     # enough tiles per CTA (>= 8 x #SMs) for the tile-ownership heuristic to switch on by itself
     _run(32, 32, 3, 1, 400, 416, K.ACT_GELU, K.EPI_PLAIN, True)
     _run(64, 32, 3, 1, 400, 416, K.ACT_NONE, K.EPI_RESIDUAL, True, r_bf16=True)
+
+
+# ---- several MMA-issuing warps: which warp issues a tile's MMAs must not change its accumulation order or its bits
+@pytest.mark.parametrize("H,W", [(96, 96), (256, 256)])
+@pytest.mark.parametrize("cin,cout,ks,act,out_bf16", [
+    (32, 32, 3, K.ACT_GELU, True), (64, 64, 3, K.ACT_GELU, True), (76, 64, 3, K.ACT_GELU, True), (3, 32, 3, K.ACT_GELU, True),
+    (32, 8, 1, K.ACT_GELU, True), (8, 1, 3, K.ACT_SIGMOID, False), (16, 3, 3, K.ACT_SIGMOID, False),
+    (128, 3, 3, K.ACT_NONE, False), (3, 128, 3, K.ACT_GELU, True), (128, 128, 1, K.ACT_NONE, False),
+    (96, 32, 3, K.ACT_GELU, True), (32, 32, 3, K.ACT_NONE, False),
+])
+def test_conv_tc_issue_warps_leave_bits_unchanged(monkeypatch, H, W, cin, cout, ks, act, out_bf16):
+    if not torch.cuda.is_available():
+        pytest.skip("needs a CUDA device")
+    dev = torch.device("cuda:0")
+    g = torch.Generator().manual_seed(cin + cout)
+    x = torch.randn(1, H, W, (cin + 7) // 8 * 8, generator=g).to(dev).bfloat16()
+    wt = torch.randn(cout, cin, ks, ks, generator=g) / (cin * ks * ks) ** 0.5
+    eng = FusionEngine(isr_b200.CompleteEnhancedFusionSR(None))
+    eng._stream = eng._get_stream(dev)
+    eng._w = {"t": _pack_conv(wt).to(dev), "t.b": torch.randn(cout, generator=g).to(dev)}
+
+    def launch():
+        out = torch.zeros(1, H, W, (cout + 7) // 8 * 8, device=dev, dtype=torch.bfloat16 if out_bf16 else torch.float32)
+        with torch.cuda.device(dev):
+            eng.conv(nhwc(x), 1, H, W, cin, "t", cout, ks, nhwc(out), act=act)
+            torch.cuda.synchronize()
+        return out.cpu()
+
+    multi = launch()
+    monkeypatch.setattr(K, "CONV_MULTI_ISSUE", 0)                  # one issuing warp
+    single = launch()
+    assert torch.equal(multi, single), f"{int((multi != single).sum())} values differ"

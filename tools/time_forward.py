@@ -1,7 +1,6 @@
 """Wall-clock-free timing of the C3 fusion forward in its launch modes (CUDA events, inputs resident):
 eager launches with / without the routing side stream, CUDA-graph replay, and host time per eager forward.
     python tools/time_forward.py [--lr 339 510] [--steps 10] [--precision bf16]
-Environment toggles read per launch by the library (e.g. FFSR_TC_LEAN0=1) can be compared with --env NAME.
 """
 import argparse
 import os
@@ -18,7 +17,6 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--lr", type=int, nargs=2, default=[339, 510])
 ap.add_argument("--steps", type=int, default=10)
 ap.add_argument("--precision", default="bf16")
-ap.add_argument("--env", action="append", default=[], help="also time eager forwards with this variable set to 1")
 a = ap.parse_args()
 dev = torch.device("cuda:0")
 torch.manual_seed(0)
@@ -59,8 +57,3 @@ with torch.cuda.graph(g):
     out = fwd()
 ms, host = timed(g.replay)
 print(f"CUDA graph, single stream  : {ms:7.3f} ms / forward  (host enqueue time {host:.3f} ms)")
-for name in a.env:
-    os.environ[name] = "1"
-    ms, host = timed(fwd)
-    print(f"eager, single stream, {name}=1 : {ms:7.3f} ms / forward")
-    del os.environ[name]
