@@ -496,6 +496,53 @@ def augment_code(seed: int, epoch: int, position: int) -> int:
     return dihedral_code(hflip, vflip, rng.randint(0, 3))
 
 
+def epoch_schedule(total: int, batch_size: int, shuffle: bool, seed: int, epoch: int, rank: int = 0, world: int = 1,
+                   drop_last: bool = True, world_invariant: bool = False, augment: bool = True,
+                   rng: Optional[random.Random] = None, start: int = 0):
+    """``DeviceBatchLoader``'s host plan of one epoch from batch ``start`` on: yields (sample indices, dihedral codes,
+    state of ``rng`` after the batch's draws or None).  World-invariant codes come from ``augment_code`` by position;
+    default codes are the reference's three draws per sample from ``rng``, in batch order.  The batches before
+    ``start`` are skipped without a draw: resuming restores the ``rng`` state those draws left."""
+    if world_invariant:
+        plan = world_invariant_batches(total, batch_size, shuffle, seed, epoch, rank, world, drop_last)
+    else:
+        plan = [(None, b) for b in epoch_batches(total, batch_size, shuffle, seed, epoch, rank, world, drop_last)]
+    for pos, idxs in plan[start:]:
+        codes = [0] * len(idxs)
+        if augment and pos is not None:
+            codes = [augment_code(seed, epoch, p) for p in pos]
+        elif augment:
+            for j in range(len(idxs)):
+                hflip = rng.random() < 0.5
+                vflip = rng.random() < 0.5
+                codes[j] = dihedral_code(hflip, vflip, rng.randint(0, 3))
+        yield idxs, codes, (rng.getstate() if augment and pos is None else None)
+
+
+_LOADER_KEYS = ("samples", "seed", "shuffle", "drop_last", "augment", "world_invariant")
+
+
+def check_loader_resume(saved: dict, now: dict) -> None:
+    """Raise ``ValueError`` naming the field when a ``DeviceBatchLoader.state_dict()`` ``saved`` cannot continue in a
+    loader configured as ``now`` (the same keys).  World-invariant mode resumes on another world size when
+    world * batch_size is unchanged: a position keeps its step and augmentation.  The default mode keeps its world
+    size and batch size, except that the world size may change at an epoch boundary (batch 0)."""
+    for k in _LOADER_KEYS:
+        if saved[k] != now[k]:
+            raise ValueError(f"loader state: {k} is {saved[k]!r} in the checkpoint, {now[k]!r} here")
+    if now["world_invariant"]:
+        if saved["world"] * saved["B"] != now["world"] * now["B"]:
+            raise ValueError(f"loader state: world * batch_size is {saved['world']} * {saved['B']} in the checkpoint, "
+                             f"{now['world']} * {now['B']} here; a world-invariant resume keeps the product")
+        return
+    if saved["B"] != now["B"]:
+        raise ValueError(f"loader state: batch_size is {saved['B']} in the checkpoint, {now['B']} here")
+    if saved["world"] != now["world"] and saved["batch"] != 0:
+        raise ValueError(f"loader state: world is {saved['world']} in the checkpoint, {now['world']} here, and the "
+                         f"checkpoint is mid-epoch (batch {saved['batch']}): the default mode's batches depend on the "
+                         "world size, so it changes only at an epoch boundary")
+
+
 def batches_per_epoch(total: int, batch_size: int, world: int = 1, drop_last: bool = True) -> int:
     """len(epoch_batches(...)) without building them (identical on every rank)."""
     if world > 1:
@@ -522,7 +569,13 @@ class DeviceBatchLoader:
     [t*world*B + r*B, t*world*B + (r+1)*B) of the shared permutation, and each sample's augmentation is drawn from a
     generator keyed by (seed, epoch, position) (``world_invariant_batches``, ``augment_code``).  For a fixed world*B,
     every micro-batch of a step then gets the same samples and flips for any world size: the loader of
-    ``FusionTrainer(world_invariant=True)``.  ``rng`` is not used in this mode."""
+    ``FusionTrainer(world_invariant=True)``.  ``rng`` is not used in this mode.
+
+    ``state_dict()`` / ``load_state_dict()``: the epoch and the index of the next batch the consumer has not received
+    yet, the ``rng`` state those batches' draws leave (default mode), and the settings the batch plan depends on.  A
+    loaded loader's next iteration yields exactly the remaining batches of that epoch -- same samples, dihedral codes
+    and tensor bits, skipped batches never read -- then continues into the next epochs.  A world-invariant state
+    resumes on another world size when world * batch_size is unchanged (``check_loader_resume``)."""
 
     def __init__(self, shard: str, batch_size: int, device, augment: bool = True, shuffle: bool = True,
                  drop_last: bool = True, load_features: bool = True, repeat_factor: int = 1, rank: int = 0, world: int = 1,
@@ -551,6 +604,8 @@ class DeviceBatchLoader:
         # allocator wait for blocks still in use by the training step (measured: +35 ms per step).
         self.reuse_buffers = bool(reuse_buffers)
         self.epoch = 0
+        self._start = 0                                       # first batch of the next iteration (load_state_dict)
+        self._cursor = None                                   # (epoch, next batch, rng state) of the consumer
         self.copy_threads = max(1, int(copy_threads))
         self._codes_bytes = _round_up(4 * self.B, _ALIGN_REC)
         self._slots = None
@@ -566,7 +621,11 @@ class DeviceBatchLoader:
         return batches_per_epoch(total, self.B, self.world, self.drop_last)
 
     def set_epoch(self, epoch: int) -> None:
+        """The epoch the next iteration runs.  Setting the epoch a loaded state resumes keeps its batch position."""
+        if int(epoch) != self.epoch:
+            self._start = 0
         self.epoch = int(epoch)
+        self._cursor = None
 
     # ---- one batch --------------------------------------------------------------------------------
     def _slot(self, k: int, rbytes: int):
@@ -577,7 +636,7 @@ class DeviceBatchLoader:
                             "outs": {}} for _ in range(self.depth + 1)]
         return self._slots[k % len(self._slots)]
 
-    def _produce(self, k: int, idxs: List[int], positions: Optional[List[int]] = None, epoch: int = 0) -> dict:
+    def _produce(self, k: int, idxs: List[int], batch_codes: List[int]) -> dict:
         K, cache = self.K, self.cache
         n = len(idxs)
         recs = [i % cache.count for i in idxs]
@@ -587,15 +646,7 @@ class DeviceBatchLoader:
             slot["ev"].synchronize()                          # the H2D that last used this staging buffer has finished
         host = slot["host"].numpy()
         codes = np.zeros(self.B, dtype=np.int32)
-        if self.augment and positions is not None:
-            for j in range(n):
-                codes[j] = augment_code(self.seed, epoch, positions[j])
-        elif self.augment:
-            for j in range(n):
-                hflip = self.rng.random() < 0.5
-                vflip = self.rng.random() < 0.5
-                rot_k = self.rng.randint(0, 3)
-                codes[j] = dihedral_code(hflip, vflip, rot_k)
+        codes[:n] = batch_codes
         host[:4 * self.B] = codes.view(np.uint8)
         base = self._codes_bytes
 
@@ -661,35 +712,57 @@ class DeviceBatchLoader:
         out["_event"], out["_tensors"], out["_slot"] = ev, tensors, slot
         return out
 
-    def _batches(self) -> List[Tuple[Optional[List[int]], List[int]]]:
-        """(positions or None, sample indices) per batch of the current epoch."""
-        total = self.cache.count * self.repeat_factor
-        if self.world_invariant:
-            return world_invariant_batches(total, self.B, self.shuffle, self.seed, self.epoch, self.rank, self.world,
-                                           self.drop_last)
-        return [(None, b) for b in epoch_batches(total, self.B, self.shuffle, self.seed, self.epoch, self.rank,
-                                                 self.world, self.drop_last)]
+    # ---- resuming ---------------------------------------------------------------------------------
+    def _resume_config(self) -> dict:
+        return {"samples": self.cache.count * self.repeat_factor, "seed": self.seed, "shuffle": bool(self.shuffle),
+                "drop_last": bool(self.drop_last), "augment": bool(self.augment),
+                "world_invariant": self.world_invariant, "B": self.B, "world": self.world}
+
+    def state_dict(self) -> dict:
+        """Position of the consumer: the epoch and index of the next batch it has not received (a state taken after an
+        epoch's last batch is batch 0 of the next epoch), the ``rng`` state (default mode) and the plan's settings.
+        The producer thread runs ahead; what it drew for batches not yet handed out is not part of the state."""
+        epoch, nxt, rng = self._cursor if self._cursor is not None else (self.epoch, self._start, None)
+        if nxt >= len(self):
+            epoch, nxt = epoch + 1, 0
+        if rng is None and not self.world_invariant:
+            rng = self.rng.getstate()
+        return dict(self._resume_config(), epoch=int(epoch), batch=int(nxt), rng=rng)
+
+    def load_state_dict(self, state: dict) -> None:
+        """Continue from ``state``: the next iteration yields the remaining batches of its epoch.  Raises ValueError
+        (``check_loader_resume``) when this loader's settings cannot continue it."""
+        check_loader_resume(state, self._resume_config())
+        self.epoch, self._start, self._cursor = int(state["epoch"]), int(state["batch"]), None
+        if not self.world_invariant and state["world"] == self.world and state["rng"] is not None:
+            self.rng.setstate(state["rng"])
 
     def __iter__(self) -> Iterator[dict]:
-        batches = self._batches()
-        epoch = self.epoch
+        epoch, start = self.epoch, self._start
         self.epoch += 1
+        self._start = 0
+        self._cursor = (epoch, start, None if self.world_invariant else self.rng.getstate())
+        sched = epoch_schedule(self.cache.count * self.repeat_factor, self.B, self.shuffle, self.seed, epoch, self.rank,
+                               self.world, self.drop_last, self.world_invariant, self.augment, self.rng, start)
         q: "queue.Queue" = queue.Queue(maxsize=self.depth - 1)
         stop = threading.Event()
 
         def worker():
             try:
                 with torch.cuda.device(self.device):
-                    for k, (pos, idxs) in enumerate(batches):
+                    for k, (idxs, codes, rng_after) in enumerate(sched):
                         if stop.is_set():
                             return
-                        q.put(self._produce(k, idxs, pos, epoch))
+                        item = self._produce(k, idxs, codes)
+                        item["_rng"] = rng_after
+                        q.put(item)
                 q.put(None)
             except BaseException as exc:                      # surface loader errors in the consumer
                 q.put(exc)
 
         th = threading.Thread(target=worker, daemon=True)
         th.start()
+        nxt = start
         try:
             while True:
                 item = q.get()
@@ -702,6 +775,9 @@ class DeviceBatchLoader:
                 for t in item.pop("_tensors"):
                     t.record_stream(cur)
                 slot = item.pop("_slot")
+                nxt += 1
+                rng_after = item.pop("_rng")
+                self._cursor = (epoch, nxt, rng_after if rng_after is not None else self._cursor[2])
                 yield item
                 if self.reuse_buffers:                         # the consumer is done enqueueing work on this batch
                     done = torch.cuda.Event()

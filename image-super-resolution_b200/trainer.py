@@ -26,6 +26,8 @@ is re-pointed into the flat bucket.
 from __future__ import annotations
 
 import ctypes as C
+import os
+import uuid
 from typing import Dict, Iterable, List, Optional
 
 import torch
@@ -323,7 +325,13 @@ class FusionTrainer:
     ``accumulation_steps=k``: ``step()`` takes the rank's k*b patches and runs them as k contiguous micro-batches along
     dim 0; the returned loss and components are their mean.  ``world_invariant=True`` (module docstring): the same
     results for every world size N dividing M = N*k; ``global_micro_batches=M`` instead of k sets M directly and
-    raises ``ValueError`` when N does not divide it."""
+    raises ``ValueError`` when N does not divide it.
+
+    Resuming: ``state_dict()`` / ``load_state_dict()`` (and ``save_checkpoint`` / ``load_checkpoint`` with the
+    loader's state) continue a run bit for bit -- in the default mode on the same world size, in world-invariant mode on
+    any N dividing M.  Each capture records the host dropout seeds it freezes; a trainer loaded from a checkpoint
+    taken after a capture runs its warm-up steps and its own capture on those seeds, so with the restored device
+    counter they compute what the interrupted run's replays would."""
 
     def __init__(self, model, criterion, lr: float = 2e-4, betas=(0.9, 0.999), eps: float = 1e-8,
                  weight_decay: float = 1e-4, max_grad_norm: float = 1.0, ema_decay: Optional[float] = 0.999,
@@ -371,6 +379,9 @@ class FusionTrainer:
         self._graph = None
         self._static = None
         self._sig = None
+        # host dropout seeds of the current capture, in call order (recorded by it, or loaded with a checkpoint taken
+        # after one): a step that uses them plus the device counter gives the bits of that capture's replay
+        self._capture_seeds: Optional[List[int]] = None
 
     def _split(self, lr_img, expert_imgs, expert_feats, hr_img):
         """The rank's batch as accumulation_steps contiguous micro-batches along dim 0."""
@@ -502,13 +513,24 @@ class FusionTrainer:
                 self.accumulation_steps)
 
     def _capture(self, lr_img, expert_imgs, expert_feats, hr_img):
+        from .training import seed_tape
         self._static = (lr_img.clone(), {k: v.clone() for k, v in expert_imgs.items()},
                         {k: v.clone() for k, v in expert_feats.items()} if expert_feats else None, hr_img.clone())
         self._graph = torch.cuda.CUDAGraph()
         torch.cuda.synchronize()
-        with torch.cuda.graph(self._graph):
-            self._out = self._step_body(*self._static)
+        with seed_tape(self._capture_seeds) as tape:          # records the seeds it freezes (replays loaded ones)
+            with torch.cuda.graph(self._graph):
+                self._out = self._step_body(*self._static)
+        self._capture_seeds = tape.seeds
         self._sig = self._signature(lr_img, expert_imgs, expert_feats, hr_img)
+
+    def _eager_step(self, lr_img, expert_imgs, expert_feats, hr_img):
+        """An executed step outside a graph.  After loading a checkpoint taken after a capture it takes that capture's
+        seeds instead of drawing: with the restored counter it computes what the interrupted run's replay would."""
+        import contextlib
+        from .training import seed_tape
+        with seed_tape(self._capture_seeds) if self._capture_seeds is not None else contextlib.nullcontext():
+            return self._step_body(lr_img, expert_imgs, expert_feats, hr_img)
 
     def step(self, lr_img, expert_imgs, expert_feats, hr_img):
         """forward -> clamp -> loss -> backward -> all-reduce -> clip + AdamW + EMA.  Returns the
@@ -516,14 +538,16 @@ class FusionTrainer:
         self.model.train()
         opt = self.optimizer
         if not self.cuda_graph:
-            return self._step_body(lr_img, expert_imgs, expert_feats, hr_img)
+            if self._capture_seeds is not None and self._signature(lr_img, expert_imgs, expert_feats, hr_img) != self._sig:
+                self._capture_seeds = None
+            return self._eager_step(lr_img, expert_imgs, expert_feats, hr_img)
         sig = self._signature(lr_img, expert_imgs, expert_feats, hr_img)
-        if self._graph is not None and sig != self._sig:
-            self._graph, self._static, self._eager_steps = None, None, 0       # new shapes: warm up and re-capture
+        if self._capture_seeds is not None and sig != self._sig:      # new shapes: warm up and re-capture
+            self._graph, self._static, self._eager_steps, self._capture_seeds = None, None, 0, None
         if self._graph is None:
             if self._eager_steps < self.graph_warmup:
                 self._eager_steps += 1
-                return self._step_body(lr_img, expert_imgs, expert_feats, hr_img)
+                return self._eager_step(lr_img, expert_imgs, expert_feats, hr_img)
             self._capture(lr_img, expert_imgs, expert_feats, hr_img)     # capture does not execute the step
         lr_now = float(opt.param_groups[0]["lr"])
         if lr_now != opt._lr_host:
@@ -540,6 +564,77 @@ class FusionTrainer:
         opt.steps += 1
         opt.bump_versions()
         return self._out
+
+    # ---- checkpointing ----------------------------------------------------------------------------
+    def _resume_config(self) -> dict:
+        o = self.optimizer
+        return {"bucket": (int(o.bucket.numel), [int(x) for x in o.bucket.offsets]),
+                "precision": getattr(self.model, "precision", None), "world_invariant": self.world_invariant,
+                "accumulation_steps": self.accumulation_steps, "world": _world(),
+                "micro_batches": _world() * self.accumulation_steps}
+
+    def state_dict(self) -> dict:
+        """Everything the next steps depend on: the model's parameters and buffers (BatchNorm statistics and
+        ``num_batches_tracked``), ``optimizer.state_dict()``, the dropout state (device counter, world-invariant seed
+        base, the seeds of the current capture, torch's CPU generator), the eager-step count and capture signature,
+        the criterion's weights and the configuration a resume is checked against."""
+        from .training import seed_counter
+        crit = self.criterion
+        captured = self._capture_seeds is not None
+        return {"model": {k: v.detach().clone() for k, v in self.model.state_dict().items()},
+                "optimizer": self.optimizer.state_dict(),
+                "seed_counter": int(seed_counter(self.optimizer.bucket.flat.device).item()),
+                "seed_base": self._seed_base,
+                "eager_steps": int(self._eager_steps),
+                "capture_seeds": list(self._capture_seeds) if captured else None,
+                "signature": self._sig if captured else None,
+                "cpu_rng": torch.get_rng_state(),
+                "criterion": {"weights": dict(getattr(crit, "weights", {})), "use_swt": getattr(crit, "use_swt", None),
+                              "use_fft": getattr(crit, "use_fft", None)},
+                "config": self._resume_config()}
+
+    @torch.no_grad()
+    def load_state_dict(self, state: dict, at_epoch_boundary: bool = False) -> None:
+        """Continue the run ``state`` was taken from: the next steps give the bits the uninterrupted run's would (same
+        build, GPU model, inputs and step sequence).  Drops any captured graph; a checkpoint taken after a capture
+        warms up and re-captures on that capture's seeds, one taken during warm-up finishes the remaining warm-up steps
+        from the restored CPU generator.  Restores torch's CPU generator state.  With a process group every rank ends
+        with rank 0's state.  Raises ``ValueError`` naming the field when this trainer cannot continue it
+        (``check_resume``); ``at_epoch_boundary`` allows a default-mode resume on another world size (not bitwise)."""
+        from .training import seed_counter
+        check_resume(state["config"], self._resume_config(), at_epoch_boundary)
+        world = _world()
+        self.model.load_state_dict(state["model"])
+        if world > 1:
+            for n, b in self.model.named_buffers():
+                if n.endswith(("running_mean", "running_var", "num_batches_tracked")):
+                    dist.broadcast(b, src=0)
+        self.optimizer.load_state_dict(state["optimizer"])          # moments, EMA, step, LR; sync_from_rank0
+        self.optimizer.bump_versions()                               # the packed-weight caches are version-keyed
+        self.optimizer.zero_grad()
+        dev = self.optimizer.bucket.flat.device
+        counter = seed_counter(dev)
+        counter.fill_(int(state["seed_counter"]))
+        base = state["seed_base"]
+        if world > 1:
+            dist.broadcast(counter, src=0)
+            if base is not None:
+                b = torch.tensor([base], dtype=torch.int64, device=dev)
+                dist.broadcast(b, src=0)
+                base = int(b.item())
+        self._seed_base = base
+        self._graph, self._static, self._out = None, None, None
+        if state["capture_seeds"] is not None:
+            self._capture_seeds, self._sig, self._eager_steps = list(state["capture_seeds"]), state["signature"], 0
+        else:
+            self._capture_seeds, self._sig, self._eager_steps = None, None, int(state["eager_steps"])
+        crit = state["criterion"]
+        if hasattr(self.criterion, "set_weights"):
+            self.criterion.set_weights(crit["weights"])
+        for k in ("use_swt", "use_fft"):
+            if crit[k] is not None:
+                setattr(self.criterion, k, crit[k])
+        torch.set_rng_state(state["cpu_rng"])
 
     # ---- validation -----------------------------------------------------------------------------
     def ema_weights(self):
@@ -559,6 +654,91 @@ class FusionTrainer:
         """``validate_epoch`` of the reference's cached mode (train.py:415-515) on this trainer's model."""
         return validate_epoch(self.model, val_loader, self.model.residual_scale.device, crop_border, test_y_channel,
                               self.optimizer if (use_ema and self.optimizer.ema is not None) else None)
+
+
+def check_resume(saved: dict, now: dict, at_epoch_boundary: bool = False) -> None:
+    """Raise ``ValueError`` naming the field when a trainer configured as ``now`` cannot continue a checkpoint whose
+    configuration is ``saved`` (both ``FusionTrainer._resume_config()``): another bucket layout or precision mode; in
+    world-invariant mode a world size N that does not divide the checkpoint's M micro-batches per step, or a trainer
+    whose N * accumulation_steps is not M; in the default mode another accumulation_steps, or another world size
+    unless the checkpoint was taken at an epoch boundary (the default step's bits depend on N)."""
+    if saved["bucket"] != now["bucket"]:
+        raise ValueError("trainer checkpoint: the parameter bucket layout differs from this model's")
+    if saved["precision"] != now["precision"]:
+        raise ValueError(f"trainer checkpoint: precision is {saved['precision']!r} in the checkpoint, "
+                         f"{now['precision']!r} here")
+    if saved["world_invariant"] != now["world_invariant"]:
+        raise ValueError(f"trainer checkpoint: world_invariant is {saved['world_invariant']} in the checkpoint, "
+                         f"{now['world_invariant']} here")
+    if now["world_invariant"]:
+        M = saved["micro_batches"]
+        if M % now["world"]:
+            raise ValueError(f"trainer checkpoint: world size {now['world']} does not divide the checkpoint's "
+                             f"micro_batches M={M}")
+        if now["micro_batches"] != M:
+            raise ValueError(f"trainer checkpoint: micro_batches is M={M} in the checkpoint, {now['micro_batches']} "
+                             f"here: use accumulation_steps={M // now['world']} (or global_micro_batches={M})")
+        return
+    if saved["accumulation_steps"] != now["accumulation_steps"]:
+        raise ValueError(f"trainer checkpoint: accumulation_steps is {saved['accumulation_steps']} in the checkpoint, "
+                         f"{now['accumulation_steps']} here")
+    if saved["world"] != now["world"] and not at_epoch_boundary:
+        raise ValueError(f"trainer checkpoint: world size is {saved['world']} in the checkpoint, {now['world']} here; "
+                         "the default mode changes it only at an epoch boundary (use world_invariant=True to resume "
+                         "mid-epoch on another GPU count)")
+
+
+def atomic_save(obj, path: str) -> None:
+    """``torch.save`` to a temporary file beside ``path``, flushed to disk, then renamed over it: a reader sees the old
+    file or the complete new one, and an interrupted write leaves neither a partial file nor the temporary."""
+    path = os.fspath(path)
+    tmp = f"{path}.{os.getpid()}.{uuid.uuid4().hex}.tmp"
+    try:
+        with open(tmp, "xb") as f:
+            torch.save(obj, f)
+            f.flush()
+            os.fsync(f.fileno())
+        os.replace(tmp, path)
+    except BaseException:
+        if os.path.exists(tmp):
+            os.unlink(tmp)
+        raise
+
+
+def save_checkpoint(path: str, trainer: FusionTrainer, loader=None, extra=None) -> None:
+    """Write ``trainer.state_dict()``, the loader's state (every rank's, for the default mode's per-rank augmentation
+    generators) and ``extra`` (caller state such as an LR scheduler's ``state_dict()`` or the epoch: plain containers,
+    numbers, strings and tensors) to ``path``.  Under a process group every rank calls it and rank 0 writes the file
+    (``atomic_save``).  Take it between steps, after the step's loader batch was consumed."""
+    world = _world()
+    state = {"trainer": trainer.state_dict(), "loader": None, "extra": extra}
+    if loader is not None:
+        mine = loader.state_dict()
+        if world > 1:
+            states = [None] * world
+            dist.all_gather_object(states, mine)
+        else:
+            states = [mine]
+        state["loader"] = states
+    if world == 1 or dist.get_rank() == 0:
+        atomic_save(state, path)
+    if world > 1:
+        dist.barrier()
+
+
+def load_checkpoint(path: str, trainer: FusionTrainer, loader=None):
+    """Load a ``save_checkpoint`` file into ``trainer`` (and ``loader``) on every rank and return its ``extra``.  The
+    default mode may change the world size only when the loader state is at an epoch boundary; a file written
+    without a loader counts as mid-epoch."""
+    ck = torch.load(path, map_location="cpu", weights_only=True)
+    states = ck["loader"]
+    if loader is not None and states is None:
+        raise ValueError(f"checkpoint {path} holds no loader state")
+    trainer.load_state_dict(ck["trainer"], at_epoch_boundary=states is not None and all(s["batch"] == 0 for s in states))
+    if loader is not None:
+        rank = dist.get_rank() if _world() > 1 else 0
+        loader.load_state_dict(states[rank] if rank < len(states) else states[0])
+    return ck["extra"]
 
 
 @torch.no_grad()

@@ -751,6 +751,53 @@ def micro_batch(index: int, seed_base: Optional[int]):
         _MICRO = prev
 
 
+class SeedTape:
+    """The host dropout seeds of one step, in call order.  ``seeds=None`` records: every seed the step hands a dropout
+    kernel is appended, and nothing else changes.  A list replays: the default draws are taken from it in order
+    instead of from torch's CPU generator (hashed world-invariant seeds are computed as usual), so an eager step can
+    use exactly the frozen seeds of a CUDA-graph capture (trainer.py: resuming from a checkpoint)."""
+
+    def __init__(self, seeds: Optional[List[int]] = None):
+        self.replay = seeds is not None
+        self.seeds = [int(s) for s in seeds] if seeds is not None else []
+        self.pos = 0
+
+    def take(self) -> int:
+        if self.pos >= len(self.seeds):
+            raise RuntimeError(f"seed tape holds {len(self.seeds)} dropout seeds; the step asked for more: it differs "
+                               "from the step the seeds were recorded from")
+        self.pos += 1
+        return self.seeds[self.pos - 1]
+
+
+_TAPE: Optional[SeedTape] = None
+
+
+@contextlib.contextmanager
+def seed_tape(seeds: Optional[List[int]] = None):
+    """``with seed_tape() as t:`` records the step's host dropout seeds in ``t.seeds``; ``seed_tape(seeds)`` replays."""
+    global _TAPE
+    prev, _TAPE = _TAPE, SeedTape(seeds)
+    try:
+        yield _TAPE
+    finally:
+        _TAPE = prev
+
+
+def dropout_host_seed() -> int:
+    """Host seed of one train-mode dropout call: the micro-batch hash in a world-invariant step of several
+    micro-batches, else the replaying tape's next seed, else a fresh ``_draw_seed``.  A recording tape logs it."""
+    if _MICRO is not None and _MICRO.seed_base is not None:
+        s = _MICRO.seed()
+    elif _TAPE is not None and _TAPE.replay:
+        return _TAPE.take()
+    else:
+        s = _draw_seed()
+    if _TAPE is not None and not _TAPE.replay:
+        _TAPE.seeds.append(s)
+    return s
+
+
 _SEED_COUNTERS: Dict[str, torch.Tensor] = {}
 _CHECKED = set()
 
@@ -771,7 +818,7 @@ def mha_tokens(x, mha: torch.nn.MultiheadAttention, B: int, T: int, training: bo
     x: [B*T, E, H, W] channels-last token-major.  (large_kernel_attention.py:192-197, 294-299)"""
     qkv = conv2d(x, mha.in_proj_weight, mha.in_proj_bias, tc)
     p = float(mha.dropout) if training else 0.0
-    seed = (_MICRO.seed() if _MICRO is not None else _draw_seed()) if p > 0 else 0
+    seed = dropout_host_seed() if p > 0 else 0
     ctx = _TokenAttention.apply(qkv, B, T, p, seed, seed_counter(x.device) if p > 0 else None)
     return conv2d(ctx, mha.out_proj.weight, mha.out_proj.bias, tc)
 
