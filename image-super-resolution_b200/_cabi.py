@@ -75,6 +75,8 @@ PROTOTYPES = {
     "ffsr_dct_bands": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     "ffsr_dwt_sub_size": (_I, [_I, _I, C.POINTER(_I), C.POINTER(_I)]),
     "ffsr_dwt_bands": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "ffsr_dct_bands_adjoint": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "ffsr_dwt_bands_adjoint": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P]),
     "ffsr_fft_twiddles": (_I, [_I, _P, _P]),
     "ffsr_fft_workspace_bytes": (_SZ, [_I, _I, _I]),
     "ffsr_fft_bands": (_I, [_P, _I, _I, _I, _P, _I, _P, _P, _P, _P, _P, _SZ, _P, _P]),
@@ -136,6 +138,7 @@ PROTOTYPES = {
     "ffsr_bn_apply": (_I, [_P, _I, _L, _I, _P, _P, _P, _P, _P, _P]),
     "ffsr_bn_backward_workspace_bytes": (_SZ, [_I, _L, _I]),
     "ffsr_bn_backward": (_I, [_P, _P, _I, _L, _I, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "ffsr_bn_eval_backward": (_I, [_P, _P, _L, _I, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "ffsr_token_attention_train": (_I, [_P, _I, _I, _L, _I, _P, _P, _F, _U64, _P, _P]),
     "ffsr_token_attention_backward": (_I, [_P, _P, _P, _I, _I, _L, _I, _P, _P, _F, _U64, _P, _P]),
     "ffsr_dwconv_stage": (_I, [_P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),

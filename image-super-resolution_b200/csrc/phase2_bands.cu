@@ -4,6 +4,7 @@
 // Output layout: raw9[B][9][3][H][W] fp32 (band-major planar), so raw9[:, i] is the
 // reference's i-th [B,3,H,W] band.  HBM-bound, tiny next to the HR phases.
 #include "common.cuh"
+#include "../../include/ffsr_b200.h"
 
 // ------------------------------------------------------------------------------------
 // DCT: one 8x8 block of one channel per 64-thread CTA.
@@ -137,6 +138,166 @@ extern "C" int ffsr_dwt_bands(const float* lr, int B, int H, int W, const float*
   dim3 g2(ceil_div(W, 128), H, B * 12);
   k_dwt_resize<<<g2, 128, 0, stream>>>(sub_ws, Hs, Ws, H, W, subband_scale, raw9, B);
   return ffsr_check_launch("dwt_resize");
+}
+
+// ------------------------------------------------------------------------------------
+// Adjoints of the unit-scale DCT and DWT bands: the input gradient of Phase 2.  Gathers only: every output element
+// is written by one thread that sums its sources in a fixed order (no atomics), so the gradient is bitwise
+// reproducible like every training kernel.
+// ------------------------------------------------------------------------------------
+// Per 8x8 block of the padded grid: P = Dt (sum_b M_b .* (D G_b Dt)) D, with G_b the band gradient zero-extended to the
+// padded grid.  X -> Dt (M .* (D X Dt)) D is its own adjoint for any D (the adjoint of X -> D X Dt is G -> Dt G D), so
+// this is exact even though the fp32 basis is not exactly orthogonal.
+__global__ void __launch_bounds__(64) k_dct_adjoint_blocks(
+    const float* __restrict__ g3, int H, int W, int Hp, int Wp,
+    const float* __restrict__ D, const float* __restrict__ Dt,
+    const float* __restrict__ m_low, const float* __restrict__ m_mid, const float* __restrict__ m_high,
+    float* __restrict__ pad) {
+  __shared__ float sD[64], sDt[64], sG[64], sT[64];
+  const int t = threadIdx.x, i = t >> 3, j = t & 7;
+  const int bc = blockIdx.z, b = bc / 3, c = bc % 3;
+  const int y = blockIdx.y * 8 + i, xx = blockIdx.x * 8 + j;
+  sD[t] = D[t];
+  sDt[t] = Dt[t];
+  const bool inside = (y < H) && (xx < W);
+  const float* masks[3] = {m_low, m_mid, m_high};
+  float z = 0.f, acc;
+#pragma unroll
+  for (int band = 0; band < 3; ++band) {
+    __syncthreads();
+    sG[t] = inside ? g3[(((long)b * 3 + band) * 3 + c) * H * W + (long)y * W + xx] : 0.f;
+    __syncthreads();
+    acc = 0.f;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) acc = fmaf(sG[i * 8 + k], sDt[k * 8 + j], acc);   // G Dt
+    sT[t] = acc;
+    __syncthreads();
+    acc = 0.f;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) acc = fmaf(sD[i * 8 + k], sT[k * 8 + j], acc);    // D G Dt
+    z = fmaf(acc, masks[band][t], z);
+  }
+  __syncthreads();
+  sG[t] = z;
+  __syncthreads();
+  acc = 0.f;
+#pragma unroll
+  for (int k = 0; k < 8; ++k) acc = fmaf(sG[i * 8 + k], sD[k * 8 + j], acc);     // Z D
+  sT[t] = acc;
+  __syncthreads();
+  acc = 0.f;
+#pragma unroll
+  for (int k = 0; k < 8; ++k) acc = fmaf(sDt[i * 8 + k], sT[k * 8 + j], acc);    // Dt Z D
+  pad[((long)bc * Hp + y) * Wp + xx] = acc;
+}
+
+// fold of the bottom/right reflect pad: dx[y][x] = sum of P over the padded positions that read (y, x)
+__global__ void k_dct_adjoint_fold(const float* __restrict__ pad, int H, int W, int Hp, int Wp, float* __restrict__ dx) {
+  const int xx = blockIdx.x * blockDim.x + threadIdx.x;
+  const int y = blockIdx.y, bc = blockIdx.z;
+  if (xx >= W) return;
+  const int my = 2 * H - 2 - y, mx = 2 * W - 2 - xx;        // the mirror of y (x) in the pad, if it lies there
+  const bool ry = my >= H && my < Hp, rx = mx >= W && mx < Wp;
+  const float* p = pad + (long)bc * Hp * Wp;
+  float v = p[(long)y * Wp + xx];
+  if (rx) v += p[(long)y * Wp + mx];
+  if (ry) {
+    v += p[(long)my * Wp + xx];
+    if (rx) v += p[(long)my * Wp + mx];
+  }
+  dx[((long)bc * H + y) * W + xx] = v;
+}
+
+extern "C" int ffsr_dct_bands_adjoint(const float* g3, int B, int H, int W, const float* basis, const float* basis_t,
+                                      const float* m_low, const float* m_mid, const float* m_high, float* pad_ws, float* dx,
+                                      cudaStream_t stream) {
+  FFSR_REQUIRE(g3 && dx && pad_ws && basis && basis_t && m_low && m_mid && m_high, FFSR_ERR_ARG, "dct_bands_adjoint: null pointer");
+  FFSR_REQUIRE(B > 0 && H >= 8 && W >= 8, FFSR_ERR_ARG, "dct_bands_adjoint: need B>0 and H,W>=8 (got %d,%d,%d)", B, H, W);
+  const int Hp = ceil_div(H, 8) * 8, Wp = ceil_div(W, 8) * 8;
+  k_dct_adjoint_blocks<<<dim3(Wp / 8, Hp / 8, B * 3), 64, 0, stream>>>(g3, H, W, Hp, Wp, basis, basis_t, m_low, m_mid, m_high, pad_ws);
+  const int rc = ffsr_check_launch("dct_adjoint_blocks");
+  if (rc) return rc;
+  k_dct_adjoint_fold<<<dim3(ceil_div(W, 128), H, B * 3), 128, 0, stream>>>(pad_ws, H, W, Hp, Wp, dx);
+  return ffsr_check_launch("dct_adjoint_fold");
+}
+
+// padded positions p in [-7, pmax] of a 7+7 reflect-padded axis of length n that read element y (pad 7 < n: at most
+// one mirror on each side)
+__device__ __forceinline__ int dwt_sources(int y, int n, int pmax, int (&p)[3]) {
+  int k = 0;
+  p[k++] = y;
+  if (y >= 1 && y <= 7) p[k++] = -y;
+  const int q = 2 * n - 2 - y;
+  if (q >= n && q <= pmax) p[k++] = q;
+  return k;
+}
+
+// dx[y][x] += adjoint of k_dwt_analysis at (y, x): the transposed 8x1 stride-2 column filters (into the lo-row / hi-row
+// intermediates at (y, j)) and the transposed 1x8 stride-2 row filters, each folding its reflect pad.  Input: the
+// subband gradients sub[B][4][3][Hs][Ws] (LL, LH, HL, HH).
+__global__ void k_dwt_analysis_adjoint(const float* __restrict__ sub, int H, int W, int Hs, int Ws,
+                                       const float* __restrict__ lo_row, const float* __restrict__ hi_row,
+                                       const float* __restrict__ lo_col, const float* __restrict__ hi_col,
+                                       float* __restrict__ dx) {
+  const int xx = blockIdx.x * blockDim.x + threadIdx.x;
+  const int y = blockIdx.y;
+  const int bc = blockIdx.z, b = bc / 3, c = bc % 3;
+  if (xx >= W) return;
+  float lr_[8], hr_[8], lc_[8], hc_[8];
+#pragma unroll
+  for (int k = 0; k < 8; ++k) {
+    lr_[k] = lo_row[k]; hr_[k] = hi_row[k]; lc_[k] = lo_col[k]; hc_[k] = hi_col[k];
+  }
+  const long plane = (long)Hs * Ws;
+  const float* sLL = sub + (((long)b * 4 + 0) * 3 + c) * plane;
+  const float* sLH = sub + (((long)b * 4 + 1) * 3 + c) * plane;
+  const float* sHL = sub + (((long)b * 4 + 2) * 3 + c) * plane;
+  const float* sHH = sub + (((long)b * 4 + 3) * 3 + c) * plane;
+  int py[3], px[3];
+  const int ny = dwt_sources(y, H, 2 * Hs - 2, py), nx = dwt_sources(xx, W, 2 * Ws - 2, px);
+  float acc = 0.f;
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    if (a >= nx) break;
+#pragma unroll
+    for (int v = 0; v < 8; ++v) {
+      const int tj = px[a] + 7 - v;                  // p = 2 j + v - 7
+      if (tj & 1) continue;
+      const int j = tj >> 1;
+      if (j < 0 || j >= Ws) continue;
+      float tlo = 0.f, thi = 0.f;                    // gradients of the lo-row / hi-row intermediates at (y, j)
+#pragma unroll
+      for (int e = 0; e < 3; ++e) {
+        if (e >= ny) break;
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+          const int ti = py[e] + 7 - u;
+          if (ti & 1) continue;
+          const int i = ti >> 1;
+          if (i < 0 || i >= Hs) continue;
+          const long o = (long)i * Ws + j;
+          tlo = fmaf(lc_[u], sLL[o], fmaf(hc_[u], sLH[o], tlo));
+          thi = fmaf(lc_[u], sHL[o], fmaf(hc_[u], sHH[o], thi));
+        }
+      }
+      acc = fmaf(lr_[v], tlo, fmaf(hr_[v], thi, acc));
+    }
+  }
+  dx[((long)bc * H + y) * W + xx] += acc;
+}
+
+extern "C" int ffsr_dwt_bands_adjoint(const float* g4, int B, int H, int W, const float* lo_row, const float* hi_row,
+                                      const float* lo_col, const float* hi_col, float* sub_ws, float* dx, cudaStream_t stream) {
+  FFSR_REQUIRE(g4 && dx && sub_ws && lo_row && hi_row && lo_col && hi_col, FFSR_ERR_ARG, "dwt_bands_adjoint: null pointer");
+  FFSR_REQUIRE(B > 0 && H >= 8 && W >= 8, FFSR_ERR_ARG, "dwt_bands_adjoint: need H,W>=8 (reflect pad 7)");
+  int Hs, Ws;
+  ffsr_dwt_sub_size(H, W, &Hs, &Ws);
+  // bilinear (Hs,Ws) -> (H,W) adjoint of the B*12 planes: planar data is channels-last with one channel
+  int rc = ffsr_bilinear_backward(g4, B * 12, H, W, 1, sub_ws, Hs, Ws, FFSR_DT_F32, stream);
+  if (rc) return rc;
+  k_dwt_analysis_adjoint<<<dim3(ceil_div(W, 128), H, B * 3), 128, 0, stream>>>(sub_ws, H, W, Hs, Ws, lo_row, hi_row, lo_col,
+                                                                              hi_col, dx);
+  return ffsr_check_launch("dwt_analysis_adjoint");
 }
 
 // ------------------------------------------------------------------------------------

@@ -23,7 +23,7 @@ int ffsr_check_launch(const char* what) {
 }
 
 extern "C" const char* ffsr_last_error(void) { return g_err; }
-extern "C" const char* ffsr_version(void) { return "ffsr_b200 0.4 (sm_100a)"; }
+extern "C" const char* ffsr_version(void) { return "ffsr_b200 0.5 (sm_100a)"; }
 
 // The library carries sm_100a SASS only: refuse anything else loudly instead of falling back.
 extern "C" int ffsr_device_check(void) {

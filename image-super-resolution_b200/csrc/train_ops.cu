@@ -1259,6 +1259,39 @@ extern "C" int ffsr_bn_backward(const float* x, const float* dy, int G, long R, 
   return ffsr_check_launch("bn_backward_apply");
 }
 
+// eval-mode BatchNorm: the statistics are constants, so dx = dy * w * rstd (float4 over channels, C % 4 == 0)
+__global__ void __launch_bounds__(256) k_bn_eval_dx(const float* __restrict__ dy, long n4, int C, const float* __restrict__ rstd,
+                                                    const float* __restrict__ w, float* __restrict__ dx) {
+  const int C4 = C >> 2;
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
+    const int c = (int)(i % C4) << 2;
+    const float4 g = reinterpret_cast<const float4*>(dy)[i];
+    const float4 rs = *reinterpret_cast<const float4*>(rstd + c), wv = *reinterpret_cast<const float4*>(w + c);
+    reinterpret_cast<float4*>(dx)[i] = make_float4(g.x * (wv.x * rs.x), g.y * (wv.y * rs.y), g.z * (wv.z * rs.z), g.w * (wv.w * rs.w));
+  }
+}
+
+extern "C" int ffsr_bn_eval_backward(const float* x, const float* dy, long R, int C, const float* mean, const float* rstd,
+                                     const float* w, float* sdy, float* sdyx, float* dx, void* ws, size_t ws_bytes,
+                                     cudaStream_t stream) {
+  FFSR_REQUIRE(x && dy && mean && rstd && w && sdy && sdyx && dx && ws && R > 0 && C > 0 && C % 4 == 0, FFSR_ERR_ARG,
+               "bn_eval_backward: bad argument (C %% 4 == 0)");
+  FFSR_REQUIRE(ws_bytes >= ffsr_bn_backward_workspace_bytes(1, R, C), FFSR_ERR_ARG, "bn_eval_backward: workspace too small");
+  dim3 block, grid;
+  long rpb;
+  bn_geom(1, R, C, block, grid, rpb);
+  float* part = (float*)ws;
+  k_bn_bwd_reduce<<<grid, block, 2 * 256 * sizeof(float), stream>>>(x, dy, R, C, rpb, mean, rstd, part);
+  int rc = ffsr_check_launch("bn_eval_backward_reduce");
+  if (rc) return rc;
+  launch_sum_slots<float>(part, (int)grid.x, 2L * C, sdy, stream, sdyx, (long)C);
+  rc = ffsr_check_launch("bn_eval_backward_sum");
+  if (rc) return rc;
+  const long n4 = R * (C / 4);
+  k_bn_eval_dx<<<(int)min((long)148 * 16, (n4 + 255) / 256), 256, 0, stream>>>(dy, n4, C, rstd, w, dx);
+  return ffsr_check_launch("bn_eval_backward_dx");
+}
+
 extern "C" int ffsr_token_attention_train(const float* qkv, int B, int T, long HW, int E, float* ctx, float* probs,
                                           float drop_p, unsigned long long seed, const unsigned long long* seed_dev,
                                           cudaStream_t stream) {

@@ -117,9 +117,13 @@ class CompleteEnhancedFusionSR(nn.Module):
             raise NotImplementedError(
                 "the sm_100a path implements the all-phases-on 4-expert x4 configuration "
                 "(configs/train_config.yaml:63-80); other flag combinations are not built")
-        if self.training:
+        wants_input_grad = torch.is_grad_enabled() and any(
+            t.requires_grad for t in (lr_input, *expert_output_list, *expert_features.values()))
+        if self.training or wants_input_grad:
             # train mode: differentiable graph of library kernels (BN batch statistics, attention
-            # dropout, no output clamps) -- train.py:331-357 calls this under autograd
+            # dropout, no output clamps) -- train.py:331-357 calls this under autograd.  Eval mode with an input that
+            # requires grad (gradient attribution, an upstream module learning through the fusion): the same graph
+            # with eval semantics (BN running statistics, no dropout, the eval clamps)
             from .training import train_forward
             sr, inter = train_forward(self, lr_input, expert_output_list, expert_features, return_intermediates)
             if return_intermediates:

@@ -593,6 +593,44 @@ class _BatchNormTrain(torch.autograd.Function):
         return dx, red[1].sum(0), red[0].sum(0), None
 
 
+class _BatchNormEval(torch.autograd.Function):
+    """nn.BatchNorm2d in eval mode over the running statistics (constants of the graph): gradients to x, weight and
+    bias; the running buffers and num_batches_tracked are not touched."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias, mean, rstd):
+        x = _cl(x)
+        N, Cc, H, W = x.shape
+        y = torch.empty_like(x)
+        w = weight.detach().contiguous()
+        b = bias.detach().contiguous()
+        _ck(_lib().ffsr_bn_apply(x.data_ptr(), 1, N * H * W, Cc, mean.data_ptr(), rstd.data_ptr(), w.data_ptr(), b.data_ptr(),
+                                 y.data_ptr(), _S(x)), "bn_apply(eval)")
+        ctx.save_for_backward(x, mean, rstd, w)
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        x, mean, rstd, w = ctx.saved_tensors
+        N, Cc, H, W = x.shape
+        R = N * H * W
+        gy = _cl(gy)
+        red = _zeros((2, Cc), x.device)
+        dx = torch.empty_like(x)
+        lib = _lib()
+        ws = _ws(lib.ffsr_bn_backward_workspace_bytes(1, R, Cc), x.device)
+        _ck(lib.ffsr_bn_eval_backward(x.data_ptr(), gy.data_ptr(), R, Cc, mean.data_ptr(), rstd.data_ptr(), w.data_ptr(),
+                                      red[0].data_ptr(), red[1].data_ptr(), dx.data_ptr(), ws.data_ptr(), ws.numel(), _S(x)),
+            "bn_eval_backward")
+        return dx, red[1], red[0], None, None
+
+
+def batchnorm_eval(x, bn: torch.nn.BatchNorm2d):
+    mean = bn.running_mean.detach().float().contiguous()
+    rstd = torch.rsqrt(bn.running_var.detach().float() + _BN_EPS)
+    return _BatchNormEval.apply(x, bn.weight, bn.bias, mean, rstd)
+
+
 def batchnorm_train(x, bn: torch.nn.BatchNorm2d, G: int, stats_sink: list):
     """Batch-statistic BN over G groups; the per-group (mean, biased var, n) are appended to
     ``stats_sink`` so the caller can fold the running-stat EMA in call order."""
@@ -866,15 +904,19 @@ class _DwStage(torch.autograd.Function):
 # --------------------------------------------------------------------------------------
 # LKABlock (large_kernel_attention.py:92-105, 143-149), train mode, G statistic groups
 # --------------------------------------------------------------------------------------
-def lka_block_train(x, blk, G: int, sink: list, stats_only: bool = False, tc: bool = False):
-    n = batchnorm_train(x, blk.norm1, G, sink)
+def lka_block_train(x, blk, G: int, sink: list, stats_only: bool = False, tc: bool = False, training: bool = True):
+    """training=False: BatchNorm over the running statistics (the G groups share them)."""
+    def norm(t, bn):
+        return batchnorm_train(t, bn, G, sink) if training else batchnorm_eval(t, bn)
+
+    n = norm(x, blk.norm1)
     a = _DwStage.apply(n, blk.lka.local_conv.weight, 0)
     a = _DwStage.apply(a, blk.lka.h_conv.weight, 1)
     a = _DwStage.apply(a, blk.lka.v_conv.weight, 2)
     a = conv2d(a, blk.lka.pw_conv.weight, None, tc)
-    a = sigmoid(batchnorm_train(a, blk.lka.bn, G, sink))
+    a = sigmoid(norm(a, blk.lka.bn))
     x1 = axpby(x, n * a, blk.scale1)
-    h = batchnorm_train(x1, blk.norm2, G, sink)
+    h = norm(x1, blk.norm2)
     if stats_only:
         return None
     h = conv_chain(h, [(blk.ffn[0].weight, blk.ffn[0].bias, K.ACT_GELU), (blk.ffn[2].weight, blk.ffn[2].bias, K.ACT_NONE)], tc)
@@ -944,37 +986,75 @@ def _to_group_major(x, B, T):
 # --------------------------------------------------------------------------------------
 # Phase 2 in train mode
 # --------------------------------------------------------------------------------------
+def _c32(t):
+    t = t.detach()
+    return t if (t.dtype == torch.float32 and t.is_contiguous()) else t.float().contiguous()
+
+
+def _dwt_sub(B, H, W, dev):
+    hs, ws_ = C.c_int(), C.c_int()
+    _lib().ffsr_dwt_sub_size(H, W, C.byref(hs), C.byref(ws_))
+    return torch.empty(B, 4, 3, hs.value, ws_.value, device=dev)
+
+
+class _Phase2Bands(torch.autograd.Function):
+    """Unit-scale DCT (bands 0-2) and DWT (bands 3-6) sub-bands of lr: raw [B,9,3,H,W], bands 7 and 8 left zero for
+    the FFT pair.  The backward runs the adjoint kernels (ffsr_dct_bands_adjoint / ffsr_dwt_bands_adjoint)."""
+
+    @staticmethod
+    def forward(ctx, lr, fd):
+        lib = _lib()
+        B, _, H, W = lr.shape
+        dev = lr.device
+        S = _S(lr)
+        raw = torch.zeros(B, 9, 3, H, W, device=dev)
+        ones = torch.ones(4, device=dev)
+        d = fd.dct
+        keep = [_c32(d.dct_basis), _c32(d.dct_basis_t), _c32(d.low_mask), _c32(d.mid_mask), _c32(d.high_mask)]
+        _ck(lib.ffsr_dct_bands(lr.data_ptr(), B, H, W, keep[0].data_ptr(), keep[1].data_ptr(), keep[2].data_ptr(),
+                               keep[3].data_ptr(), keep[4].data_ptr(), ones.data_ptr(), raw.data_ptr(), S), "dct_bands")
+        sub = _dwt_sub(B, H, W, dev)
+        w_ = fd.dwt
+        k2 = [_c32(w_.lo_row), _c32(w_.hi_row), _c32(w_.lo_col), _c32(w_.hi_col)]
+        _ck(lib.ffsr_dwt_bands(lr.data_ptr(), B, H, W, k2[0].data_ptr(), k2[1].data_ptr(), k2[2].data_ptr(),
+                               k2[3].data_ptr(), ones.data_ptr(), sub.data_ptr(), raw.data_ptr(), S), "dwt_bands")
+        ctx.fd = fd
+        return raw
+
+    @staticmethod
+    def backward(ctx, g):
+        lib = _lib()
+        B, _, _, H, W = g.shape
+        dev = g.device
+        S = _S(g)
+        g = g.float()
+        g3 = g[:, :3].contiguous()
+        g4 = g[:, 3:7].contiguous()
+        dx = torch.empty(B, 3, H, W, device=dev)
+        d = ctx.fd.dct
+        keep = [_c32(d.dct_basis), _c32(d.dct_basis_t), _c32(d.low_mask), _c32(d.mid_mask), _c32(d.high_mask)]
+        pad = torch.empty(B * 3 * ((H + 7) // 8 * 8) * ((W + 7) // 8 * 8), device=dev)
+        _ck(lib.ffsr_dct_bands_adjoint(g3.data_ptr(), B, H, W, keep[0].data_ptr(), keep[1].data_ptr(), keep[2].data_ptr(),
+                                       keep[3].data_ptr(), keep[4].data_ptr(), pad.data_ptr(), dx.data_ptr(), S),
+            "dct_bands_adjoint")
+        w_ = ctx.fd.dwt
+        k2 = [_c32(w_.lo_row), _c32(w_.hi_row), _c32(w_.lo_col), _c32(w_.hi_col)]
+        sub = _dwt_sub(B, H, W, dev)
+        _ck(lib.ffsr_dwt_bands_adjoint(g4.data_ptr(), B, H, W, k2[0].data_ptr(), k2[1].data_ptr(), k2[2].data_ptr(),
+                                       k2[3].data_ptr(), sub.data_ptr(), dx.data_ptr(), S), "dwt_bands_adjoint")
+        return dx, None
+
+
 def _phase2_train(m, lr):
-    """9 sub-bands [B,9,3,H,W] with gradients to band_scale / subband_scale / FFT mask parameters.
-    The DCT and DWT analysis run on the library kernels with unit scales (the input needs no
-    gradient, so they are constants of the graph) and are scaled by the learnable factors here;
+    """9 sub-bands [B,9,3,H,W] with gradients to band_scale / subband_scale / FFT mask parameters, and to lr when it
+    requires grad.  The DCT and DWT analysis run on the library kernels with unit scales (_Phase2Bands; without an
+    input gradient they are constants of the graph) and are scaled by the learnable factors here;
     the FFT low-pass and the gradient of its learnable mask run on the library's dense-DFT kernels
     (ffsr_fft_lowpass / ffsr_fft_lowpass_backward); the 64x64 -> HxWf mask resize runs on the bilinear node, the sigmoid is a
     tensor op."""
-    lib = _lib()
     fd = m.freq_decomp
     B, _, H, W = lr.shape
-    dev = lr.device
-    S = _S(lr)
-    with torch.no_grad():
-        raw = torch.zeros(B, 9, 3, H, W, device=dev)
-        ones = torch.ones(4, device=dev)
-
-        def c32(t):
-            t = t.detach()
-            return t if (t.dtype == torch.float32 and t.is_contiguous()) else t.float().contiguous()
-
-        d = fd.dct
-        keep = [c32(d.dct_basis), c32(d.dct_basis_t), c32(d.low_mask), c32(d.mid_mask), c32(d.high_mask)]
-        _ck(lib.ffsr_dct_bands(lr.data_ptr(), B, H, W, keep[0].data_ptr(), keep[1].data_ptr(), keep[2].data_ptr(),
-                               keep[3].data_ptr(), keep[4].data_ptr(), ones.data_ptr(), raw.data_ptr(), S), "dct_bands")
-        hs, ws_ = C.c_int(), C.c_int()
-        lib.ffsr_dwt_sub_size(H, W, C.byref(hs), C.byref(ws_))
-        sub = torch.empty(B, 4, 3, hs.value, ws_.value, device=dev)
-        w_ = fd.dwt
-        k2 = [c32(w_.lo_row), c32(w_.hi_row), c32(w_.lo_col), c32(w_.hi_col)]
-        _ck(lib.ffsr_dwt_bands(lr.data_ptr(), B, H, W, k2[0].data_ptr(), k2[1].data_ptr(), k2[2].data_ptr(),
-                               k2[3].data_ptr(), ones.data_ptr(), sub.data_ptr(), raw.data_ptr(), S), "dwt_bands")
+    raw = _Phase2Bands.apply(lr, fd)
     scale7 = torch.cat([fd.dct.band_scale, fd.dwt.subband_scale])
     b7 = raw[:, :7] * scale7[None, :, None, None, None]
     Wf = W // 2 + 1
@@ -1003,8 +1083,9 @@ def _twiddles(n: int, dev) -> torch.Tensor:
 
 
 class _FFTLowpass(torch.autograd.Function):
-    """low = irfft2(mask * rfft2(x), ortho) on the library's dense-DFT kernels (any H, W); gradient w.r.t. the
-    mask only (x is the cached LR input and needs none)."""
+    """low = irfft2(mask * rfft2(x), ortho) on the library's dense-DFT kernels (any H, W) and its gradients.  For a real
+    mask on the half spectrum the map is self-adjoint (on the DC and Nyquist columns irfft2 drops the imaginary parts,
+    which symmetrises the mask there), so the input gradient is one more low-pass of the output gradient."""
 
     @staticmethod
     def forward(ctx, x, mask):
@@ -1016,13 +1097,13 @@ class _FFTLowpass(torch.autograd.Function):
         low = torch.empty_like(x)
         _ck(lib.ffsr_fft_lowpass(x.data_ptr(), B, H, W, m.data_ptr(), _twiddles(H, x.device).data_ptr(),
                                  _twiddles(W, x.device).data_ptr(), ws.data_ptr(), nb, low.data_ptr(), _S(x)), "fft_lowpass")
-        ctx.save_for_backward(x)
+        ctx.save_for_backward(x, m)
         ctx.mask_shape = mask.shape
         return low
 
     @staticmethod
     def backward(ctx, g):
-        (x,) = ctx.saved_tensors
+        x, m = ctx.saved_tensors
         B, _, H, W = x.shape
         lib = _lib()
         g = g.float().contiguous()
@@ -1032,7 +1113,13 @@ class _FFTLowpass(torch.autograd.Function):
         _ck(lib.ffsr_fft_lowpass_backward(x.data_ptr(), g.data_ptr(), B, H, W, _twiddles(H, x.device).data_ptr(),
                                           _twiddles(W, x.device).data_ptr(), ws.data_ptr(), nb, dmask.data_ptr(), _S(x)),
             "fft_lowpass_backward")
-        return None, dmask.view(ctx.mask_shape)
+        dx = None
+        if ctx.needs_input_grad[0]:
+            dx = torch.empty_like(x)
+            _ck(lib.ffsr_fft_lowpass(g.data_ptr(), B, H, W, m.data_ptr(), _twiddles(H, x.device).data_ptr(),
+                                     _twiddles(W, x.device).data_ptr(), ws.data_ptr(), nb, dx.data_ptr(), _S(x)),
+                "fft_lowpass(adjoint)")
+        return dx, dmask.view(ctx.mask_shape)
 
 
 # --------------------------------------------------------------------------------------
@@ -1050,13 +1137,21 @@ def train_forward(m, lr: torch.Tensor, img_list: List[torch.Tensor], feats: Dict
         return _train_forward(m, lr, img_list, feats, want_inter)
 
 
+def _keep(t: torch.Tensor) -> torch.Tensor:
+    """Inputs that require grad stay in the graph (their .float() casts return gradients in their own dtype)."""
+    return t if t.requires_grad else t.detach()
+
+
 def _train_forward(m, lr, img_list, feats, want_inter):
+    """m.training=False: the eval forward as a differentiable graph (for input gradients): BatchNorm over the running
+    statistics, no dropout, no running-stat update, the eval clamps, and phases 2/3/6 in fp32 in both precisions (as at
+    inference, so the derived gate indices are those of the inference path)."""
     if len(img_list) != 4:
         raise ValueError(f"expected the 4 expert outputs drct/grl/nafnet/mamba, got {len(img_list)}")
     B, _, H, W = lr.shape
     Hh, Wh = 4 * H, 4 * W
-    lr = lr.detach().float().contiguous()
-    imgs = [t.detach().float() for t in img_list]
+    lr = _keep(lr).float().contiguous()
+    imgs = [_keep(t).float() for t in img_list]
     training = m.training
     sink: list = []
     inter: Dict = {}
@@ -1081,14 +1176,16 @@ def _train_forward(m, lr, img_list, feats, want_inter):
 
     # ---------------- Phase 3 ----------------
     cb = m.cross_band
+    tc3 = tc and training                                                 # eval: fp32, as at inference
     tok_in = raw9.reshape(B * 9, 3, H, W)                                 # token-major images, NCHW planes
-    proj = cv(tok_in, cb.band_proj)                                       # [B*9,64,H,W]
-    att = mha_tokens(layernorm(proj, cb.norm), cb.band_attention, B, 9, training, tc) + proj
+    proj = conv_mod(tok_in, cb.band_proj, tc3)                            # [B*9,64,H,W]
+    att = mha_tokens(layernorm(proj, cb.norm), cb.band_attention, B, 9, training, tc3) + proj
     gm = _to_group_major(att, B, 9)                                       # [9*B,64,H,W], band-major
-    x_used = lka_block_train(gm[:3 * B], cb.lka_block, 3, sink, tc=tc)
-    with torch.no_grad():                                                 # bands 3..8 feed nothing downstream:
-        lka_block_train(gm[3 * B:].detach(), cb.lka_block, 6, sink, stats_only=True, tc=tc)   # BN running stats only
-    enh = cv(x_used, cb.out_proj).reshape(3, B, 3, H, W) + raw9[:, :3].transpose(0, 1)
+    x_used = lka_block_train(gm[:3 * B], cb.lka_block, 3, sink, tc=tc3, training=training)
+    if training:
+        with torch.no_grad():                                             # bands 3..8 feed nothing downstream:
+            lka_block_train(gm[3 * B:].detach(), cb.lka_block, 6, sink, stats_only=True, tc=tc)   # BN running stats only
+    enh = conv_mod(x_used, cb.out_proj, tc3).reshape(3, B, 3, H, W) + raw9[:, :3].transpose(0, 1)
     routing = enh.sum(0)                                                  # [B,3,H,W]
 
     # ---------------- Phase 6 nets ----------------
@@ -1121,7 +1218,7 @@ def _train_forward(m, lr, img_list, feats, want_inter):
             if n not in feats:
                 aligned.append(None)
                 continue
-            f = feats[n].detach().float()
+            f = _keep(feats[n]).float()
             if tuple(f.shape[2:]) != (H, W):
                 f = _bilinear(_cl(f), (H, W))
             al = co.align_layers[n]
@@ -1146,7 +1243,7 @@ def _train_forward(m, lr, img_list, feats, want_inter):
         x = tokens + mha_tokens(layernorm(tokens, co.norm1), co.cross_attn, B, 4, training, tc)
         x = x + conv_chain(layernorm(x, co.norm2), [(co.ffn[0].weight, co.ffn[0].bias, K.ACT_GELU),
                                                     (co.ffn[2].weight, co.ffn[2].bias, K.ACT_NONE)], tc)
-        xg = lka_block_train(_to_group_major(x, B, 4), co.lka_global, 4, sink, tc=tc)      # [4*B,128,H,W]
+        xg = lka_block_train(_to_group_major(x, B, 4), co.lka_global, 4, sink, tc=tc, training=training)  # [4*B,128,H,W]
         ecol = []
         for i in range(4):
             mod = co.modulation[i]
@@ -1249,4 +1346,6 @@ def _train_forward(m, lr, img_list, feats, want_inter):
         inter["fused_before_dynamic"] = fused_before
         inter["gates"] = gates
         inter["difficulty"] = diff
+        if not training:
+            inter["active"] = graw > (0.7 - 0.5 * diff)                   # as FusionEngine reports it
     return out, inter

@@ -71,6 +71,15 @@ int ffsr_dwt_sub_size(int H, int W, int* Hs, int* Ws);
 int ffsr_dwt_bands(const float* lr, int B, int H, int W, const float* lo_row, const float* hi_row,
                    const float* lo_col, const float* hi_col, const float* subband_scale, float* sub_ws,
                    float* raw9, cudaStream_t stream);
+/* Adjoints of the unit-scale DCT / DWT bands (input gradient of Phase 2; gathers, no atomics, fixed summation order).
+ * ffsr_dct_bands_adjoint: g3[B][3][3][H][W] (low, mid, high) -> dx[B][3][H][W] (WRITTEN); pad_ws: float[B*3*Hp*Wp],
+ *   Hp / Wp = H / W rounded up to a multiple of 8.
+ * ffsr_dwt_bands_adjoint: g4[B][4][3][H][W] (LL, LH, HL, HH) -> dx[B][3][H][W] (ACCUMULATED); sub_ws as for ffsr_dwt_bands. */
+int ffsr_dct_bands_adjoint(const float* g3, int B, int H, int W, const float* basis, const float* basis_t,
+                           const float* m_low, const float* m_mid, const float* m_high, float* pad_ws, float* dx,
+                           cudaStream_t stream);
+int ffsr_dwt_bands_adjoint(const float* g4, int B, int H, int W, const float* lo_row, const float* hi_row,
+                           const float* lo_col, const float* hi_col, float* sub_ws, float* dx, cudaStream_t stream);
 /* FFTDecomposition.forward      src/models/multi_domain_frequency.py:352-385
  * tw_h / tw_w: double2[H] / double2[W] tables from ffsr_fft_twiddles; ws from ffsr_fft_workspace_bytes */
 int ffsr_fft_twiddles(int n, void* out, cudaStream_t stream);
@@ -326,6 +335,12 @@ int ffsr_bn_apply(const float* x, int G, long R, int C, const float* mean, const
 size_t ffsr_bn_backward_workspace_bytes(int G, long R, int C);
 int ffsr_bn_backward(const float* x, const float* dy, int G, long R, int C, const float* mean, const float* rstd,
                      const float* w, float* sdy, float* sdyx, float* dx, void* ws, size_t ws_bytes, cudaStream_t stream);
+/* nn.BatchNorm2d in eval mode with gradients (running statistics as constants) on channels-last [R][C]: forward is
+ * ffsr_bn_apply with G = 1 and (running_mean, rsqrt(running_var + eps)); the backward gives
+ *   sdy[c] += sum dy, sdyx[c] += sum dy*xhat (ACCUMULATED, fixed order), dx = dy * w * rstd;
+ * ws sized by ffsr_bn_backward_workspace_bytes(1, R, C). */
+int ffsr_bn_eval_backward(const float* x, const float* dy, long R, int C, const float* mean, const float* rstd,
+                          const float* w, float* sdy, float* sdyx, float* dx, void* ws, size_t ws_bytes, cudaStream_t stream);
 
 /* nn.MultiheadAttention core in train mode (T = 4 or 9 tokens per LR pixel, head_dim 16,
  * attention-probability dropout): probs[B][HW][E/16][T][T] saved for the backward; the dropout
